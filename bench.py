@@ -16,8 +16,13 @@ tries, hashed level-synchronously.
   e2e    the same metric through the C ABI (ppd_block_decode) with HOST buffers: FlatBlock in,
          IrDump out, every host<->device copy and all host work inside the timed region
 One JSON line on stdout (rank 0).
+
+  --dump-outputs DIR   after the timed steps, write what the last timed step returned to its caller as .npy files
+                       (see dump_ir_records); the inputs depend on the arguments alone, so two builds can be compared
+                       file for file
 """
 import argparse
+import hashlib
 import json
 import os
 import subprocess
@@ -145,9 +150,48 @@ def c2_blocks(seeds, scale, procs):
     return [c2_block(s, scale) for s in seeds]
 
 
-def oracle_time_block(flat_bytes, repeats, threads):
+DUMP_CHUNKS, DUMP_CHUNK, DUMP_SEED = 64, 512, 20250101  # 32 KiB of every IrDump, 128 KiB as float32
+
+
+def ir_dump_record(view):
+    """What --dump-outputs keeps of one IrDump (bytes or a memoryview): its length, its SHA-256 (which covers every byte)
+    and DUMP_CHUNKS runs of DUMP_CHUNK bytes at offsets drawn from a fixed seed, so that two dumps of the same length are
+    sampled at the same places.  Cheap enough to run on the library's callback thread before the buffer is released."""
+    import numpy as np
+
+    a = np.frombuffer(view, dtype=np.uint8)
+    n = a.size
+    offsets = np.sort((np.random.default_rng(DUMP_SEED).random(DUMP_CHUNKS) * max(n - DUMP_CHUNK, 0)).astype(np.int64))
+    idx = offsets[:, None] + np.arange(DUMP_CHUNK)
+    sample = np.full(idx.shape, -1.0, dtype=np.float32)  # -1: past the end of a dump shorter than one run
+    inside = idx < n
+    sample[inside] = a[idx[inside]]
+    return n, hashlib.sha256(view).digest(), offsets, sample
+
+
+def dump_ir_records(out_dir, records):
+    """records: one ir_dump_record per block, in the order of the step's input list.  Writes
+      ir_dump_nbytes.npy          float64 [blocks]               length of each IrDump
+      ir_dump_sha256.npy          float32 [blocks, 32]           its SHA-256, one byte per entry
+      ir_dump_sample_offsets.npy  float64 [blocks, CHUNKS]       where each sampled run starts
+      ir_dump_sample.npy          float32 [blocks, CHUNKS, CHUNK] the sampled bytes (-1 past the end)"""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        "ir_dump_nbytes": np.array([r[0] for r in records], dtype=np.float64),
+        "ir_dump_sha256": np.array([list(r[1]) for r in records], dtype=np.float32).reshape(len(records), 32),
+        "ir_dump_sample_offsets": np.array([r[2] for r in records], dtype=np.float64).reshape(len(records), DUMP_CHUNKS),
+        "ir_dump_sample": np.array([r[3] for r in records], dtype=np.float32).reshape(len(records), DUMP_CHUNKS, DUMP_CHUNK),
+    }
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    print(f"bench: wrote {', '.join(arrays)} ({len(records)} blocks) to {out_dir}", file=sys.stderr, flush=True)
+
+
+def oracle_time_block(flat_bytes, repeats, threads, keep=None):
     """Decode `flat_bytes` `repeats` times on each of `threads` host threads (ctypes releases the GIL).
-    Returns (wall seconds, stats of one decode)."""
+    Returns (wall seconds, stats of one decode).  With a list as `keep`, the IrDump of the last decode is appended to it."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import ppd_oracle_lib
 
@@ -156,8 +200,10 @@ def oracle_time_block(flat_bytes, repeats, threads):
 
     def work():
         for _ in range(repeats):
-            oracle.block_decode(flat_bytes)
+            out = oracle.block_decode(flat_bytes)
         stats.update(oracle.last_stats())
+        if keep is not None and not keep:
+            keep.append(out)
 
     ts = [threading.Thread(target=work) for _ in range(threads)]
     t0 = time.perf_counter()
@@ -179,10 +225,12 @@ def run_reference(args, rank, world):
     flat_bytes = c2_block(2, sample_scale)
     for _ in range(max(1, min(args.warmup, 1))):
         oracle_time_block(flat_bytes, 1, cores)
-    t_total, st = 0.0, {}
-    for _ in range(args.steps):
-        t, st = oracle_time_block(flat_bytes, 1, cores)
+    t_total, st, last = 0.0, {}, []
+    for k in range(args.steps):
+        t, st = oracle_time_block(flat_bytes, 1, cores, keep=last if k == args.steps - 1 else None)
         t_total += t
+    if args.dump_outputs:
+        dump_ir_records(args.dump_outputs, [ir_dump_record(last[0])])
     nodes = st["nodes_hashed"] * cores * args.steps
     value = nodes / t_total
     workload = "C2 mainnet-shaped block (BASELINE.json configs[1])" + ("" if sample_scale == 1.0 else f" at {sample_scale:g}x scale")
@@ -502,13 +550,16 @@ def run_b200(args, rank, world, local_rank):
     # blocks; outputs are consumed as they finish, so only those in flight are held
     e2e_mult = max(1, args.e2e_mult)
 
-    def decode_step(mult=1):
-        # ppd_blocks_decode_stream: every block's IrDump is handed over (and read, and released) as soon as it is done
+    def decode_step(mult=1, records=None):
+        # ppd_blocks_decode_stream: every block's IrDump is handed over (and read, and released) as soon as it is done;
+        # with `records`, the first decode of every distinct block also leaves its ir_dump_record there
         got = []
 
         def on_done(i, o):
             if isinstance(o, Exception):
                 raise o
+            if records is not None and i < len(flats):
+                records[i] = ir_dump_record(o.view)
             got.append(o.nbytes + o.view[0] + o.view[o.nbytes - 1])  # read the result
             o.close()
 
@@ -545,14 +596,18 @@ def run_b200(args, rank, world, local_rank):
     dump_ms = replay(ctx.REPLAY_DUMP) if on_device else 0.0
     all_ms = replay(ctx.REPLAY_ALL)
     # ---- end to end through the C ABI with host buffers ----
+    # (--dump-outputs: rank 0 records the last step's IrDumps; hashing them adds host work to that step alone)
+    records = {} if args.dump_outputs and rank == 0 else None
     barrier()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        ir_len = decode_step(e2e_mult)
+    for k in range(args.steps):
+        ir_len = decode_step(e2e_mult, records if k == args.steps - 1 else None)
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
     barrier()
     e2e_s = max_over_ranks(e2e_s)
+    if records is not None:
+        dump_ir_records(args.dump_outputs, [records[j] for j in range(n_blocks)])
     clocks = sampler.stop()
     st = ctx.stats()
     # latency of one block alone, and the node count of the seed-2 block (rank 0) for the normalisation below
@@ -769,6 +824,7 @@ def run_b200(args, rank, world, local_rank):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing there, bytecode included
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
@@ -783,7 +839,12 @@ def main():
     ap.add_argument("--c5-leaves", type=int, default=32_000_000, help="leaves of the config-5 trie that is split over the GPUs")
     ap.add_argument("--c3-slots", type=int, default=1_000_000, help="slots of each of the four config-3 storage tries that are sharded over the GPUs")
     ap.add_argument("--no-split", action="store_true", help="skip the c5_split / c3_sharded legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the IrDumps the last end-to-end step returned (length, SHA-256 and a "
+                         "fixed sample of each distinct block's dump) to DIR as .npy files; rank 0's blocks only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
