@@ -80,12 +80,9 @@ bool gpu_pre_image(Lane* L, Job& J, BlockJob& b, bool check_version, Slots* slot
     fprintf(stderr, "[ppd]   %-12s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
     t_prev = now;
   };
+  // the waits while the slot is held sleep too: polling measured +3 % blocks/s for 3.5x the host CPU (DESIGN.md §3), and
+  // polling threads of several GPUs' ranks would take cores from each other
   SlotGuard slot(slots, &L->stats.host_wait_ms);
-  // (PPD_SLOT_POLL=1: poll instead of sleeping while a parse slot is held — round 1's host-heavy pipeline woke sleeping
-  // threads late; with the txn loop on the device the cores are mostly idle, and polling threads of several GPUs' ranks
-  // would take them from each other)
-  static const bool slot_poll = getenv("PPD_SLOT_POLL") != nullptr && atoi(getenv("PPD_SLOT_POLL")) != 0;
-  auto sync_in_slot = [&] { (slots && slot_poll) ? lane_sync_poll(L) : lane_sync(L); };
   // the result words a host thread waits for: written into page-locked memory by a kernel when the whole block stays on
   // the device (a copy engine would serve them behind every bulk upload other lanes have queued)
   auto small_to_host = [&](void* dst, const void* src, size_t bytes) {
@@ -145,7 +142,7 @@ bool gpu_pre_image(Lane* L, Job& J, BlockJob& b, bool check_version, Slots* slot
   CUDA_OK(cudaGetLastError());
   CUDA_OK(cudaEventRecord(L->ev1, st));
   result_to_host();
-  sync_in_slot();
+  lane_sync(L);
   phase_ms();
   lap("p:upload+A");
   trace_mark(L, "parse_a");
@@ -198,7 +195,7 @@ bool gpu_pre_image(Lane* L, Job& J, BlockJob& b, bool check_version, Slots* slot
   CUDA_OK(cudaGetLastError());
   CUDA_OK(cudaEventRecord(L->ev1, st));
   result_to_host();
-  sync_in_slot();
+  lane_sync(L);
   phase_ms();
   lap("p:B");
   trace_mark(L, "parse_b");

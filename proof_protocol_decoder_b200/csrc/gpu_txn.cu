@@ -511,25 +511,19 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
   }
 #endif
   trace_mark(L, "prep");
-  if (c->batcher && L->lease) {
-    // the loop runs on a loop stream, batched with the loops of other lanes that are due; this lane's main stream goes
-    // back to the pool meanwhile
-    lane_copy_flush(L);
-    CUDA_OK(cudaEventRecord(L->ev_ready, st));
-    L->lease->release();
-    L->stats.kernel_launches += loop_batcher_run(c->batcher, v, b.state_root, T.max_ops, L->ev_ready, L->ev_loop0, L->ev_loop1, L->ev_loop_done);
-    {
-      const auto tw = std::chrono::steady_clock::now();
-      CUDA_OK(cudaEventSynchronize(L->ev_loop_done));
-      L->stats.host_wait_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw).count();
-    }
-    L->lease->acquire();
-    st = L->st;
-  } else {
-    CUDA_OK(cudaEventRecord(L->ev_loop0, st));
-    L->stats.kernel_launches += launch_txn_loop(L->h_task, v, b.state_root, T.max_ops, st);
-    CUDA_OK(cudaEventRecord(L->ev_loop1, st));
+  // the loop runs on a loop stream, batched with the loops of other lanes that are due; this lane's main stream goes
+  // back to the pool meanwhile
+  lane_copy_flush(L);
+  CUDA_OK(cudaEventRecord(L->ev_ready, st));
+  L->lease->release();
+  L->stats.kernel_launches += loop_batcher_run(c->batcher, v, b.state_root, T.max_ops, L->ev_ready, L->ev_loop0, L->ev_loop1, L->ev_loop_done);
+  {
+    const auto tw = std::chrono::steady_clock::now();
+    CUDA_OK(cudaEventSynchronize(L->ev_loop_done));
+    L->stats.host_wait_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw).count();
   }
+  L->lease->acquire();
+  st = L->st;
   trace_mark(L, "loop");
   // ---- the loop's nodes sorted by (level, class) ----
   L->d_order2.reserve(4ull * H.cap_tail + 16);

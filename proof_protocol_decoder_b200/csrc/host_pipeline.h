@@ -144,11 +144,9 @@ struct SlotGuard {
   }
   ~SlotGuard() { done(); }
 };
-inline int parse_slots() {
-  const char* e = getenv("PPD_PARSE_SLOTS");
-  int v = e ? atoi(e) : 8;
-  return v < 1 ? 1 : v;
-}
+// Lanes admitted at once.  A sweep of 12, 16 and 32 (profiles/r02b_knobs.txt: 512 config-2 blocks per stream call)
+// moved no further from 8 than two runs at 8 differ (578 and 617 blocks/s); 32 gave 623, not re-measured.
+constexpr int PARSE_SLOTS = 8;
 
 }  // namespace ppd
 
@@ -183,7 +181,7 @@ struct StreamPool {
     cv.notify_one();
   }
 };
-// a decode's hold on a pool stream (no pool: the lane keeps its own stream throughout)
+// a decode's hold on a pool stream (no pool, in the host-only profiling build PPD_HOSTPROF: the lane keeps its own stream)
 struct StreamLease {
   StreamPool* pool;
   Lane* L;
@@ -221,9 +219,9 @@ uint32_t loop_batcher_run(LoopBatcher* b, const txn::View& v, uint32_t initial_s
 
 struct ppd_ctx {
   int device = 0;
-  ppd::StreamPool* pool = nullptr;      // null: every lane works on its own stream
+  ppd::StreamPool* pool = nullptr;      // (both null only in the host-only profiling build PPD_HOSTPROF)
   ppd::LoopBatcher* batcher = nullptr;
-  ppd::Slots parse_slots_sem{ppd::parse_slots()};
+  ppd::Slots parse_slots_sem{ppd::PARSE_SLOTS};
   cudaStream_t st = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::string err;
@@ -241,7 +239,6 @@ namespace ppd {
 
 void stats_reset(ppd_ctx* c);
 void lane_sync(Lane* l);
-void lane_sync_poll(Lane* l);
 // PPD_TRACE=<file>: one row per stage boundary of every block (lane, block, label, device ms, host ms since the
 // context was made), for the pipeline timeline in profiles/.  Off: trace_mark costs one predictable branch.
 // copy by kernel (CopyBatch): queue, and launch what is queued.  Anything launched after a flush sees the copies.

@@ -58,23 +58,6 @@ void lane_sync(Lane* l) {
   CUDA_OK(cudaEventSynchronize(l->ev_sync));
   l->stats.host_wait_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
 }
-// The same by polling, for the short waits a lane makes while it holds a parse slot (at most PPD_PARSE_SLOTS
-// threads poll at a time): a sleeping thread is woken late when every core is busy shaping other blocks, and
-// everything queued behind the slot waits with it.
-void lane_sync_poll(Lane* l) {
-  lane_copy_flush(l);
-  const auto t0 = std::chrono::steady_clock::now();
-  CUDA_OK(cudaEventRecord(l->ev_sync, l->st));
-  for (unsigned spins = 0;; spins++) {
-    cudaError_t e = cudaEventQuery(l->ev_sync);
-    if (e == cudaSuccess) {
-      l->stats.host_wait_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-      return;
-    }
-    if (e != cudaErrorNotReady) CUDA_OK(e);
-    if (spins > 200) std::this_thread::yield();
-  }
-}
 
 // ---- PPD_TRACE ----
 namespace {
@@ -559,28 +542,22 @@ int ppd_ctx_create(int device, ppd_ctx** out) {
     return PPD_ERR_CUDA;
   }
   // the stream pool and the loop streams (host_pipeline.h: StreamPool): made first and together, so that they sit on
-  // hardware queues of their own; PPD_STREAM_POOL=0: every lane on its own stream, loops included
-  {
-    const char* e = getenv("PPD_STREAM_POOL");
-    const int n_main = e ? atoi(e) : 22;
-    const char* e2 = getenv("PPD_LOOP_STREAMS");
-    const int n_loop = e2 ? std::max(1, atoi(e2)) : 8;
-    if (n_main > 0) {
-      c->pool = new StreamPool();
-      for (int k = 0; k < n_main; k++) {
-        cudaStream_t s = nullptr;
-        if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) != cudaSuccess) {
-          ppd_ctx_destroy(c);
-          return PPD_ERR_CUDA;
-        }
-        c->pool->all.push_back(s), c->pool->free_.push_back(s);
-      }
-      c->batcher = loop_batcher_create(device, n_loop);
-      if (!c->batcher) {
-        ppd_ctx_destroy(c);
-        return PPD_ERR_CUDA;
-      }
+  // hardware queues of their own.  22 + 8 stay below the 32 queues.  In a sweep (profiles/r02b_knobs.txt: 512 config-2
+  // blocks per stream call) 24 + 6 gave 619 blocks/s and 26 + 4 588, against two runs of 22 + 8 at 578 and 617.
+  constexpr int MAIN_STREAMS = 22, LOOP_STREAMS = 8;
+  c->pool = new StreamPool();
+  for (int k = 0; k < MAIN_STREAMS; k++) {
+    cudaStream_t s = nullptr;
+    if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) != cudaSuccess) {
+      ppd_ctx_destroy(c);
+      return PPD_ERR_CUDA;
     }
+    c->pool->all.push_back(s), c->pool->free_.push_back(s);
+  }
+  c->batcher = loop_batcher_create(device, LOOP_STREAMS);
+  if (!c->batcher) {
+    ppd_ctx_destroy(c);
+    return PPD_ERR_CUDA;
   }
   *out = c;
   return PPD_OK;
@@ -722,49 +699,17 @@ int ppd_replay_last(ppd_ctx* c, unsigned what, double* gpu_ms_out) {
               ((what & (PPD_REPLAY_TXN | PPD_REPLAY_DUMP)) && L->has_last_txn);
     }
     if (!used) fail(PPD_ERR_BAD_ARGUMENT, "nothing of the requested kind is resident");
-    // all lanes start after ev0 on the main stream; the main stream then waits for every lane.  One host thread queues
-    // all lanes by default; PPD_REPLAY_THREADS=<n> spreads the lanes over n threads, as the decode itself does.  Measured
-    // (profiles/r02b_replay_threads.txt): 30 lanes' parse replay 13.4 ms queued by one thread, 13.7 ms by thirty -- the
-    // replays are bound by the device, not by the queueing thread (one thread launches 0.29 M kernels/s, r02b_launch_rate.txt).
-    static const unsigned replay_threads = [] {
-      const char* e = getenv("PPD_REPLAY_THREADS");
-      const long v = e ? atol(e) : 1;
-      return (unsigned)(v > 0 ? v : 1);
-    }();
-    const unsigned workers = (unsigned)std::min<size_t>(replay_threads, n_lanes);
-    // the threads exist and wait before ev0 is recorded, so that starting them is not inside the timed region
-    std::atomic<unsigned> ready{0};
-    std::atomic<bool> go{false}, failed{false};
-    Fail first{PPD_OK, ""};
-    std::mutex mu;
-    auto body = [&](unsigned t) {
-      try {
-        if (t) {
-          CUDA_OK(cudaSetDevice(c->device));
-          ready.fetch_add(1);
-          while (!go.load(std::memory_order_acquire)) std::this_thread::yield();
-        }
-        for (size_t w = t; w < n_lanes && !failed.load(); w += workers) {
-          Lane* L = c->lanes[w];
-          CUDA_OK(cudaStreamWaitEvent(L->st, c->ev0, 0));
-          replay_lane(L, what);
-          CUDA_OK(cudaEventRecord(L->ev1, L->st));
-        }
-      } catch (const Fail& e) {
-        if (t && !go.load()) ready.fetch_add(1);  // (cudaSetDevice failed before the thread reported in)
-        std::lock_guard<std::mutex> g(mu);
-        if (!failed.exchange(true)) first = e;
-      }
-    };
-    std::vector<std::thread> th;
-    for (unsigned t = 1; t < workers; t++) th.emplace_back(body, t);
-    while (ready.load() + 1 < workers) std::this_thread::yield();
-    cudaError_t e0 = cudaEventRecord(c->ev0, c->st);
-    go.store(true, std::memory_order_release);
-    if (e0 == cudaSuccess) body(0);
-    for (auto& t : th) t.join();
-    CUDA_OK(e0);
-    if (failed.load()) throw first;
+    // all lanes start after ev0 on the main stream; the main stream then waits for every lane.  The calling thread
+    // queues every lane: the replays are bound by the device, not by the queueing thread (profiles/r02b_replay_threads.txt:
+    // 30 lanes' parse replay 13.4 ms queued by one thread, 13.7 ms by thirty; one thread launches 0.29 M kernels/s,
+    // r02b_launch_rate.txt).
+    CUDA_OK(cudaEventRecord(c->ev0, c->st));
+    for (size_t w = 0; w < n_lanes; w++) {
+      Lane* L = c->lanes[w];
+      CUDA_OK(cudaStreamWaitEvent(L->st, c->ev0, 0));
+      replay_lane(L, what);
+      CUDA_OK(cudaEventRecord(L->ev1, L->st));
+    }
     for (size_t w = 0; w < n_lanes; w++) CUDA_OK(cudaStreamWaitEvent(c->st, c->lanes[w]->ev1, 0));
     CUDA_OK(cudaEventRecord(c->ev1, c->st));
     CUDA_OK(cudaStreamSynchronize(c->st));

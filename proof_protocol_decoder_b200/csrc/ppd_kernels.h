@@ -130,9 +130,6 @@ enum {  // per-instruction size counters, scanned together
   PARSE_C_CODE = 6,   // inline code strings
   PARSE_N_CNT = 7
 };
-struct Pyramid16 {
-  const int16_t *L, *m1, *m2, *m3;
-};
 struct ParseBounds {
   const uint8_t* wit;     // witness bytes (readable up to n + 16)
   uint32_t n;

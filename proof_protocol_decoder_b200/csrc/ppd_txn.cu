@@ -230,6 +230,9 @@ uint32_t launch_txn_prep(const View& v, const AcctInit& a, uint32_t n_ops1, uint
   }
   return launches;
 }
+// txns per launch of the loop kernel: a raised flag stops the batch at the next launch.  64 gave 615 blocks/s in a sweep
+// (profiles/r02b_knobs.txt: 512 config-2 blocks per stream call), within two runs of 16 at 578 and 617.
+constexpr uint32_t LOOP_CHUNK = 16;
 uint32_t txn_loop_uses_shared(uint32_t max_keys) { return max_keys <= SH_KEYS ? 1u : 0u; }  // max_keys: the most keys any txn of the block has
 uint32_t launch_txn_loops(const LoopTask* tasks, uint32_t n, uint32_t max_txns, bool any_shared, cudaStream_t st) {
   static const bool attr = [] {
@@ -238,17 +241,12 @@ uint32_t launch_txn_loops(const LoopTask* tasks, uint32_t n, uint32_t max_txns, 
   }();
   (void)attr;
   const size_t smem = LOOP_SCRATCH_BYTES + (any_shared ? sizeof(LoopShared) : 0);
-  static const uint32_t chunk = [] {
-    const char* e = getenv("PPD_LOOP_CHUNK");
-    const int x = e ? atoi(e) : 16;
-    return (uint32_t)(x < 1 ? 1 : x);
-  }();
   if (n > LOOP_BATCH_MAX) n = LOOP_BATCH_MAX;
   static thread_local LoopBatchArg A;  // (copied into the launch: the caller's array is free again on return)
   for (uint32_t k = 0; k < n; k++) A.t[k] = tasks[k];
   uint32_t launches = 0;
-  for (uint32_t t0 = 0; t0 < max_txns || launches == 0; t0 += chunk) {
-    txn_loop_kernel<<<n, LOOP_THREADS, smem, st>>>(A, t0, t0 + chunk);
+  for (uint32_t t0 = 0; t0 < max_txns || launches == 0; t0 += LOOP_CHUNK) {
+    txn_loop_kernel<<<n, LOOP_THREADS, smem, st>>>(A, t0, t0 + LOOP_CHUNK);
     launches++;
   }
   return launches;

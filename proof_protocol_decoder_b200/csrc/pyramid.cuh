@@ -1,7 +1,7 @@
-// pyramid.cuh — nearest-smaller-value queries over an integer array (int8 `Pyramid`, int16 `Pyramid16`) through a 3-level min-pyramid
-// (64 / 4 096 / 262 144 positions per cell).  Shared by the sorted-leaf trie builder (ppd_build.cu:
-// branch runs of the LCP array) and the witness parser (ppd_parse.cu: the parent of a post-order
-// instruction is the next instruction whose stack height is not larger).
+// pyramid.cuh — nearest-smaller-value queries over an int8 array (`Pyramid`) through a 3-level min-pyramid
+// (64 / 4 096 / 262 144 positions per cell).  Used by the sorted-leaf trie builder (ppd_build.cu: branch runs
+// of the LCP array); the witness parser has its own int16 form with an extra 8-wide level (ppd_parse.cu,
+// scan_right8).
 #pragma once
 #include <cstdint>
 
@@ -10,8 +10,7 @@
 namespace ppd {
 
 // largest p < q with L[p] < thr (thr >= 0; L[0] = -1 guarantees termination)
-template <class PyramidT>
-static __device__ __forceinline__ uint32_t scan_left(const PyramidT& P, uint32_t q, int thr) {
+static __device__ __forceinline__ uint32_t scan_left(const Pyramid& P, uint32_t q, int thr) {
   uint32_t p = q - 1;
   for (;;) {
     if ((p & 63u) == 63u) {
@@ -35,8 +34,7 @@ static __device__ __forceinline__ uint32_t scan_left(const PyramidT& P, uint32_t
   }
 }
 // smallest r > q with L[r] < thr (L[N] = -1 guarantees termination)
-template <class PyramidT>
-static __device__ __forceinline__ uint32_t scan_right(const PyramidT& P, uint32_t q, int thr) {
+static __device__ __forceinline__ uint32_t scan_right(const Pyramid& P, uint32_t q, int thr) {
   uint32_t p = q + 1;
   for (;;) {
     if ((p & 63u) == 0u) {
