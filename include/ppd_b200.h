@@ -146,8 +146,10 @@ int ppd_trie_root_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, const
 
 /* One huge trie over several streams or GPUs (SURVEY.md 8e (3)): the leaves are split by their first `base_depth`
  * nibbles; each part is hashed like a whole trie, except that its nodes sit `base_depth` nibbles below the root
- * (ref_out = the 32 bytes the node above embeds; every key of the part must share those nibbles, and the part's top
- * node must encode to at least 32 bytes, which a 64-nibble key guarantees).  DEVICE pointers. */
+ * (ref_out = the hash of the part's top node, the 32 bytes the node above embeds).  Every key of the part must share
+ * those nibbles, and the top node must encode to at least 32 bytes, or the node above would embed its raw encoding
+ * instead: either violation returns PPD_ERR_BAD_ARGUMENT.  Short tops exist from base_depth 9 on (one leaf with a
+ * one-byte value encodes to 31 bytes there); base_depth 1 always gives 32 bytes or more.  DEVICE pointers. */
 int ppd_trie_subroot_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n,
                                        size_t vals_bytes, uint32_t base_depth, uint8_t ref_out[32]);
 /* ... and the branch over them: child_hashes16x32[i] is the ref of the part whose next nibble is i (used when bit i of

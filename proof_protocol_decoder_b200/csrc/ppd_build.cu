@@ -53,9 +53,11 @@ __device__ __forceinline__ int lcp_nibbles(const uint4* a, const uint4* bq, int*
   return 64;
 }
 
-// L[0] = L[N] = -1;  L[i] = lcp(key[i-1], key[i]).  flags[0] |= 1 if not strictly ascending.
+// L[0] = L[N] = -1;  L[i] = lcp(key[i-1], key[i]).  flags[0] |= BUILD_F_UNSORTED if not strictly ascending.
 // (for a SUB-trie whose keys share their first base_depth nibbles the two ends get base_depth - 1, which is what
-// they are inside the whole trie: every node then sits where it sits there)
+// they are inside the whole trie: every node then sits where it sits there.  A pair sharing fewer nibbles raises
+// BUILD_F_PREFIX and stores base_depth, so that the ends stay below every interior L and the scans stay in range
+// until the host rejects the input.)
 __global__ void lcp_kernel(const uint8_t* __restrict__ keys, uint32_t n, int8_t* __restrict__ L, uint32_t* __restrict__ flags, int boundary) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i > n) return;
@@ -69,7 +71,11 @@ __global__ void lcp_kernel(const uint8_t* __restrict__ keys, uint32_t n, int8_t*
   ka[0] = __ldg(pa), ka[1] = __ldg(pa + 1), kb[0] = __ldg(pb), kb[1] = __ldg(pb + 1);
   int cmp;
   int l = lcp_nibbles(ka, kb, &cmp);
-  if (cmp >= 0) atomicOr(flags, 1u);
+  if (cmp >= 0) atomicOr(flags, BUILD_F_UNSORTED);
+  if (boundary >= 0 && l <= boundary) {
+    atomicOr(flags, BUILD_F_PREFIX);
+    l = boundary + 1;
+  }
   L[i] = (int8_t)(l > 63 ? 63 : l);
 }
 
@@ -279,6 +285,7 @@ __global__ void __launch_bounds__(B, 4) hash_sorted_leaves_kernel(BuildView V) {
     payload = hex_prefix_str_size(nib_len) + vhdr + vlen;
     total = len_prefix_size(payload) + payload;
     nunit = 1 + ((vlen + 127) >> 7);
+    if (is_root && V.base_depth > 0 && total < 32) atomicOr(V.flags, BUILD_F_SHORT_TOP);
   }
   const bool inline_ref = !is_root && total < 32;
   Stage<B> s;
@@ -425,6 +432,8 @@ __global__ void __launch_bounds__(B, 4) hash_branch_level_kernel(BuildView V, co
         inline_ref_words(s, total, rx, ry);
         rlen = total;
       } else {
+        // (total < 32 here only for the root's last message; a sub-trie's parent would embed it, not its hash)
+        if (total < 32 && V.base_depth > 0) atomicOr(V.flags, BUILD_F_SHORT_TOP);
         last = s.bytes() < 136;
         if (last) s.pad();
         absorb_stage<B>(a, s);

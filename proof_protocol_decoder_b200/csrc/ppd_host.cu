@@ -863,7 +863,8 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   CUDA_OK(cudaMemcpyAsync(&h_flags, small, 4, cudaMemcpyDeviceToHost, st));
   CUDA_OK(cudaMemcpyAsync(&nb, bidx + n, 4, cudaMemcpyDeviceToHost, st));
   CUDA_OK(cudaStreamSynchronize(st));
-  if (h_flags & 1) fail(PPD_ERR_UNSORTED_KEYS, "keys are not strictly ascending");
+  if (h_flags & BUILD_F_UNSORTED) fail(PPD_ERR_UNSORTED_KEYS, "keys are not strictly ascending");
+  if (h_flags & BUILD_F_PREFIX) fail(PPD_ERR_BAD_ARGUMENT, "the keys of a sub-trie do not share their first base_depth nibbles");
   c->stats.kernel_launches += 11 + 3;
 
   D[B_DEPTH].reserve(2ull * nb + 64);
@@ -886,7 +887,8 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   V.rep = D[B_REP].as<uint32_t>();
   V.child = D[B_CHILD].as<uint32_t>();
   V.root_id = small + 1;
-  V.ref = c->d_ref.as<uint8_t>();
+  V.flags = small + 0;
+  V.ref =c->d_ref.as<uint8_t>();
   V.ref_len = c->d_ref_len.as<uint8_t>();
   V.root_out = reinterpret_cast<uint8_t*>(small + 8);
   V.counters = reinterpret_cast<unsigned long long*>(small + 2);
@@ -930,6 +932,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   uint32_t out[16];
   CUDA_OK(cudaMemcpyAsync(out, small, 64, cudaMemcpyDeviceToHost, st));
   CUDA_OK(cudaStreamSynchronize(st));
+  if (out[0] & BUILD_F_SHORT_TOP) fail(PPD_ERR_BAD_ARGUMENT, "the sub-trie's top node encodes to fewer than 32 bytes: its parent embeds it, not its hash");
   memcpy(root_out, out + 8, 32);
   float ms = 0;
   CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));

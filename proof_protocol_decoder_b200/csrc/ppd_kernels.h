@@ -36,6 +36,13 @@ struct Pyramid {
   const int8_t *L, *m1, *m2, *m3;
 };
 
+// bits of the builder's flags word: checked by the host after the LCP pass (the first two) and after hashing (the last)
+enum : uint32_t {
+  BUILD_F_UNSORTED = 1,   // keys not strictly ascending
+  BUILD_F_PREFIX = 2,     // sub-trie: two adjacent keys share fewer than base_depth nibbles
+  BUILD_F_SHORT_TOP = 4,  // sub-trie: the top node encodes to fewer than 32 bytes (the parent embeds it, not its hash)
+};
+
 struct BuildView {
   const uint8_t* keys;       // [N][32]
   const uint64_t* val_off;   // [N+1]
@@ -51,6 +58,7 @@ struct BuildView {
   uint32_t* rep;             // [B]  an item below the branch
   uint32_t* child;           // [B][16]
   uint32_t* root_id;         // id of the root node (leaf or branch)
+  uint32_t* flags;           // BUILD_F_* (atomicOr)
   // results
   uint8_t* ref;              // [N + B][32]
   uint8_t* ref_len;          // [N + B]

@@ -1,7 +1,7 @@
 """Differential tests on drawn blocks (hypothesis): three implementations that share no code for the trie mutations.
 
   model    the final state as the GENERATOR tracked it (plain dicts), hashed as the canonical Merkle-Patricia trie of its
-           items by a recursive pure-Python builder: no insert, no delete, no collapse rule — a trie's shape is a function
+           items by a recursive pure-Python builder (trie_model.py): no insert, no delete, no collapse rule — a trie's shape is a function
            of its key set, so whatever sequence of inserts / deletes (with branch collapse, extension merge) led there must
            hash to the same root;
   oracle   the CPU restatement of the reference (insert / delete on pointer tries, per-txn subsets);
@@ -15,47 +15,9 @@ from hypothesis import HealthCheck, given, settings
 from hypothesis import strategies as st
 
 from proof_protocol_decoder_b200 import flat, synth
+from trie_model import trie_root
 
-EMPTY_TRIE_HASH = synth.keccak256(b"\x80")
 EMPTY_CODE_HASH = synth.keccak256(b"")
-
-
-def _hp(nib, leaf):
-    flag = (2 if leaf else 0) + (len(nib) & 1)
-    out = [(flag << 4) | nib[0]] if len(nib) & 1 else [flag << 4]
-    rest = nib[1:] if len(nib) & 1 else nib
-    out += [(rest[i] << 4) | rest[i + 1] for i in range(0, len(rest), 2)]
-    return bytes(out)
-
-
-def _ref(raw):
-    return synth.rlp_str(synth.keccak256(raw)) if len(raw) >= 32 else raw
-
-
-def _build(items, depth):
-    """RLP of the canonical trie node over items [(nibbles, value)] that share their first `depth` nibbles"""
-    if len(items) == 1:
-        nib, val = items[0]
-        return synth.rlp_list([synth.rlp_str(_hp(nib[depth:], True)), synth.rlp_str(val)])
-    first, last = items[0][0], items[-1][0]
-    cp = depth
-    while first[cp] == last[cp]:
-        cp += 1
-    if cp > depth:
-        return synth.rlp_list([synth.rlp_str(_hp(first[depth:cp], False)), _ref(_build(items, cp))])
-    kids = []
-    for n in range(16):
-        sub = [it for it in items if it[0][depth] == n]
-        kids.append(_ref(_build(sub, depth + 1)) if sub else b"\x80")
-    return synth.rlp_list(kids + [b"\x80"])
-
-
-def trie_root(pairs):
-    """root of the trie of {32-byte key: value bytes}"""
-    if not pairs:
-        return EMPTY_TRIE_HASH
-    items = sorted(([x for b in k for x in (b >> 4, b & 15)], v) for k, v in pairs.items())
-    return synth.keccak256(_build(items, 0))
 
 
 def model_state_root(blk):

@@ -229,10 +229,12 @@ def test_unsorted_keys_are_rejected(ctx):
     from proof_protocol_decoder_b200 import PpdError, synth
 
     keys, val_off, vals = synth.gen_sorted_leaves(100, seed=9)
-    keys = keys[::-1].copy()
-    with pytest.raises(PpdError) as e:
-        ctx.trie_root_sorted_leaves(keys, val_off, vals)
-    assert e.value.code == 63
+    duplicated = keys.copy()
+    duplicated[51] = duplicated[50]  # still ascending, but one key twice
+    for bad in (keys[::-1].copy(), duplicated):
+        with pytest.raises(PpdError) as e:
+            ctx.trie_root_sorted_leaves(bad, val_off, vals)
+        assert e.value.code == 63
 
 
 def test_sorted_leaves_root_one_million(ctx, oracle):
