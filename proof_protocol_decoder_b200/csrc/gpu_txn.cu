@@ -193,6 +193,7 @@ struct HookState {
   TxnTables* T;
   const uint8_t* d_flat;
   size_t n_txns;
+  const PVec<H256>* keep;  // a direct pre-image: the hashed addresses of its storage map (page-locked), else null
   // out
   TxnBases B{};
   txn::View v{};
@@ -227,8 +228,9 @@ void after_emit(void* arg, const ParseEmit& E) {
   // ---- device memory of the loop ----
   uint32_t table = 64;
   while (table < 2 * n_traces) table <<= 1;
+  const size_t n_keep = H.keep ? H.keep->size() : 0;
   uint32_t jtable = 64;
-  while (jtable < 2 * n_acct) jtable <<= 1;
+  while (jtable < 2 * std::max(n_acct, n_keep)) jtable <<= 1;
   H.table_slots = table;
   txn::View& v = H.v;
   txn::JoinView& j = H.j;
@@ -247,6 +249,7 @@ void after_emit(void* arg, const ParseEmit& E) {
     j.join_storage = c.take<uint32_t>(n_acct + 1);
     j.join_root = c.take<uint32_t>(n_acct + 1);
     j.pre_flags = c.take<uint8_t>(n_acct + 1);
+    j.keep = H.keep ? c.take<uint8_t>(32 * n_keep + 32) : nullptr;
     v.pre_slot = c.take<uint32_t>(n_acct + 1);
     H.d_withdrawals = c.take<txn::Withdrawal>(T.withdrawals.size() + 1);
     H.d_export = c.take<txn::AcctExport>(T.needs_dummies() ? n_acct + 1 : 1);
@@ -289,6 +292,11 @@ void after_emit(void* arg, const ParseEmit& E) {
   // (tables and read-backs go by kernel copy, lane_copy: the copy engines are left to the FlatBlock and the IrDump)
   lane_copy(L, H.d_withdrawals, T.withdrawals.data(), sizeof(txn::Withdrawal) * v.n_withdrawals);
   j.acct_list = E.acct_list, j.n_acct = (uint32_t)n_acct, j.table_mask = jtable - 1;
+  if (H.keep) {
+    j.n_keep = (uint32_t)n_keep;
+    lane_copy(L, const_cast<uint8_t*>(j.keep), H.keep->data(), 32 * n_keep);
+    L->stats.h2d_bytes += 32.0 * n_keep;
+  }
   // ---- the byte strings to hash: straight out of the resident FlatBlock ----
   lane_copy(L, v.traces, T.traces.data(), sizeof(txn::TxnTrace) * n_traces);
   lane_copy_flush(L);
@@ -340,21 +348,37 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
   cudaStream_t st = L->st;
   const ppd_stats stats0 = L->stats;
   // ---- the FlatBlock to the device; the witness inside it lands 256-byte aligned ----
-  const size_t wit_off = (size_t)(b.compact.p - flat);
-  const size_t lead = (256 - (wit_off & 255)) & 255;
-  L->d_flat.reserve(lead + len + 512);
+  // A direct pre-image (kind 2) was re-spelled as a witness in the job's page-locked buffer: the witness gets a region of
+  // its own after the FlatBlock, and of the FlatBlock only what follows the DirectPreImage payload goes up.  Nothing on
+  // the device reads the payload or the header before it (every offset of the tables points past them), so the
+  // pre-image crosses PCIe once.
+  const bool direct = b.pre_image_kind == 2;
+  const size_t up_from = direct ? (size_t)(b.direct.p - flat) + b.direct.n : 0;
+  const size_t wit_off = direct ? (len + 256 + 255) & ~(size_t)255 : (size_t)(b.compact.p - flat);
+  const size_t lead = direct ? 0 : (256 - (wit_off & 255)) & 255;
+  L->d_flat.reserve(lead + (direct ? wit_off + b.compact.n + 256 : len + 512));
   uint8_t* d_flat = L->d_flat.as<uint8_t>() + lead;
+  if (direct) {
+    J.direct_keep.resize(b.direct_keep.size());
+    if (!b.direct_keep.empty()) memcpy(J.direct_keep.data(), b.direct_keep.data(), sizeof(H256) * b.direct_keep.size());
+  }
   L->tr_n = 0;
   trace_mark(L, "begin");
-  upload_bytes(L, J, d_flat, flat, len);
-  trace_mark(L, "uploaded");
+  upload_bytes(L, J, d_flat + up_from, flat + up_from, len - up_from);
   CUDA_OK(cudaMemsetAsync(d_flat + len, 0, 256, st));
-  L->stats.h2d_bytes += (double)len;
+  L->stats.h2d_bytes += (double)(len - up_from);
+  if (direct) {
+    // (page-locked: the copy engine reads it as it is; J.wit_stage may still feed the FlatBlock's copy)
+    CUDA_OK(cudaMemcpyAsync(d_flat + wit_off, b.compact.p, b.compact.n, cudaMemcpyHostToDevice, st));
+    CUDA_OK(cudaMemsetAsync(d_flat + wit_off + b.compact.n, 0, 256, st));
+    L->stats.h2d_bytes += (double)b.compact.n;
+  }
+  trace_mark(L, "uploaded");
   // page-locked landing areas
   const size_t h_words = 2 * ORDER_MAX_BINS + sizeof(txn::Cursors) / 4 + 64;
   J.txn_host.resize(h_words + 8 * T.code_write_traces.size() + 8);
   HookState H;
-  H.L = L, H.J = &J, H.T = &T, H.d_flat = d_flat, H.n_txns = b.txns.size();
+  H.L = L, H.J = &J, H.T = &T, H.d_flat = d_flat, H.n_txns = b.txns.size(), H.keep = direct ? &J.direct_keep : nullptr;
   H.h_bins = J.txn_host.data();
   H.h_code_digests = reinterpret_cast<uint8_t*>(J.txn_host.data() + h_words);
   PreImageDeviceOnly X{};
@@ -385,7 +409,9 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
     CD* x = (CD*)arg;
     return x->H->h_code_digests + 32ull * x->slot_of[t];
   };
-  if (!txn_tables_phase2(b, flat, H.B, code_digest, &cd, T)) {
+  // (the plan copies code bytes out of the resident FlatBlock: a re-spelled witness has no code strings, so a direct
+  // pre-image's code comes from the resolved-code table, which is inside it)
+  if ((direct && !b.pre_code.empty()) || !txn_tables_phase2(b, flat, H.B, code_digest, &cd, T)) {
     L->stats = stats0;
     return GPU_BLOCK_DECLINED;
   }
@@ -480,7 +506,7 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
   }
   CUDA_OK(cudaEventRecord(L->ev1, st));
   trace_mark(L, "pre_hashed");
-  // ---- join, account table, sorted ops, the loop ----
+  // ---- join (by root, or by address for a direct pre-image), account table, sorted ops, the loop ----
   H.j.ref = V.ref;
   CUDA_OK(cudaMemsetAsync(H.j.slot_owner, 0xff, 4ull * (H.j.table_mask + 1), st));
   CUDA_OK(cudaMemsetAsync(H.j.slot_best, 0, 4ull * (H.j.table_mask + 1), st));
@@ -491,7 +517,10 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
   init.state_root = b.state_root, init.txn_root = NODE_EMPTY, init.receipt_root = NODE_EMPTY;
   launch_txn_init(v, init, H.table_slots, st);
   H.j.flag = &v.cur->flag;
-  launch_join(H.j, st);
+  if (direct)
+    launch_join_by_address(v, H.j, st);
+  else
+    launch_join(H.j, st);
   H.ai = txn::AcctInit{H.table_slots - 1, b.state_root, H.j.join_storage, H.j.join_root};
   const uint32_t max_writes = T.max_trace_keys;
   L->stats.kernel_launches += 3 + launch_txn_prep(v, H.ai, T.n_ops1, T.n_ops2, max_writes, st);

@@ -5,16 +5,17 @@
 // and extra_code_hash_mappings is None (:139); process_multiple_storage_tries is todo!() (:164-168).  Kind 2 completes
 // it the way process_state_trie is written: every entry of the map is the trie it holds, keyed by hashed address.
 //
-// Nothing new runs for it on the device.  A direct pre-image is the SAME tree the compact witness spells in
-// post-order, so the host re-spells it: one pass over the pre-order Node form (include/ppd_flat.h) writes the
-// witness opcodes of compact_prestate_processing.rs:744-875 -- a hashed-out node as HASH, a branch as its children then
-// BRANCH(mask), an account leaf as [HASH(code hash)] [its storage trie | HASH(storage root)] ACCOUNT_LEAF(key, flags,
-// nonce, balance) -- and the block then takes the witness path: GPU parse, GPU hashing, GPU IR dump.  Structure
-// only: no hashing here.
+// A direct pre-image is the SAME tree the compact witness spells in post-order, so the host re-spells it: one pass
+// over the pre-order Node form (include/ppd_flat.h) writes the witness opcodes of compact_prestate_processing.rs:744-875
+// -- a hashed-out node as HASH, a branch as its children then BRANCH(mask), an account leaf as [HASH(code hash)] [its
+// storage trie | HASH(storage root)] ACCOUNT_LEAF(key, flags, nonce, balance) -- and the block then takes the witness
+// path: GPU parse, GPU hashing, the device txn loop, GPU IR dump.  Structure only: no hashing here.  The witness is
+// written into a caller-owned buffer (page-locked for a decode: the copy engine reads it as it is).
 //
 // What differs from a Combined pre-image is WHICH accounts have a storage trie: by hashed address as given, not by
-// root hash (compact_to_partial_trie.rs:167-190).  `direct_keep` records the addresses of the map; the caller drops
-// every other entry after the pre-image is built and skips the by-root join.
+// root hash (compact_to_partial_trie.rs:167-190).  `direct_keep` records the addresses of the map.  The device txn loop
+// joins accounts to tries by these addresses (ppd_txn.cu: join_addr_*_kernel); the host path drops every other entry
+// after the pre-image is built (direct_filter_storage) and skips the by-root join.
 //
 // Preconditions (a pre-image a tracer would send meets them; an input that does not is rejected with
 // PPD_ERR_BAD_FLAT_INPUT, or noted): every state leaf is an RLP account (else PPD_PANIC_PRE_IMAGE_ACCOUNT_DECODE, as
@@ -30,7 +31,7 @@ namespace {
 
 struct DirectEncoder {
   FlatReader r;
-  std::vector<uint8_t>& out;
+  PVec<uint8_t>& out;
   std::unordered_map<H256, std::pair<size_t, bool>, H256Hasher> storage_at;  // hashed address -> (offset of its trie, used)
   uint8_t path[160];
 
@@ -48,7 +49,7 @@ struct DirectEncoder {
   }
   void cbor_bytes(const uint8_t* p, size_t n) {
     cbor_head(2, n);
-    out.insert(out.end(), p, p + n);
+    out.append(p, n);
   }
   // the inverse of key_bytes_to_nibbles (compact_prestate_processing.rs:1338-1390): a flag byte (bit 0: odd count), then
   // the nibbles packed high first
@@ -108,7 +109,7 @@ struct DirectEncoder {
       case PPD_NODE_HASH: {
         const uint8_t* h = r.raw(32);
         out.push_back(PPD_OP_HASH);
-        out.insert(out.end(), h, h + 32);
+        out.append(h, 32);
         return true;
       }
       case PPD_NODE_BRANCH: {
@@ -180,7 +181,7 @@ struct DirectEncoder {
     if (memcmp(f[3].payload, EMPTY_CODE_HASH, 32) != 0) {
       flags |= 1;
       out.push_back(PPD_OP_HASH);
-      out.insert(out.end(), f[3].payload, f[3].payload + 32);
+      out.append(f[3].payload, 32);
     }
     auto s = storage_at.find(haddr);
     if (s != storage_at.end()) {
@@ -198,7 +199,7 @@ struct DirectEncoder {
     } else if (memcmp(f[2].payload, EMPTY_TRIE_HASH, 32) != 0) {
       flags |= 2;  // storage that was not sent: the root alone
       out.push_back(PPD_OP_HASH);
-      out.insert(out.end(), f[2].payload, f[2].payload + 32);
+      out.append(f[2].payload, 32);
     }
     if (nonce) flags |= 4;
     if (f[1].payload_len) flags |= 8;
@@ -213,10 +214,10 @@ struct DirectEncoder {
 
 }  // namespace
 
-void direct_to_compact(BlockJob& b) {
-  b.compact_owned.clear();
-  b.compact_owned.reserve((size_t)b.direct.n + (size_t)b.direct.n / 8 + 64);
-  DirectEncoder e{FlatReader{b.direct.p, b.direct.n}, b.compact_owned, {}, {}};
+void direct_to_compact(BlockJob& b, PVec<uint8_t>& wit) {
+  wit.clear();
+  wit.reserve((size_t)b.direct.n + (size_t)b.direct.n / 8 + 64);
+  DirectEncoder e{FlatReader{b.direct.p, b.direct.n}, wit, {}, {}};
   // where every storage trie starts
   e.skip(0);
   const uint32_t ns = e.r.u32();
@@ -240,8 +241,9 @@ void direct_to_compact(BlockJob& b) {
     if (!s.second.second) e.bad("a storage trie for an account the state trie does not hold");
   if (e.out.size() >= 0xfff00000ull) e.bad("too large");
   const size_t n = e.out.size();
-  e.out.resize(n + 64, 0);  // readable past the end, like every witness buffer
-  b.compact = Span{b.compact_owned.data(), (uint32_t)n};
+  e.out.resize(n + 64);
+  memset(e.out.data() + n, 0, 64);  // readable past the end, like every witness buffer
+  b.compact = Span{e.out.data(), (uint32_t)n};
 }
 
 // after the pre-image is built: the accounts that have a storage trie are those of the map (by hashed address)
@@ -259,8 +261,9 @@ extern "C" int ppd_direct_to_compact(const uint8_t* direct, size_t len, uint8_t*
   if (len > 0xfff00000ull) return PPD_ERR_BAD_FLAT_INPUT;
   try {
     ppd::BlockJob b;
+    ppd::PVec<uint8_t> wit;
     b.direct = ppd::Span{direct, (uint32_t)len};
-    ppd::direct_to_compact(b);
+    ppd::direct_to_compact(b, wit);
     uint8_t* p = (uint8_t*)malloc(b.compact.n ? b.compact.n : 1);
     if (!p) return PPD_ERR_BAD_ARGUMENT;
     memcpy(p, b.compact.p, b.compact.n);

@@ -469,8 +469,7 @@ struct BlockJob {
   // input views
   Span compact;
   uint32_t pre_image_kind = 0;         // 0 Combined{compact}; 2 Separate{Direct, MultipleTries{Direct}} (host_direct.cu)
-  Span direct;                         // kind 2: the DirectPreImage payload; `compact` then points into compact_owned
-  std::vector<uint8_t> compact_owned;  // kind 2: the pre-image re-spelled as a compact witness
+  Span direct;                         // kind 2: the DirectPreImage payload; `compact` then points into Job::direct_wit
   std::vector<H256> direct_keep;       // kind 2: the hashed addresses that have a storage trie
   std::vector<TxnV> txns;
   std::unordered_map<H256, Span, H256Hasher> resolved_code;
@@ -510,8 +509,9 @@ struct BlockJob {
 };
 
 void read_flat_block(const uint8_t* p, size_t n, BlockJob& b);
-// host_direct.cu: a kind-2 pre-image as a compact witness (b.compact, b.direct_keep); the storage map cut to b.direct_keep
-void direct_to_compact(BlockJob& b);
+// host_direct.cu: a kind-2 pre-image as a compact witness written into `wit` (b.compact points there; b.direct_keep); the
+// storage map cut to b.direct_keep
+void direct_to_compact(BlockJob& b, PVec<uint8_t>& wit);
 void direct_filter_storage(BlockJob& b);
 // ---- minimal RLP helpers (structure only; no hashing): host_txn.cu ----
 uint32_t u256_sig(const uint8_t* be);
@@ -546,6 +546,10 @@ struct Job {
   bool pools_on_host = true;
   PVec<uint32_t> acct_list, code_list;
   PVec<uint8_t> wit_stage;  // page-locked staging of a pageable witness
+  // a kind-2 block's pre-image re-spelled as a witness (host_direct.cu), and the hashed addresses of its storage map
+  // as the device's by-address join reads them: page-locked, read by the copy engine / copy kernel directly
+  PVec<uint8_t> direct_wit;
+  PVec<H256> direct_keep;
   std::vector<HostArena::MarkItem> mark_items;  // scratch of the txn loop
   std::vector<HostArena::BatchItem> batch_items;
   std::vector<uint32_t> haddr_keys, haddr_leaves;
@@ -567,6 +571,7 @@ struct Job {
     acct_list.alloc_fn = code_list.alloc_fn = pinned_alloc, acct_list.free_fn = code_list.free_fn = pinned_free;
     code_digest.alloc_fn = pinned_alloc, code_digest.free_fn = pinned_free;
     wit_stage.alloc_fn = pinned_alloc, wit_stage.free_fn = pinned_free;
+    direct_wit.alloc_fn = direct_keep.alloc_fn = pinned_alloc, direct_wit.free_fn = direct_keep.free_fn = pinned_free;
     txn.set_allocator(pinned_alloc, pinned_free);
     txn_host.alloc_fn = pinned_alloc, txn_host.free_fn = pinned_free;
     txn_export.alloc_fn = pinned_alloc, txn_export.free_fn = pinned_free;

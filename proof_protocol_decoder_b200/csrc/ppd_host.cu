@@ -398,6 +398,10 @@ void decode_one_inner(ppd_ctx* c, Lane* L, const uint8_t* flat, size_t len, uint
   // would report, a witness the GPU parser hands to the host builder, a capacity limit) starts over on the host path:
   // the host shapes the tries, in the reference's order of operations, and the device hashes and serialises them.
   StreamLease lease(c->pool, L);
+  // a direct pre-image (kind 2) is re-spelled as a witness once, into the job's page-locked buffer; a block the device
+  // declines keeps it (and its map's addresses) for the host attempt
+  Span respelled{};
+  std::vector<H256> keep;
   for (int on_device = gpu_txn_enabled() ? 1 : 0; on_device >= 0; on_device--) {
     PhaseTimer pt;
     Job& J = job_of(L, 1);
@@ -406,17 +410,19 @@ void decode_one_inner(ppd_ctx* c, Lane* L, const uint8_t* flat, size_t len, uint
       read_flat_block(flat, len, b);
       pt.lap("read-flat");
       if (b.pre_image_kind == 2) {
-        // a direct pre-image is re-spelled as a witness on the host; its storage map is by address, which the
-        // device path's by-root join does not express: the host-shaped path takes it
-        if (on_device) continue;
-        direct_to_compact(b);
-        pt.lap("direct");
+        if (!respelled.p) {
+          direct_to_compact(b, J.direct_wit);
+          pt.lap("direct");
+        } else {
+          b.compact = respelled, b.direct_keep.swap(keep);
+        }
       }
       if (on_device) {
         if (gpu_block(c, L, J, flat, len, out, out_len) == GPU_BLOCK_DONE) {
           *status = PPD_OK;
           return;
         }
+        if (b.pre_image_kind == 2) respelled = b.compact, keep.swap(b.direct_keep);
         continue;
       }
       if (gpu_parse_enabled()) gpu_pre_image(L, J, b, true, &c->parse_slots_sem);
@@ -630,7 +636,7 @@ int ppd_keccak256_batch(ppd_ctx* c, const uint8_t* data, const uint64_t* offsets
 // pipeline order on its own stream, lanes concurrently, as in the call itself:
 //   PPD_REPLAY_PARSE  witness parse + pre-image arena (ppd_parse.cu)
 //   PPD_REPLAY_HASH   key hashing and the level sweeps (ppd_kernels.cu); with TXN, the loop runs between the two sweeps
-//   PPD_REPLAY_TXN    by-root join, account table, op sort, the txn loop, the order of its nodes (ppd_txn.cu)
+//   PPD_REPLAY_TXN    join (by root or by address), account table, op sort, the txn loop, the order of its nodes (ppd_txn.cu)
 //   PPD_REPLAY_DUMP   IR sizing and emit (ppd_dump.cu)
 // TXN and DUMP exist for lanes whose block took the device txn loop (gpu_txn.cu).
 static void replay_lane(Lane* L, unsigned what) {
@@ -668,7 +674,10 @@ static void replay_lane(Lane* L, unsigned what) {
     CUDA_OK(cudaMemsetAsync(L->last_join.slot_best, 0, 4ull * (L->last_join.table_mask + 1), st));
     CUDA_OK(cudaMemsetAsync(v.pre_slot, 0xff, 4ull * (L->last_join.n_acct + 1), st));
     launch_txn_init(v, L->last_init, L->last_table_slots, st);
-    launch_join(L->last_join, st);
+    if (L->last_join.keep)  // the lane's last block was a direct pre-image: its map's addresses are still resident
+      launch_join_by_address(v, L->last_join, st);
+    else
+      launch_join(L->last_join, st);
     launch_txn_prep(v, L->last_ai, L->last_n_ops1, L->last_n_ops2, L->last_max_writes, st);
     launch_txn_loop(L->h_task, v, L->last_init.state_root, L->last_max_keys, st);
     CUDA_OK(cudaMemsetAsync(L->last_bins_tail, 0, 4ull * ORDER_MAX_BINS, st));

@@ -196,6 +196,8 @@ void launch_parse_emit(const ParseEmit& E, cudaStream_t st);
 void launch_txn_msgs(const txn::View& v, uint64_t* se, cudaStream_t st);
 void launch_txn_init(const txn::View& v, const txn::Cursors& init, uint32_t table_slots, cudaStream_t st);
 void launch_join(const txn::JoinView& j, cudaStream_t st);
+// direct pre-images (j.keep set): the by-address join; slot_owner / slot_best cleared as for launch_join
+void launch_join_by_address(const txn::View& v, const txn::JoinView& j, cudaStream_t st);
 uint32_t launch_txn_prep(const txn::View& v, const txn::AcctInit& a, uint32_t n_ops1, uint32_t n_ops2, uint32_t max_writes, cudaStream_t st);
 // max_keys: the most keys (accessed + written) any txn of the block has; returns the number of launches
 // the loops of n blocks as one series of launches (one thread block per task; tasks: device-accessible, e.g. page-locked

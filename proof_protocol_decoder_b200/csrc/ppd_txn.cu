@@ -3,6 +3,7 @@
 //   txn_msgs_kernel      byte ranges of the FlatBlock to hash (addresses, slot keys, written code), one thread per trace
 //   join_*_kernel        convert_storage_trie_root_keyed_hashmap_to_account_addr_keyed (compact_to_partial_trie.rs:167-190):
 //                        accounts get the storage trie witnessed LAST under their storage root, whoever witnessed it
+//   join_addr_*_kernel   the same for a direct pre-image, whose storage map is by hashed address (txn_core.h)
 //   acct_claim_kernel    one table slot per distinct address; the account's entry in the initial PartialTrieState
 //   prep_*_kernel        ops of every txn sorted per trie (rank sort: batches are tens of keys, O(n^2) is parallel and tiny),
 //                        written values RLP-encoded into val_pool, LCPs of neighbours
@@ -91,6 +92,16 @@ __global__ void join_resolve_kernel(JoinView j) {
     h = (h + 1) & j.table_mask;
   }
   j.join_storage[r] = storage, j.join_root[r] = root;
+}
+
+// ---- the by-address join (direct pre-images; txn_core.h: join_addr_insert / join_addr_resolve) -------------------
+__global__ void join_addr_insert_kernel(JoinView j, uint32_t n) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) join_addr_insert(j, i);
+}
+__global__ void join_addr_resolve_kernel(View v, JoinView j) {
+  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < j.n_acct) join_addr_resolve(v, j, r);
 }
 
 __global__ void acct_claim_kernel(View v, AcctInit a) {
@@ -210,6 +221,12 @@ void launch_join(const JoinView& j, cudaStream_t st) {
   if (!j.n_acct) return;
   join_insert_kernel<<<cdiv(j.n_acct, 128), 128, 0, st>>>(j);
   join_resolve_kernel<<<cdiv(j.n_acct, 128), 128, 0, st>>>(j);
+}
+void launch_join_by_address(const View& v, const JoinView& j, cudaStream_t st) {
+  if (!j.n_acct) return;
+  const uint32_t n = j.n_keep > j.n_acct ? j.n_keep : j.n_acct;
+  join_addr_insert_kernel<<<cdiv(n, 128), 128, 0, st>>>(j, n);
+  join_addr_resolve_kernel<<<cdiv(j.n_acct, 128), 128, 0, st>>>(v, j);
 }
 uint32_t launch_txn_prep(const View& v, const AcctInit& a, uint32_t n_ops1, uint32_t n_ops2, uint32_t max_writes, cudaStream_t st) {
   uint32_t launches = 0;

@@ -259,6 +259,10 @@ struct JoinView {
   uint32_t* join_root;        // [n_acct] out
   uint8_t* pre_flags;         // [n_acct] out
   uint32_t* flag;             // &Cursors::flag
+  // the by-address join of a direct pre-image (FlatBlock kind 2) instead, when keep is set: the hashed addresses of its
+  // storage map; slot_owner then holds map indices, slot_best[0] 1 + the last account whose witnessed trie is empty
+  const uint8_t* keep;        // [n_keep][32], or null
+  uint32_t n_keep;
 };
 
 PPD_HD PPD_INLINE bool is_hash_id(uint32_t n) { return n >= HASH_BASE && n < HASH_END; }
@@ -1240,6 +1244,64 @@ PPD_HD PPD_INLINE void acct_claim(const View& v, const AcctInit& a, uint32_t t) 
     }
     h = (h + 1) & a.table_mask;
   }
+}
+
+// ---- the by-address join of a direct pre-image (kind 2, host_direct.cu) -------------------------------------------
+// The storage map of a Separate pre-image is keyed by hashed address: an account has a storage trie iff its address is
+// in the map, and then it is the trie sent for it (its own, in the re-spelled witness).  This is the map the host path
+// builds (build_pre_image, then direct_filter_storage), account by account:
+//   not in the map                      ST_ABSENT / NONE, even when its root is that of a trie in the map
+//   in the map, trie not empty          its own trie (a bare hash node included) and its NK_ROOT node
+//   in the map, trie empty (its root is EMPTY_TRIE_HASH: an empty trie, or a hash node of that root)
+//                                       the empty-rooted trie witnessed LAST (the host builder's empty form) / NONE
+// Every account keeps a trie of its own or the empty form, so this join never shares an expanded trie.
+PPD_HD PPD_INLINE uint32_t addr_slot_hash(const uint8_t* k, uint32_t mask) {
+  return ((uint32_t)k[8] | ((uint32_t)k[9] << 8) | ((uint32_t)k[10] << 16) | ((uint32_t)k[11] << 24)) & mask;
+}
+PPD_HD PPD_INLINE bool eq32(const uint8_t* a, const uint8_t* b) {
+  bool same = true;
+  for (int i = 0; i < 32; i++) same &= a[i] == b[i];
+  return same;
+}
+// thread i: map entry i into the table; account i, if its witnessed storage trie is empty, into the empty-form cell
+PPD_HD PPD_INLINE void join_addr_insert(const JoinView& j, uint32_t i) {
+  if (i < j.n_acct && (j.acct_list[5ull * i + 3] & 3u) == 1u) PPD_ATOMIC_MAX(&j.slot_best[0], i + 1u);
+  if (i >= j.n_keep) return;
+  const uint8_t* key = j.keep + 32ull * i;
+  uint32_t h = addr_slot_hash(key, j.table_mask);
+  for (;;) {
+    const uint32_t prev = PPD_ATOMIC_CAS(&j.slot_owner[h], 0xffffffffu, i);
+    if (prev == 0xffffffffu || eq32(j.keep + 32ull * prev, key)) return;  // (the map has no duplicates: host_direct.cu)
+    h = (h + 1) & j.table_mask;
+  }
+}
+// account r: its hashed address from its leaf key, right-aligned as export_account assembles it (utils.rs:49-59)
+PPD_HD PPD_INLINE void join_addr_resolve(const View& v, const JoinView& j, uint32_t r) {
+  const uint32_t* al = j.acct_list + 5ull * r;
+  const NodeRec nr = v.nodes[al[0]];
+  const uint32_t ns = (nr.w0 >> 8) & 0xffu, nl = (nr.w0 >> 16) & 0xffu, klen = ns + nl;
+  uint8_t haddr[32];
+  for (int i = 0; i < 32; i++) haddr[i] = 0;
+  for (uint32_t k = 0; k < klen && k < 64; k++) {
+    const uint32_t posn = 64 - klen + k, nib = key_nib(v, nr.a0, k);
+    haddr[posn >> 1] |= (uint8_t)((posn & 1) ? nib : (nib << 4));
+  }
+  const uint32_t flags = al[3];
+  j.pre_flags[r] = (uint8_t)((flags >> 1) & 1u);
+  uint32_t storage = ST_ABSENT, root = NONE;
+  for (uint32_t h = addr_slot_hash(haddr, j.table_mask);; h = (h + 1) & j.table_mask) {
+    const uint32_t own = j.slot_owner[h];
+    if (own == 0xffffffffu) break;
+    if (!eq32(j.keep + 32ull * own, haddr)) continue;
+    if (flags & 2u) {
+      storage = al[1], root = al[2] == NODE_EMPTY ? NONE : al[2];
+    } else {
+      const uint32_t last = j.slot_best[0];
+      if (last) storage = j.acct_list[5ull * (last - 1u) + 1];
+    }
+    break;
+  }
+  j.join_storage[r] = storage, j.join_root[r] = root;
 }
 
 // ---- the loop itself: one thread block per block of txns (the harness runs it as a block of one thread) ------
