@@ -144,6 +144,22 @@ int ppd_trie_root_sorted_leaves(ppd_ctx* ctx, const uint8_t* keys32, const uint6
 int ppd_trie_root_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals,
                                     size_t n, size_t vals_bytes, uint8_t root_out[32]);
 
+#define PPD_LEAVES_HASH_KEYS 1u /* key i is keccak256(keys[i*key_len .. +key_len)), not the bytes themselves */
+/* HashedPartialTrie::hash() of the trie obtained by inserting (key_0, val_0) ... (key_{n-1}, val_{n-1}) in this order
+ * into an empty trie (eth_trie_utils `insert`, compact_to_partial_trie.rs:105,125): any key order, and a repeated key
+ * keeps the value of its LAST occurrence.  Without PPD_LEAVES_HASH_KEYS key_len must be 32; with it, 1 <= key_len <= 135
+ * (20: addresses, 32: slots).  Values as for ppd_trie_root_sorted_leaves (already-RLP-encoded payloads, taken as given).
+ * Inputs are only read, never reordered in place.  Never returns PPD_ERR_UNSORTED_KEYS.  PPD_ERR_BAD_ARGUMENT for unknown
+ * flag bits, a bad key_len, n >= 2^31 - 2, or val_off decreasing anywhere or ending past vals_bytes.  The leaves are
+ * sorted, de-duplicated and gathered on the GPU (csrc/ppd_leaves.cu), then built as by the sorted entry.
+ * DEVICE pointers, complete when the call is made (the library reads them on a stream of its own); vals_bytes =
+ * readable bytes of d_vals. */
+int ppd_trie_root_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off,
+                             const uint8_t* d_vals, size_t n, size_t vals_bytes, uint8_t root_out[32]);
+/* The same from host buffers. */
+int ppd_trie_root_leaves(ppd_ctx* ctx, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off,
+                         const uint8_t* vals, size_t n, uint8_t root_out[32]);
+
 /* One huge trie over several streams or GPUs (SURVEY.md 8e (3)): the leaves are split by their first `base_depth`
  * nibbles; each part is hashed like a whole trie, except that its nodes sit `base_depth` nibbles below the root
  * (ref_out = the hash of the part's top node, the 32 bytes the node above embeds).  Every key of the part must share

@@ -233,6 +233,7 @@ struct ppd_ctx {
   ppd::DevBuf d_keys, d_vals, d_ref, d_ref_len, d_counters;
   ppd::DevBuf d_msg, d_msg_off, d_digest;
   ppd::DevBuf d_build[12];
+  ppd::DevBuf d_leaves[24];  // sort / de-duplication / gather of ppd_trie_root_leaves[_dev]
 };
 
 namespace ppd {

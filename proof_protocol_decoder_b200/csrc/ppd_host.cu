@@ -586,6 +586,7 @@ void ppd_ctx_destroy(ppd_ctx* c) {
   DevBuf* bufs[] = {&c->d_keys, &c->d_vals, &c->d_ref, &c->d_ref_len, &c->d_counters, &c->d_msg, &c->d_msg_off, &c->d_digest};
   for (DevBuf* b : bufs) b->release();
   for (DevBuf& b : c->d_build) b.release();
+  for (DevBuf& b : c->d_leaves) b.release();
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->st) cudaStreamDestroy(c->st);
@@ -956,6 +957,158 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   c->stats.d2h_bytes += 64 + 4096 + 8;
 }
 
+// ---- trie root over leaves in any order (ppd_leaves.cu): sort, keep the last of each key, gather, then the builder ----
+
+// byte digits of the n keys that take more than one value (bit p: digit p): the passes a sort cannot skip
+uint32_t varying_digits(ppd_ctx* c, const uint64_t* keys, uint32_t n, uint32_t* counts) {
+  CUDA_OK(cudaMemsetAsync(counts, 0, 8 * 256 * 4, c->st));
+  launch_digit_counts(keys, n, counts, c->st);
+  CUDA_OK(cudaGetLastError());
+  std::vector<uint32_t> h(8 * 256);
+  CUDA_OK(cudaMemcpyAsync(h.data(), counts, 8 * 256 * 4, cudaMemcpyDeviceToHost, c->st));
+  CUDA_OK(cudaStreamSynchronize(c->st));
+  c->stats.kernel_launches += 1;
+  c->stats.d2h_bytes += 8 * 256 * 4;
+  uint32_t mask = 0;
+  for (int p = 0; p < 8; p++)
+    if (std::find(h.begin() + 256 * p, h.begin() + 256 * (p + 1), n) == h.begin() + 256 * (p + 1)) mask |= 1u << p;
+  return mask;
+}
+
+// stable LSD radix sort of the pairs (k[in][i], v[in][i]) by key over the digits of `digits`; k[1 - in] / v[1 - in] are the
+// other halves of the ping-pong.  Returns which half holds the result.
+int sort_pairs(ppd_ctx* c, uint64_t* const k[2], uint32_t* const v[2], int in, uint32_t n, uint32_t digits, uint32_t* hist, uint32_t* tmp) {
+  for (int p = 0; p < 8; p++) {
+    if (!(digits & (1u << p))) continue;
+    c->stats.kernel_launches += launch_radix_pass(k[in], v[in], k[1 - in], v[1 - in], n, p, hist, hist + radix_hist_words(n), tmp, c->st);
+    in = 1 - in;
+  }
+  CUDA_OK(cudaGetLastError());
+  return in;
+}
+
+void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
+                          size_t n_, size_t vals_bytes, uint8_t root_out[32]) {
+  if (flags & ~PPD_LEAVES_HASH_KEYS) fail(PPD_ERR_BAD_ARGUMENT, "unknown flag bits");
+  const bool hash = flags & PPD_LEAVES_HASH_KEYS;
+  if (hash ? (key_len < 1 || key_len > 135) : key_len != 32)
+    fail(PPD_ERR_BAD_ARGUMENT, hash ? "hashed keys are 1 to 135 bytes long" : "keys are 32 bytes long unless PPD_LEAVES_HASH_KEYS is set");
+  if (n_ == 0) {
+    memcpy(root_out, EMPTY_TRIE_HASH, 32);
+    return;
+  }
+  if (n_ >= 0x7fffffffull) fail(PPD_ERR_BAD_ARGUMENT, "at most 2^31 - 2 leaves per call");
+  const uint32_t n = (uint32_t)n_;
+  cudaStream_t st = c->st;
+  enum { B_HKEYS, B_K0, B_K1, B_V0, B_V1, B_V2, B_TIE, B_MEMBER, B_MPOS, B_START, B_SPOS, B_CPOS, B_CIDX, B_CRUN, B_CWORD,
+         B_LEN, B_KOFF, B_HIST, B_TMP, B_TMP64, B_SMALL, B_OKEYS, B_OOFF, B_OVALS };
+  DevBuf* D = c->d_leaves;
+  const size_t hist_words = radix_hist_words(n);
+  for (int b : {B_K0, B_K1, B_CWORD}) D[b].reserve(8ull * n);
+  for (int b : {B_V0, B_V1, B_V2, B_CPOS, B_CIDX, B_CRUN}) D[b].reserve(4ull * n);
+  for (int b : {B_TIE, B_MEMBER, B_MPOS, B_START, B_SPOS}) D[b].reserve(4ull * (n + 1));
+  for (int b : {B_LEN, B_KOFF}) D[b].reserve(8ull * (n + 1));
+  D[B_HIST].reserve(4 * 2 * hist_words);
+  D[B_TMP].reserve(4 * scan_tmp_words(std::max<size_t>(hist_words, (size_t)n + 1)));
+  D[B_TMP64].reserve(8 * scan_tmp_words((size_t)n + 1));
+  D[B_SMALL].reserve(16384);
+  uint32_t* small = D[B_SMALL].as<uint32_t>();  // [0] bad offsets, [1] ties, [2] members and [3] runs (read back), [1024..3071] digit counts
+  uint32_t* hist = D[B_HIST].as<uint32_t>();
+  uint32_t* tmp = D[B_TMP].as<uint32_t>();
+  uint64_t* const K[2] = {D[B_K0].as<uint64_t>(), D[B_K1].as<uint64_t>()};
+  uint32_t* tie = D[B_TIE].as<uint32_t>();
+
+  CUDA_OK(cudaMemsetAsync(small, 0, 4096, st));
+  CUDA_OK(cudaEventRecord(c->ev0, st));
+  launch_check_offsets(d_val_off, n, vals_bytes, small + 0, st);
+  const uint8_t* keys32 = d_keys;
+  if (hash) {
+    D[B_HKEYS].reserve(32ull * n);
+    launch_hash_fixed_keys(d_keys, key_len, n, D[B_HKEYS].as<uint8_t>(), st);
+    keys32 = D[B_HKEYS].as<uint8_t>();
+    c->stats.key_hashes = n, c->stats.key_permutations = n, c->stats.kernel_launches += 1;
+  }
+  // the whole set on word 0: (word, input position) pairs
+  launch_key_word(keys32, n, 0, K[0], D[B_V0].as<uint32_t>(), st);
+  c->stats.kernel_launches += 2;
+  uint32_t digits = varying_digits(c, K[0], n, small + 1024);
+  uint32_t bad = 0;
+  CUDA_OK(cudaMemcpyAsync(&bad, small + 0, 4, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  if (bad) fail(PPD_ERR_BAD_ARGUMENT, "val_off decreases somewhere or val_off[n] exceeds vals_bytes");
+  uint32_t* const V01[2] = {D[B_V0].as<uint32_t>(), D[B_V1].as<uint32_t>()};
+  const int r0 = sort_pairs(c, K, V01, 0, n, digits, hist, tmp);
+  uint32_t* idx = V01[r0];  // input position of the element at each sorted position
+  launch_tie_flags(K[r0], n, tie, small + 1, st);
+  uint32_t ties = 0;
+  CUDA_OK(cudaMemcpyAsync(&ties, small + 1, 4, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  c->stats.kernel_launches += 1;
+  c->stats.d2h_bytes += 8;
+
+  // refine the runs that tie on the words so far by the next word; runs keep their positions, so only their members move
+  TieRuns R;
+  R.member = D[B_MEMBER].as<uint32_t>(), R.mpos = D[B_MPOS].as<uint32_t>(), R.start = D[B_START].as<uint32_t>(), R.spos = D[B_SPOS].as<uint32_t>();
+  R.cpos = D[B_CPOS].as<uint32_t>(), R.cidx = D[B_CIDX].as<uint32_t>(), R.crun = D[B_CRUN].as<uint32_t>(), R.cword = D[B_CWORD].as<uint64_t>();
+  uint32_t* const VR[2] = {V01[1 - r0], D[B_V2].as<uint32_t>()};
+  for (int w = 1; w < 4 && ties; w++) {
+    launch_tie_members(tie, n, R.member, R.start, st);
+    exclusive_scan_u32(R.member, R.mpos, n + 1, tmp, st);
+    exclusive_scan_u32(R.start, R.spos, n + 1, tmp, st);
+    launch_tie_compact(R, keys32, idx, n, w, K[0], VR[0], st);
+    CUDA_OK(cudaMemcpyAsync(small + 2, R.mpos + n, 4, cudaMemcpyDeviceToDevice, st));
+    CUDA_OK(cudaMemcpyAsync(small + 3, R.spos + n, 4, cudaMemcpyDeviceToDevice, st));
+    CUDA_OK(cudaMemsetAsync(small + 1, 0, 4, st));
+    uint32_t mr[2];
+    CUDA_OK(cudaMemcpyAsync(mr, small + 2, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_OK(cudaStreamSynchronize(st));
+    const uint32_t m = mr[0], runs = mr[1];
+    c->stats.kernel_launches += 2 + 2 * scan_launches((size_t)n + 1);
+    c->stats.d2h_bytes += 8;
+    // sort A: the members by the word; sort B: stably by run (the digits a run id below `runs` can have)
+    const int ra = sort_pairs(c, K, VR, 0, m, varying_digits(c, K[0], m, small + 1024), hist, tmp);
+    launch_tie_run_key(R, VR[ra], m, K[1 - ra], VR[1 - ra], st);
+    uint32_t run_digits = 0;
+    for (int p = 0; p < 4; p++)
+      if ((uint64_t)(runs - 1) >> (8 * p)) run_digits |= 1u << p;
+    const int rb = sort_pairs(c, K, VR, 1 - ra, m, run_digits, hist, tmp);
+    launch_tie_writeback(R, VR[rb], m, idx, tie, small + 1, st);
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(&ties, small + 1, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_OK(cudaStreamSynchronize(st));
+    c->stats.kernel_launches += 2;
+    c->stats.d2h_bytes += 4;
+  }
+
+  // the last occurrence of every key, packed: sorted keys32, offsets, values
+  const uint32_t kept = n - ties;
+  uint32_t* keep = R.member;
+  uint32_t* kpos = R.mpos;
+  uint64_t* len = D[B_LEN].as<uint64_t>();
+  uint64_t* koff = D[B_KOFF].as<uint64_t>();
+  launch_keep_last(tie, idx, d_val_off, n, keep, len, st);
+  exclusive_scan_u32(keep, kpos, n + 1, tmp, st);
+  c->stats.kernel_launches += 2 + 2 * scan_launches((size_t)n + 1) + exclusive_scan_u64(len, koff, n + 1, D[B_TMP64].as<uint64_t>(), st);
+  D[B_OKEYS].reserve(32ull * kept);
+  D[B_OOFF].reserve(8ull * (kept + 1));
+  D[B_OVALS].reserve(vals_bytes + 64);  // the kept values add up to at most val_off[n] - val_off[0] <= vals_bytes
+  launch_gather_leaves(keys32, idx, d_val_off, d_vals, n, keep, kpos, koff, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(),
+                       D[B_OVALS].as<uint8_t>(), st);
+  CUDA_OK(cudaGetLastError());
+  CUDA_OK(cudaEventRecord(c->ev1, st));
+  CUDA_OK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  c->stats.gpu_ms += ms;  // the builder adds its own part
+  try {
+    trie_root_sorted_dev(c, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(), D[B_OVALS].as<uint8_t>(), kept, root_out);
+  } catch (const Fail& f) {
+    if (f.code != PPD_ERR_UNSORTED_KEYS) throw;
+    fail(PPD_ERR_CUDA, "internal error: the sorted, de-duplicated leaves are not strictly ascending (a bug of the leaf sort, or device "
+         "inputs that changed during the call)");
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -1029,6 +1182,35 @@ int ppd_trie_root_sorted_leaves(ppd_ctx* c, const uint8_t* keys32, const uint64_
     CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
     c->stats.h2d_bytes += (double)(32 * n + 8 * (n + 1) + vb);
     trie_root_sorted_dev(c, c->d_keys.as<uint8_t>(), c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, root_out);
+  });
+}
+
+int ppd_trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
+                             size_t n, size_t vals_bytes, uint8_t root_out[32]) {
+  return guarded(c, [&] {
+    stats_reset(c);
+    trie_root_leaves_dev(c, d_keys, key_len, flags, d_val_off, d_vals, n, vals_bytes, root_out);
+  });
+}
+
+int ppd_trie_root_leaves(ppd_ctx* c, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off, const uint8_t* vals, size_t n,
+                         uint8_t root_out[32]) {
+  return guarded(c, [&] {
+    stats_reset(c);
+    if (n && n < 0x7fffffffull && key_len >= 1 && key_len <= 135) {
+      // upload, then the device path checks everything (the offsets included: vals_bytes is what the caller says val_off[n] is)
+      const size_t vb = val_off[n];
+      c->d_keys.reserve((size_t)key_len * n);
+      c->d_msg_off.reserve(8 * (n + 1));
+      c->d_vals.reserve(vb + 64);
+      CUDA_OK(cudaMemcpyAsync(c->d_keys.p, keys, (size_t)key_len * n, cudaMemcpyHostToDevice, c->st));
+      CUDA_OK(cudaMemcpyAsync(c->d_msg_off.p, val_off, 8 * (n + 1), cudaMemcpyHostToDevice, c->st));
+      CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
+      c->stats.h2d_bytes += (double)((size_t)key_len * n + 8 * (n + 1) + vb);
+      trie_root_leaves_dev(c, c->d_keys.as<uint8_t>(), key_len, flags, c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, vb, root_out);
+    } else {
+      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out);  // the empty trie, or the argument error
+    }
   });
 }
 

@@ -79,6 +79,32 @@ void launch_branch_scatter(const uint8_t* depth, const uint32_t* nchild, uint32_
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st);
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st);
 
+// ---- ppd_leaves.cu: leaves in any order -> the strictly ascending, de-duplicated leaves of the builder ----
+uint32_t scan_launches(size_t n);  // kernels launched by exclusive_scan_u32 over n elements
+// tmp: at least scan_tmp_words(n) uint64 (exclusive_scan_u64 returns the number of kernels launched)
+uint32_t exclusive_scan_u64(const uint64_t* in, uint64_t* out, uint32_t n, uint64_t* tmp, cudaStream_t st);
+void launch_check_offsets(const uint64_t* val_off, uint32_t n, uint64_t vals_bytes, uint32_t* flag, cudaStream_t st);
+void launch_hash_fixed_keys(const uint8_t* keys, uint32_t key_len, uint32_t n, uint8_t* out32, cudaStream_t st);
+void launch_key_word(const uint8_t* keys32, uint32_t n, int w, uint64_t* out_key, uint32_t* out_val, cudaStream_t st);
+void launch_digit_counts(const uint64_t* keys, uint32_t n, uint32_t* counts, cudaStream_t st);  // counts[8 * 256], zeroed by the caller
+size_t radix_hist_words(uint32_t n);
+// one stable pass on byte digit `digit`; hist and hist_scan hold radix_hist_words(n) words, scan_tmp scan_tmp_words(of that)
+uint32_t launch_radix_pass(const uint64_t* keys_in, const uint32_t* vals_in, uint64_t* keys_out, uint32_t* vals_out, uint32_t n, int digit,
+                           uint32_t* hist, uint32_t* hist_scan, uint32_t* scan_tmp, cudaStream_t st);
+void launch_tie_flags(const uint64_t* sorted_keys, uint32_t n, uint32_t* tie, uint32_t* count, cudaStream_t st);
+struct TieRuns {
+  uint32_t *member, *mpos, *start, *spos;  // [n + 1]: in a tied run / its first element, and their exclusive scans
+  uint32_t *cpos, *cidx, *crun;            // per member, compacted: position, input index, run
+  uint64_t* cword;                         // ... and the key word being sorted
+};
+void launch_tie_members(const uint32_t* tie, uint32_t n, uint32_t* member, uint32_t* start, cudaStream_t st);
+void launch_tie_compact(const TieRuns& R, const uint8_t* keys32, const uint32_t* idx, uint32_t n, int w, uint64_t* key, uint32_t* val, cudaStream_t st);
+void launch_tie_run_key(const TieRuns& R, const uint32_t* order, uint32_t m, uint64_t* key, uint32_t* val, cudaStream_t st);
+void launch_tie_writeback(const TieRuns& R, const uint32_t* order, uint32_t m, uint32_t* idx, uint32_t* tie, uint32_t* count, cudaStream_t st);
+void launch_keep_last(const uint32_t* tie, const uint32_t* idx, const uint64_t* val_off, uint32_t n, uint32_t* keep, uint64_t* len, cudaStream_t st);
+void launch_gather_leaves(const uint8_t* keys32, const uint32_t* idx, const uint64_t* val_off, const uint8_t* vals, uint32_t n, const uint32_t* keep,
+                          const uint32_t* kpos, const uint64_t* koff, uint8_t* keys_out, uint64_t* off_out, uint8_t* vals_out, cudaStream_t st);
+
 // ---- ppd_dump.cu: the per-txn sub-tries serialised on the GPU ----
 // segment kinds IR_SEG_* (seg_b): arena.h
 struct IrDumpPlanView {

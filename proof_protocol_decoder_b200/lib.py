@@ -118,7 +118,11 @@ EXPORTS = [
     "ppd_replay_last_parse",
     "ppd_microbench",
     "ppd_direct_to_compact",
+    "ppd_trie_root_leaves",
+    "ppd_trie_root_leaves_dev",
 ]
+
+LEAVES_HASH_KEYS = 1  # PPD_LEAVES_HASH_KEYS: key i is keccak256 of the given key bytes
 
 
 def build_extension(verbose=False):
@@ -164,6 +168,8 @@ class PpdLibrary:
         L.ppd_trie_root_from_children.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_uint32, ctypes.c_char_p]
 
         L.ppd_direct_to_compact.argtypes = [ctypes.c_void_p, ctypes.c_size_t, u8pp, szp]
+        L.ppd_trie_root_leaves.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_char_p]
+        L.ppd_trie_root_leaves_dev.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_size_t, ctypes.c_char_p]
 
     def exported(self):
         return [name for name in EXPORTS if hasattr(self.L, name)]
@@ -387,6 +393,30 @@ class Context:
         self._check(self.lib.L.ppd_trie_root_sorted_leaves_dev(self.h, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, out))
         return out.raw
 
+
+    def trie_root_leaves(self, keys, val_off, vals, hash_keys=False) -> bytes:
+        """Root of the trie that inserting the leaves in order gives: keys in any order, a repeated key keeps its last
+        value.  keys: uint8 [n, key_len] (key_len 32, or 1..135 with hash_keys: the key is then keccak256 of the row)."""
+        import numpy as np
+
+        keys = np.ascontiguousarray(keys, dtype=np.uint8)
+        val_off = np.ascontiguousarray(val_off, dtype=np.uint64)
+        vals = np.ascontiguousarray(vals, dtype=np.uint8)
+        if keys.ndim != 2 or keys.shape[0] != len(val_off) - 1:
+            raise ValueError("keys must be [n, key_len] with n = len(val_off) - 1")
+        out = ctypes.create_string_buffer(32)
+        flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_root_leaves(self.h, keys.ctypes.data, keys.shape[1], flags, val_off.ctypes.data, vals.ctypes.data, keys.shape[0], out))
+        return out.raw
+
+    def trie_root_leaves_dev(self, d_keys_ptr, key_len, d_val_off_ptr, d_vals_ptr, n, vals_bytes, hash_keys=False, flags=None) -> bytes:
+        """trie_root_leaves on device buffers (e.g. torch tensors' data_ptr()), which must be complete when it is called: the
+        library reads them on a stream of its own (torch.cuda.synchronize() first).  `flags` overrides hash_keys when given."""
+        out = ctypes.create_string_buffer(32)
+        if flags is None:
+            flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_root_leaves_dev(self.h, d_keys_ptr, key_len, flags, d_val_off_ptr, d_vals_ptr, n, vals_bytes, out))
+        return out.raw
 
     def trie_subroot_sorted_leaves_dev(self, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, base_depth) -> bytes:
         """The ref of the sub-trie over n sorted leaves that share their first base_depth nibbles (device pointers)."""

@@ -679,3 +679,41 @@ def gen_sorted_leaves(n, seed=5, val_lo=70, val_hi=80):
     vals[val_off[:-1].astype(np.int64)] = 0xF8
     vals[val_off[:-1].astype(np.int64) + 1] = (lens - 2).astype(np.uint8)
     return keys, val_off, vals
+
+
+def gen_sorted_leaves_dev(n, seed=5, val_lo=70, val_hi=80, device="cuda"):
+    """gen_sorted_leaves on the device (torch), for sizes the host generator is too slow for: n distinct 32-byte keys,
+    ascending by construction (word 0 = i * step + r with 0 <= r < step; bytes 8..31 random), values of val_lo..val_hi
+    random bytes.  Returns (keys uint8 [n,32], val_off int64 [n+1], vals uint8) on `device`."""
+    import torch
+
+    g = torch.Generator(device=device)
+    g.manual_seed(seed)
+    step = (1 << 62) // max(n, 1)
+    w0 = torch.arange(n, dtype=torch.int64, device=device) * step + torch.randint(0, step, (n,), generator=g, device=device, dtype=torch.int64)
+    keys = torch.randint(0, 256, (n, 32), generator=g, device=device, dtype=torch.uint8)
+    sh = torch.arange(56, -8, -8, device=device, dtype=torch.int64)
+    keys[:, :8] = ((w0[:, None] >> sh) & 0xFF).to(torch.uint8)
+    lens = torch.randint(val_lo, val_hi + 1, (n,), generator=g, device=device, dtype=torch.int64)
+    val_off = torch.zeros(n + 1, dtype=torch.int64, device=device)
+    torch.cumsum(lens, 0, out=val_off[1:])
+    vals = torch.randint(0, 256, (int(val_off[-1]),), generator=g, device=device, dtype=torch.uint8)
+    return keys, val_off, vals
+
+
+def permute_leaves_dev(keys, val_off, vals, perm, chunk=1 << 23):
+    """The leaves (keys, val_off, vals) in the order perm (leaf j of the result is leaf perm[j]), values repacked
+    (chunk leaves at a time: the byte-index temporaries stay a few GB at 100 M leaves)."""
+    import torch
+
+    lens = (val_off[1:] - val_off[:-1])[perm]
+    off = torch.zeros_like(val_off)
+    torch.cumsum(lens, 0, out=off[1:])
+    out = torch.empty(int(off[-1]), dtype=torch.uint8, device=vals.device)
+    for a in range(0, len(perm), chunk):
+        b = min(a + chunk, len(perm))
+        lo, hi = int(off[a]), int(off[b])
+        src = torch.repeat_interleave(val_off[:-1][perm[a:b]] - off[a:b], lens[a:b], output_size=hi - lo)
+        src += torch.arange(lo, hi, device=vals.device, dtype=torch.int64)
+        out[lo:hi] = vals[src]
+    return keys[perm].contiguous(), off, out
