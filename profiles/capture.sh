@@ -35,7 +35,7 @@ if has 4; then
   #    capture of the second (warm) decode's parse kernels
   PR="python profiles/run_parse.py"
   $PR 5 > $RAW/${TAG}_parse_plain.log 2> $RAW/${TAG}_parse_plain.err && ncu $LIST -c 2000 --log-file $RAW/${TAG}_launches_parse.csv $PR 2 > /dev/null 2>&1
-  K="regex:tile_exit|group_exit|top_chain|tile_entry|tile_mark|ins_scatter|ins_info|heights_kernel|min64_i16|link_kernel16|shape_kernel|mscan|^emit_kernel|climb_kernel|code_list|totals_kernel"
+  K="regex:tile_exit|group_exit|top_chain|tile_entry|tile_mark|ins_scatter|ins_info|heights_kernel|min64_i16|link_kernel16|shape_kernel|scan_block_kernel|scan_add_kernel|^emit_kernel|climb_kernel|code_list|totals_kernel"
   N=$(python profiles/summarize.py --count-parse-kernels $RAW/${TAG}_launches_parse.csv)
   ncu --set full --clock-control none --import-source on -k "$K" --launch-skip $N --launch-count $N -o $RAW/${TAG}_parse_full $PR 2 > $RAW/${TAG}_ncu_parse_full.log 2>&1
 fi

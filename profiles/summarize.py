@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.environ.get("SRC", os.path.join(ROOT, "gpurun_out"))
 DST = os.environ.get("DST", os.path.join(ROOT, "profiles"))
 PARSE_KERNELS = ("tile_exit", "group_exit", "top_chain", "tile_entry", "tile_mark", "ins_scatter", "ins_info", "heights_kernel", "min64_i16",
-                 "link_kernel16", "shape_kernel", "mscan", "emit_kernel", "climb_kernel", "code_list", "totals_kernel")
+                 "link_kernel16", "shape_kernel", "scan_block_kernel", "scan_add_kernel", "emit_kernel", "climb_kernel", "code_list", "totals_kernel")
 
 
 def launches(path):

@@ -122,7 +122,7 @@ bool gpu_pre_image(Lane* L, Job& J, BlockJob& b, bool check_version, Slots* slot
     B.bitmap = c.take<uint32_t>((size_t)B.n_tiles * (PARSE_TILE / 32));
     B.tile_count = c.take<uint32_t>(B.n_tiles + 1);
     B.tile_base = c.take<uint32_t>(B.n_tiles + 1);
-    B.scan_tmp = c.take<uint32_t>(parse_scan_tmp_words(B.n_tiles + 1, 1));
+    B.scan_tmp = c.take<uint32_t>(scan_tmp_words(B.n_tiles + 1));
   };
   {
     Carve sz{nullptr};
@@ -179,7 +179,7 @@ bool gpu_pre_image(Lane* L, Job& J, BlockJob& b, bool check_version, Slots* slot
     T.lvlmax = c.take<uint32_t>(n_ins);
     T.cnt = c.take<uint32_t>(PARSE_N_CNT * T.cnt_stride);
     T.scn = c.take<uint32_t>(PARSE_N_CNT * T.cnt_stride);
-    T.scan_tmp = c.take<uint32_t>(parse_scan_tmp_words(n1, PARSE_N_CNT));
+    T.scan_tmp = c.take<uint32_t>(scan_tmp_words(n1, PARSE_N_CNT));
   };
   {
     Carve sz{nullptr};

@@ -111,73 +111,6 @@ __global__ void leader_flag_kernel(const uint32_t* __restrict__ leader, uint32_t
   flag[q] = (q >= 1 && q < n && leader[q] == q) ? 1u : 0u;
 }
 
-// ---- exclusive prefix sum of uint32 (3-phase, recursive on the block sums) ----------------------
-static constexpr int SCAN_B = 256, SCAN_ITEMS = 4;  // 1024 elements per block
-
-__global__ void scan_block_kernel(const uint32_t* __restrict__ in, uint32_t* __restrict__ out, uint32_t n, uint32_t* __restrict__ block_sums) {
-  __shared__ uint32_t warp_sums[SCAN_B / 32];
-  uint32_t base = blockIdx.x * (SCAN_B * SCAN_ITEMS) + threadIdx.x * SCAN_ITEMS;
-  uint32_t v[SCAN_ITEMS], sum = 0;
-#pragma unroll
-  for (int k = 0; k < SCAN_ITEMS; k++) {
-    v[k] = base + k < n ? in[base + k] : 0u;
-    sum += v[k];
-  }
-  uint32_t incl = sum;
-  for (int off = 1; off < 32; off <<= 1) {
-    uint32_t t = __shfl_up_sync(0xffffffffu, incl, off);
-    if ((threadIdx.x & 31) >= off) incl += t;
-  }
-  if ((threadIdx.x & 31) == 31) warp_sums[threadIdx.x >> 5] = incl;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    uint32_t w = threadIdx.x < SCAN_B / 32 ? warp_sums[threadIdx.x] : 0u;
-    uint32_t wi = w;
-    for (int off = 1; off < 32; off <<= 1) {
-      uint32_t t = __shfl_up_sync(0xffffffffu, wi, off);
-      if (threadIdx.x >= off) wi += t;
-    }
-    if (threadIdx.x < SCAN_B / 32) warp_sums[threadIdx.x] = wi - w;  // exclusive
-    if (threadIdx.x == SCAN_B / 32 - 1 && block_sums) block_sums[blockIdx.x] = wi;
-  }
-  __syncthreads();
-  uint32_t excl = incl - sum + warp_sums[threadIdx.x >> 5];
-#pragma unroll
-  for (int k = 0; k < SCAN_ITEMS; k++) {
-    if (base + k < n) out[base + k] = excl;
-    excl += v[k];
-  }
-}
-__global__ void scan_add_kernel(uint32_t* __restrict__ out, uint32_t n, const uint32_t* __restrict__ block_offsets) {
-  uint32_t i = blockIdx.x * (SCAN_B * SCAN_ITEMS) + threadIdx.x;
-  uint32_t add = block_offsets[blockIdx.x];
-#pragma unroll
-  for (int k = 0; k < SCAN_ITEMS; k++) {
-    uint32_t j = i + k * SCAN_B;
-    if (j < n) out[j] += add;
-  }
-}
-
-// tmp must hold at least scan_tmp_words(n) uint32
-size_t scan_tmp_words(size_t n) {
-  size_t total = 0;
-  while (n > 1) {
-    n = (n + SCAN_B * SCAN_ITEMS - 1) / (SCAN_B * SCAN_ITEMS);
-    total += n + 1;
-  }
-  return total + 2;
-}
-void exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint32_t n, uint32_t* tmp, cudaStream_t st) {
-  if (!n) return;
-  uint32_t nb = (n + SCAN_B * SCAN_ITEMS - 1) / (SCAN_B * SCAN_ITEMS);
-  scan_block_kernel<<<nb, SCAN_B, 0, st>>>(in, out, n, nb > 1 ? tmp : nullptr);
-  if (nb > 1) {
-    exclusive_scan_u32(tmp, tmp, nb, tmp + nb + 1, st);
-    scan_add_kernel<<<nb, SCAN_B, 0, st>>>(out, n, tmp);
-  }
-}
-
-
 // per leader: depth, extension, parent link
 __global__ void branch_info_kernel(BuildView V) {
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -210,43 +143,6 @@ __global__ void child_count_kernel(const uint32_t* __restrict__ leader, const ui
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q == 0 || q >= n) return;
   atomicAdd(nchild + bidx[leader[q]], 1u);
-}
-
-// Sort key of a branch: depth * 16 + (number of children - 1).  Lanes of a warp then walk the same
-// number of children and run the same number of permutations (a branch with k hashed children
-// encodes to 33 k + (16 - k) + 1 payload bytes: 1 rate block up to k = 3, 2 up to 7, 3 up to 12, else 4).
-static constexpr int SORT_KEYS = 1024;
-__device__ __forceinline__ uint32_t branch_sort_key(uint32_t depth, uint32_t nchild_minus_1) { return depth * 16 + min(nchild_minus_1, 15u); }
-
-// hist[key] = number of branches with that key (block-local histogram, one global atomic per bin and block)
-__global__ void depth_hist_kernel(const uint8_t* __restrict__ depth, const uint32_t* __restrict__ nchild, uint32_t nb, uint32_t* __restrict__ hist_out) {
-  __shared__ uint32_t hist[SORT_KEYS];
-  for (int k = threadIdx.x; k < SORT_KEYS; k += blockDim.x) hist[k] = 0;
-  __syncthreads();
-  uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b < nb) atomicAdd(&hist[branch_sort_key(depth[b], nchild[b])], 1u);
-  __syncthreads();
-  for (int k = threadIdx.x; k < SORT_KEYS; k += blockDim.x)
-    if (hist[k]) atomicAdd(hist_out + k, hist[k]);
-}
-
-// counting sort of the branches by key: order[start[key] + k] = b
-__global__ void branch_scatter_kernel(const uint8_t* __restrict__ depth, const uint32_t* __restrict__ nchild, uint32_t nb, uint32_t* __restrict__ cursor,
-                                      uint32_t* __restrict__ order) {
-  __shared__ uint32_t hist[SORT_KEYS], base[SORT_KEYS];
-  for (int k = threadIdx.x; k < SORT_KEYS; k += blockDim.x) hist[k] = 0;
-  __syncthreads();
-  uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-  uint32_t key = 0, rank = 0;
-  if (b < nb) {
-    key = branch_sort_key(depth[b], nchild[b]);
-    rank = atomicAdd(&hist[key], 1u);
-  }
-  __syncthreads();
-  for (int k = threadIdx.x; k < SORT_KEYS; k += blockDim.x)
-    if (hist[k]) base[k] = atomicAdd(cursor + k, hist[k]);
-  __syncthreads();
-  if (b < nb) order[base[key] + rank] = b;
 }
 
 // ------------------------------------------------------------------ hashing kernels -----------
@@ -516,14 +412,6 @@ void launch_branch_info(const BuildView& V, cudaStream_t st) {
 void launch_child_count(const uint32_t* leader, const uint32_t* bidx, uint32_t n, uint32_t* nchild, cudaStream_t st) {
   if (n < 2) return;
   child_count_kernel<<<cdiv(n, 256), 256, 0, st>>>(leader, bidx, n, nchild);
-}
-void launch_depth_hist(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint32_t* hist, cudaStream_t st) {
-  if (!nb) return;
-  depth_hist_kernel<<<cdiv(nb, 1024), 1024, 0, st>>>(depth, nchild, nb, hist);
-}
-void launch_branch_scatter(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint32_t* cursor, uint32_t* order, cudaStream_t st) {
-  if (!nb) return;
-  branch_scatter_kernel<<<cdiv(nb, 1024), 1024, 0, st>>>(depth, nchild, nb, cursor, order);
 }
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st) {
   if (!V.n) return;

@@ -20,6 +20,7 @@
 #include "../../include/ppd_flat.h"
 #include "arena.h"
 #include "ppd_kernels.h"
+#include "scan.cuh"
 
 namespace ppd {
 
@@ -292,11 +293,7 @@ __global__ void __launch_bounds__(DUMP_THREADS) ir_size_kernel(ArenaView A, IrDu
           }
         }
       }
-      uint32_t incl = sz;
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if ((threadIdx.x & 31) >= (uint32_t)o) incl += t;
-      }
+      const uint32_t incl = warp_inclusive_scan(sz, threadIdx.x & 31);
       if ((threadIdx.x & 31) == 31) scan_warp[threadIdx.x >> 5] = incl;
       __syncthreads();
       uint32_t before = scan_carry;

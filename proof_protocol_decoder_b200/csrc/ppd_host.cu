@@ -843,7 +843,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   const uint32_t n = (uint32_t)n_;
   cudaStream_t st = c->st;
   const uint32_t n1 = (n + 1 + 63) / 64, n2 = (n1 + 63) / 64, n3 = (n2 + 63) / 64;
-  enum { B_L, B_M, B_LINKA, B_LINKB, B_BIDX, B_TMP, B_SMALL, B_DEPTH, B_REP, B_CHILD, B_ORDER, B_NCHILD };
+  enum { B_L, B_M, B_LINKA, B_LINKB, B_BIDX, B_TMP, B_SMALL, B_DEPTH, B_REP, B_CHILD, B_ORDER, B_NCHILD, B_KEYS };
   DevBuf* D = c->d_build;
   D[B_L].reserve((size_t)n + 1 + 64);
   D[B_M].reserve((size_t)n1 + n2 + n3 + 192);
@@ -856,7 +856,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   int8_t* m1 = D[B_M].as<int8_t>();
   int8_t* m2 = m1 + ((n1 + 63) & ~63u);
   int8_t* m3 = m2 + ((n2 + 63) & ~63u);
-  uint32_t* small = D[B_SMALL].as<uint32_t>();  // [0] error flags, [1] root id, [2..7] counters(u64 x 3), [8..15] root, [1024..2047] hist, [2048..3071] cursor
+  uint32_t* small = D[B_SMALL].as<uint32_t>();  // [0] error flags, [1] root id, [2..7] counters(u64 x 3), [8..15] root, [1024..2047] branch bins
   CUDA_OK(cudaMemsetAsync(small, 0, 16384, st));
   CUDA_OK(cudaEventRecord(c->ev0, st));
   launch_lcp(d_keys, n, L, small + 0, st, base_depth);
@@ -867,7 +867,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   uint32_t* flag = D[B_LINKB].as<uint32_t>();
   launch_leaders(L, m1, m2, m3, n, leader, flag, flag, st);
   uint32_t* bidx = D[B_BIDX].as<uint32_t>();
-  exclusive_scan_u32(flag, bidx, n + 1, D[B_TMP].as<uint32_t>(), st);
+  exclusive_scan(flag, bidx, n + 1, D[B_TMP].as<uint32_t>(), st);
   CUDA_OK(cudaGetLastError());
   uint32_t h_flags = 0, nb = 0;
   CUDA_OK(cudaMemcpyAsync(&h_flags, small, 4, cudaMemcpyDeviceToHost, st));
@@ -908,34 +908,26 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   if (nb) CUDA_OK(cudaMemsetAsync(nchild, 0, 4ull * nb, st));
   launch_branch_info(V, st);
   launch_child_count(leader, bidx, n, nchild, st);
-  // counting sort by (depth, number of children): the lanes of a warp walk the same number of children
-  // and run the same number of permutations
-  launch_depth_hist(V.depth, nchild, nb, small + 1024, st);
-  std::vector<uint32_t> hist(1024), cursor(1024), start(1024);
-  CUDA_OK(cudaMemcpyAsync(hist.data(), small + 1024, 4096, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  // deepest level first; inside a depth, child counts ascending
-  uint32_t acc = 0;
-  for (int d = 63; d >= 0; d--)
-    for (int k = 0; k < 16; k++) {
-      cursor[16 * d + k] = start[16 * d + k] = acc;
-      acc += hist[16 * d + k];
-    }
-  if (acc != nb) fail(PPD_ERR_CUDA, "branch histogram does not add up");
-  CUDA_OK(cudaMemcpyAsync(small + 2048, cursor.data(), 4096, cudaMemcpyHostToDevice, st));
+  // counting sort by (depth, number of children), deepest depth first: the lanes of a warp walk the same number of
+  // children and run the same number of permutations
+  D[B_KEYS].reserve(2ull * nb + 64);
   uint32_t* order = D[B_ORDER].as<uint32_t>();
-  launch_branch_scatter(V.depth, nchild, nb, small + 2048, order, st);
+  launch_order_branches(V.depth, nchild, nb, D[B_KEYS].as<uint16_t>(), small + 1024, order, st);
   launch_hash_sorted_leaves(V, st);
-  c->stats.kernel_launches += 5;
+  c->stats.kernel_launches += 6;
+  std::vector<uint32_t> end(BRANCH_BINS);  // end of every bucket: depth 63 - g owns buckets 16 g .. 16 g + 15
+  CUDA_OK(cudaMemcpyAsync(end.data(), small + 1024, 4 * BRANCH_BINS, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  if (end[BRANCH_BINS - 1] != nb) fail(PPD_ERR_CUDA, "branch histogram does not add up");
   uint32_t levels = 1;
-  for (int d = 63; d >= 0; d--) {
-    uint32_t cnt = 0;
-    for (int k = 0; k < 16; k++) cnt += hist[16 * d + k];
-    if (cnt) {
-      launch_hash_branch_level(V, order, start[16 * d], start[16 * d] + cnt, st);
+  for (uint32_t g = 0, begin = 0; g < 64; g++) {
+    const uint32_t e = end[16 * g + 15];
+    if (e > begin) {
+      launch_hash_branch_level(V, order, begin, e, st);
       c->stats.kernel_launches++;
       levels++;
     }
+    begin = e;
   }
   CUDA_OK(cudaGetLastError());
   CUDA_OK(cudaEventRecord(c->ev1, st));
@@ -1053,8 +1045,8 @@ void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, u
   uint32_t* const VR[2] = {V01[1 - r0], D[B_V2].as<uint32_t>()};
   for (int w = 1; w < 4 && ties; w++) {
     launch_tie_members(tie, n, R.member, R.start, st);
-    exclusive_scan_u32(R.member, R.mpos, n + 1, tmp, st);
-    exclusive_scan_u32(R.start, R.spos, n + 1, tmp, st);
+    uint32_t scans = exclusive_scan(R.member, R.mpos, n + 1, tmp, st);
+    scans += exclusive_scan(R.start, R.spos, n + 1, tmp, st);
     launch_tie_compact(R, keys32, idx, n, w, K[0], VR[0], st);
     CUDA_OK(cudaMemcpyAsync(small + 2, R.mpos + n, 4, cudaMemcpyDeviceToDevice, st));
     CUDA_OK(cudaMemcpyAsync(small + 3, R.spos + n, 4, cudaMemcpyDeviceToDevice, st));
@@ -1063,7 +1055,7 @@ void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, u
     CUDA_OK(cudaMemcpyAsync(mr, small + 2, 8, cudaMemcpyDeviceToHost, st));
     CUDA_OK(cudaStreamSynchronize(st));
     const uint32_t m = mr[0], runs = mr[1];
-    c->stats.kernel_launches += 2 + 2 * scan_launches((size_t)n + 1);
+    c->stats.kernel_launches += 2 + scans;
     c->stats.d2h_bytes += 8;
     // sort A: the members by the word; sort B: stably by run (the digits a run id below `runs` can have)
     const int ra = sort_pairs(c, K, VR, 0, m, varying_digits(c, K[0], m, small + 1024), hist, tmp);
@@ -1087,8 +1079,9 @@ void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, u
   uint64_t* len = D[B_LEN].as<uint64_t>();
   uint64_t* koff = D[B_KOFF].as<uint64_t>();
   launch_keep_last(tie, idx, d_val_off, n, keep, len, st);
-  exclusive_scan_u32(keep, kpos, n + 1, tmp, st);
-  c->stats.kernel_launches += 2 + 2 * scan_launches((size_t)n + 1) + exclusive_scan_u64(len, koff, n + 1, D[B_TMP64].as<uint64_t>(), st);
+  uint32_t scans = exclusive_scan(keep, kpos, n + 1, tmp, st);
+  scans += exclusive_scan(len, koff, n + 1, D[B_TMP64].as<uint64_t>(), st);
+  c->stats.kernel_launches += 2 + scans;
   D[B_OKEYS].reserve(32ull * kept);
   D[B_OOFF].reserve(8ull * (kept + 1));
   D[B_OVALS].reserve(vals_bytes + 64);  // the kept values add up to at most val_off[n] - val_off[0] <= vals_bytes

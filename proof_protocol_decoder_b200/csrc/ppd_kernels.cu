@@ -328,12 +328,13 @@ void launch_keccak256_ranges(const uint8_t* data, const uint64_t* begin_end, uin
   if (!n) return;
   keccak256_batch_kernel<KB><<<(n + KB - 1) / KB, KB, 0, st>>>(data, begin_end, 2, n, out);
 }
-// ------------------------------------------------------------------ level / class ordering ----
-// order[] = node ids counting-sorted by (level, class): inside a level, nodes of one kind and one permutation
-// count are adjacent, so the lanes of a warp do the same work.  Three launches: per-CTA shared-memory
-// histograms flushed to bins[], an exclusive scan of the bins, and a scatter in which every CTA reserves one
-// range per key it holds.  The order inside a bucket is whatever the atomics give (hashing does not care).
-static constexpr int OS_THREADS = 256, OS_PER = 8;  // nodes per CTA = 2048
+// ------------------------------------------------------------------ counting sort by a small key ----
+// order[] = ids counting-sorted by a key of at most 4096 values: arena nodes by (level, class), so that inside a
+// level nodes of one kind and one permutation count are adjacent, and the builder's branches by (depth, children);
+// either way the lanes of a warp do the same work.  Three launches: per-CTA shared-memory histograms flushed to
+// bins[], an exclusive scan of the bins, and a scatter in which every CTA reserves one range per key it holds.  The
+// order inside a bucket is whatever the atomics give (hashing does not care).
+static constexpr int OS_THREADS = 256, OS_PER = 8;  // items per CTA = 2048
 
 __device__ __forceinline__ uint32_t node_class(const NodeRec& r) {
   const uint32_t kind = r.w0 & 0xff;
@@ -347,11 +348,31 @@ __device__ __forceinline__ uint32_t node_class(const NodeRec& r) {
   return kind * 8 + (perms > 8 ? 7 : perms - 1);
 }
 
-// The nodes sorted are first .. first + n (n read from *n_dev - first when n_dev is given: the txn loop's node count is
-// only known on the device); keys[] and order[] are indexed from 0, order[] holds node ids.
-__global__ void __launch_bounds__(OS_THREADS) order_hist_kernel(const NodeRec* __restrict__ nodes, const uint16_t* __restrict__ level, uint32_t n,
-                                                                uint32_t n_bins, uint16_t* __restrict__ keys, uint32_t* __restrict__ bins,
-                                                                uint32_t first, const uint32_t* __restrict__ n_dev) {
+// A sort key: Key::of(a, b, j) = the bucket of item j, read from the arrays a and b (kernel parameters, so that they
+// keep __restrict__ and are read through the read-only path).
+
+// (level, class) of arena node j
+struct LevelClassKey {
+  static __device__ __forceinline__ uint32_t of(const NodeRec* __restrict__ nodes, const uint16_t* __restrict__ level, uint32_t j) {
+    return (uint32_t)level[j] * 64u + node_class(nodes[j]);
+  }
+};
+
+// (depth, number of children) of builder branch b: deepest depth first, then child counts ascending.  Lanes of a warp
+// then walk the same number of children and run the same number of permutations (a branch with k hashed children
+// encodes to 33 k + (16 - k) + 1 payload bytes: 1 rate block up to k = 3, 2 up to 7, 3 up to 12, else 4).
+struct BranchKey {
+  static __device__ __forceinline__ uint32_t of(const uint8_t* __restrict__ depth, const uint32_t* __restrict__ nchild_minus_1, uint32_t b) {
+    return (63u - depth[b]) * 16 + min(nchild_minus_1[b], 15u);
+  }
+};
+
+// The items sorted are first .. first + n (n read from *n_dev - first when n_dev is given: the txn loop's node count is
+// only known on the device); keys[] and order[] are indexed from 0, order[] holds item ids.
+template <class Key, class A, class B>
+__global__ void __launch_bounds__(OS_THREADS) order_hist_kernel(const A* __restrict__ a, const B* __restrict__ b, uint32_t n, uint32_t n_bins,
+                                                                uint16_t* __restrict__ keys, uint32_t* __restrict__ bins, uint32_t first,
+                                                                const uint32_t* __restrict__ n_dev) {
   extern __shared__ uint32_t sh[];
   if (n_dev) n = min(n, *n_dev - first);
   if (blockIdx.x * (OS_THREADS * OS_PER) >= n) return;
@@ -362,7 +383,7 @@ __global__ void __launch_bounds__(OS_THREADS) order_hist_kernel(const NodeRec* _
   for (int q = 0; q < OS_PER; q++) {
     const uint32_t i = base + q * OS_THREADS + threadIdx.x;
     if (i < n) {
-      const uint32_t key = min((uint32_t)level[first + i] * 64u + node_class(nodes[first + i]), n_bins - 1);
+      const uint32_t key = min(Key::of(a, b, first + i), n_bins - 1);
       keys[i] = (uint16_t)key;
       atomicAdd(&sh[key], 1u);
     }
@@ -370,39 +391,6 @@ __global__ void __launch_bounds__(OS_THREADS) order_hist_kernel(const NodeRec* _
   __syncthreads();
   for (uint32_t k = threadIdx.x; k < n_bins; k += OS_THREADS)
     if (sh[k]) atomicAdd(&bins[k], sh[k]);
-}
-
-// exclusive scan of bins[0 .. n_bins) in place, one CTA (n_bins <= 4096)
-__global__ void __launch_bounds__(1024) order_scan_kernel(uint32_t* __restrict__ bins, uint32_t n_bins) {
-  __shared__ uint32_t warp_sums[32];
-  __shared__ uint32_t carry;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n_bins; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const uint32_t v = i < n_bins ? bins[i] : 0u;
-    uint32_t incl = v;
-    for (int off = 1; off < 32; off <<= 1) {
-      uint32_t t = __shfl_up_sync(0xffffffffu, incl, off);
-      if ((threadIdx.x & 31) >= (uint32_t)off) incl += t;
-    }
-    if ((threadIdx.x & 31) == 31) warp_sums[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-      uint32_t ws = warp_sums[threadIdx.x], wi = ws;
-      for (int off = 1; off < 32; off <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, wi, off);
-        if (threadIdx.x >= (uint32_t)off) wi += t;
-      }
-      warp_sums[threadIdx.x] = wi - ws;
-    }
-    __syncthreads();
-    const uint32_t excl = carry + warp_sums[threadIdx.x >> 5] + incl - v;
-    if (i < n_bins) bins[i] = excl;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry = excl + v;
-    __syncthreads();
-  }
 }
 
 __global__ void __launch_bounds__(OS_THREADS) order_scatter_kernel(const uint16_t* __restrict__ keys, uint32_t n, uint32_t n_bins,
@@ -464,13 +452,22 @@ __global__ void store_u32x2_kernel(uint32_t* dst, uint32_t a, uint32_t b) { dst[
 void launch_store_u32x2(uint32_t* dst, uint32_t a, uint32_t b, cudaStream_t st) { store_u32x2_kernel<<<1, 1, 0, st>>>(dst, a, b); }
 
 // bins: [n_bins] zeroed by the caller; on return bins[k] = end of bucket k (the scatter advances the cursors)
-void launch_order_by_level_class(const NodeRec* nodes, const uint16_t* level, uint32_t n, uint32_t n_bins, uint16_t* keys, uint32_t* bins,
-                                 uint32_t* order, cudaStream_t st, uint32_t first, const uint32_t* n_dev) {
+template <class Key, class A, class B>
+void counting_sort(const A* a, const B* b, uint32_t n, uint32_t n_bins, uint16_t* keys, uint32_t* bins, uint32_t* order, cudaStream_t st,
+                   uint32_t first, const uint32_t* n_dev) {
   if (!n) return;
   const uint32_t blocks = (n + OS_THREADS * OS_PER - 1) / (OS_THREADS * OS_PER);
-  order_hist_kernel<<<blocks, OS_THREADS, 4 * n_bins, st>>>(nodes, level, n, n_bins, keys, bins, first, n_dev);
-  order_scan_kernel<<<1, 1024, 0, st>>>(bins, n_bins);
+  order_hist_kernel<Key><<<blocks, OS_THREADS, 4 * n_bins, st>>>(a, b, n, n_bins, keys, bins, first, n_dev);
+  exclusive_scan_small(bins, n_bins, st);
   order_scatter_kernel<<<blocks, OS_THREADS, 4 * n_bins, st>>>(keys, n, n_bins, bins, order, first, n_dev);
+}
+void launch_order_by_level_class(const NodeRec* nodes, const uint16_t* level, uint32_t n, uint32_t n_bins, uint16_t* keys, uint32_t* bins,
+                                 uint32_t* order, cudaStream_t st, uint32_t first, const uint32_t* n_dev) {
+  counting_sort<LevelClassKey>(nodes, level, n, n_bins, keys, bins, order, st, first, n_dev);
+}
+void launch_order_branches(const uint8_t* depth, const uint32_t* nchild_minus_1, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
+                           cudaStream_t st) {
+  counting_sort<BranchKey>(depth, nchild_minus_1, nb, BRANCH_BINS, keys, bins, order, st, 0, nullptr);
 }
 
 void launch_hash_level(const ArenaView& A, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st) {

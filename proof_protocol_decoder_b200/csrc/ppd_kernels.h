@@ -1,4 +1,4 @@
-// ppd_kernels.h — launchers of the sm_100a kernels (ppd_kernels.cu, ppd_build.cu)
+// ppd_kernels.h — launchers of the sm_100a kernels (ppd_kernels.cu, ppd_build.cu, ...)
 #pragma once
 #include <cuda_runtime.h>
 
@@ -9,14 +9,28 @@
 
 namespace ppd {
 
+// ---- scan.cu: exclusive prefix sums ----
+// K arrays of n elements (u32 or u64), array k at in + k * stride and out + k * stride (out may be in); tmp holds
+// scan_tmp_words(n, K) elements.  Returns the number of kernels launched.
+template <class T>
+uint32_t exclusive_scan(const T* in, T* out, uint32_t n, T* tmp, cudaStream_t st, uint32_t K = 1, size_t stride = 0);
+size_t scan_tmp_words(size_t n, uint32_t K = 1);
+void exclusive_scan_small(uint32_t* bins, uint32_t n_bins, cudaStream_t st);  // in place, one launch, n_bins <= 4096
+
 void launch_keccak256_batch(const uint8_t* data, const uint64_t* offsets, uint32_t n, uint8_t* out, cudaStream_t st);
 void launch_keccak256_ranges(const uint8_t* data, const uint64_t* begin_end, uint32_t n, uint8_t* out, cudaStream_t st);
 void launch_hash_level(const ArenaView& A, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st);
+// Counting sorts by a small key (three launches; on return bins[k] = end of bucket k).
 // order[] = node ids counting-sorted by (level, class) on the device; n_bins = 64 * levels (<= 4096), bins zeroed by the caller
 static const uint32_t ORDER_MAX_BINS = 4096;
 // sorts the nodes first .. first + n (n clipped to *n_dev - first when n_dev, a device pointer, is given)
 void launch_order_by_level_class(const NodeRec* nodes, const uint16_t* level, uint32_t n, uint32_t n_bins, uint16_t* keys, uint32_t* bins,
                                  uint32_t* order, cudaStream_t st, uint32_t first = 0, const uint32_t* n_dev = nullptr);
+// order[] = the builder's branches 0 .. nb counting-sorted by (depth, number of children): bucket 16 * (63 - depth) +
+// min(children - 1, 15), so deepest depth first; keys[nb], bins[BRANCH_BINS] zeroed by the caller
+static const uint32_t BRANCH_BINS = 1024;
+void launch_order_branches(const uint8_t* depth, const uint32_t* nchild_minus_1, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
+                           cudaStream_t st);
 
 // Small and medium copies done by a kernel instead of the copy engines: either side may be page-locked host memory
 // (device-accessible under unified addressing).  A copy engine serves its queue in order, so a few words a lane's host
@@ -66,23 +80,16 @@ struct BuildView {
   unsigned long long* counters;
 };
 
-size_t scan_tmp_words(size_t n);
-void exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint32_t n, uint32_t* tmp, cudaStream_t st);
 void launch_lcp(const uint8_t* keys, uint32_t n, int8_t* L, uint32_t* flags, cudaStream_t st, int base_depth = 0);
 void launch_min64(const int8_t* in, uint32_t n_in, int8_t* out, uint32_t n_out, cudaStream_t st);
 void launch_leaders(const int8_t* L, const int8_t* m1, const int8_t* m2, const int8_t* m3, uint32_t n, uint32_t* link_a, uint32_t* link_b,
                     uint32_t* flag, cudaStream_t st);
 void launch_branch_info(const BuildView& V, cudaStream_t st);
 void launch_child_count(const uint32_t* leader, const uint32_t* bidx, uint32_t n, uint32_t* nchild, cudaStream_t st);
-void launch_depth_hist(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint32_t* hist, cudaStream_t st);
-void launch_branch_scatter(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint32_t* cursor, uint32_t* order, cudaStream_t st);
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st);
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st);
 
 // ---- ppd_leaves.cu: leaves in any order -> the strictly ascending, de-duplicated leaves of the builder ----
-uint32_t scan_launches(size_t n);  // kernels launched by exclusive_scan_u32 over n elements
-// tmp: at least scan_tmp_words(n) uint64 (exclusive_scan_u64 returns the number of kernels launched)
-uint32_t exclusive_scan_u64(const uint64_t* in, uint64_t* out, uint32_t n, uint64_t* tmp, cudaStream_t st);
 void launch_check_offsets(const uint64_t* val_off, uint32_t n, uint64_t vals_bytes, uint32_t* flag, cudaStream_t st);
 void launch_hash_fixed_keys(const uint8_t* keys, uint32_t key_len, uint32_t n, uint8_t* out32, cudaStream_t st);
 void launch_key_word(const uint8_t* keys32, uint32_t n, int w, uint64_t* out_key, uint32_t* out_val, cudaStream_t st);
@@ -176,7 +183,7 @@ struct ParseBounds {
   uint32_t* bitmap;       // [n_tiles * PARSE_TILE / 32]
   uint32_t* tile_count;   // [n_tiles + 1]
   uint32_t* tile_base;    // [n_tiles + 1]
-  uint32_t* scan_tmp;     // parse_scan_tmp_words(n_tiles + 1, 1)
+  uint32_t* scan_tmp;     // scan_tmp_words(n_tiles + 1)
   uint32_t* result;       // [PARSE_R_WORDS]
 };
 struct ParseTree {
@@ -195,7 +202,7 @@ struct ParseTree {
   uint32_t *pending, *lvlmax;
   uint32_t *cnt, *scn;      // [PARSE_N_CNT][cnt_stride]
   size_t cnt_stride;        // >= n_ins + 1
-  uint32_t* scan_tmp;       // parse_scan_tmp_words(n_ins + 1, PARSE_N_CNT)
+  uint32_t* scan_tmp;       // scan_tmp_words(n_ins + 1, PARSE_N_CNT)
   uint32_t* result;
 };
 struct ParseEmit {
@@ -211,7 +218,6 @@ struct ParseEmit {
   const uint8_t* code_digest;  // [n_code][32]
   uint32_t n_keyed;            // result[PARSE_R_NKEYED] as the host read it after phase B
 };
-size_t parse_scan_tmp_words(size_t n, uint32_t K);
 uint32_t launch_parse_bounds(const ParseBounds& B, cudaStream_t st);  // the launchers return the number of kernels launched
 void launch_parse_scatter(const ParseBounds& B, uint32_t* ins_pos, cudaStream_t st);
 uint32_t launch_parse_tree(const ParseTree& T, cudaStream_t st);

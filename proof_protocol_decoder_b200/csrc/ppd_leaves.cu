@@ -7,7 +7,7 @@
 //   key_word_kernel          big-endian 64-bit word w of every key, paired with its input position
 //   digit_counts_kernel      counts of the 8 byte digits of n 64-bit keys: a digit of one value skips its pass
 //   radix_tile_hist_kernel   one pass of a stable LSD radix sort of (u64 key, u32 value) pairs: per-tile digit counts,
-//   radix_scatter_kernel     exclusive_scan_u32 of them (digit-major), and a scatter with in-tile ranks
+//   radix_scatter_kernel     exclusive_scan of them (digit-major), and a scatter with in-tile ranks
 //   tie_*_kernel             positions equal to their predecessor on the words sorted so far; the tied runs are
 //                            compacted, re-sorted on the next word (then stably by run) and written back
 //   keep_kernel / gather_kernel   the last element of every run of equal keys, packed with its value
@@ -297,71 +297,8 @@ __global__ void gather_kernel(const uint8_t* __restrict__ keys32, const uint32_t
   copy_bytes(vals_out + o, vals + b, val_off[s + 1] - b);
 }
 
-// ------------------------------------------------------------------ exclusive scan of u64 -------
-static constexpr int SCAN64_B = 256, SCAN64_ITEMS = 4;  // 1024 elements per block
-
-__global__ void __launch_bounds__(SCAN64_B) scan64_block_kernel(const uint64_t* __restrict__ in, uint64_t* __restrict__ out, uint32_t n,
-                                                                uint64_t* __restrict__ block_sums) {
-  __shared__ uint64_t warp_sums[SCAN64_B / 32];
-  uint32_t base = blockIdx.x * (SCAN64_B * SCAN64_ITEMS) + threadIdx.x * SCAN64_ITEMS;
-  uint64_t v[SCAN64_ITEMS], sum = 0;
-#pragma unroll
-  for (int k = 0; k < SCAN64_ITEMS; k++) {
-    v[k] = base + k < n ? in[base + k] : 0ull;
-    sum += v[k];
-  }
-  uint64_t incl = sum;
-  for (int off = 1; off < 32; off <<= 1) {
-    uint64_t t = __shfl_up_sync(FULL, incl, off);
-    if ((threadIdx.x & 31) >= off) incl += t;
-  }
-  if ((threadIdx.x & 31) == 31) warp_sums[threadIdx.x >> 5] = incl;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    uint64_t w = threadIdx.x < SCAN64_B / 32 ? warp_sums[threadIdx.x] : 0ull;
-    uint64_t wi = w;
-    for (int off = 1; off < 32; off <<= 1) {
-      uint64_t t = __shfl_up_sync(FULL, wi, off);
-      if (threadIdx.x >= off) wi += t;
-    }
-    if (threadIdx.x < SCAN64_B / 32) warp_sums[threadIdx.x] = wi - w;
-    if (threadIdx.x == SCAN64_B / 32 - 1 && block_sums) block_sums[blockIdx.x] = wi;
-  }
-  __syncthreads();
-  uint64_t excl = incl - sum + warp_sums[threadIdx.x >> 5];
-#pragma unroll
-  for (int k = 0; k < SCAN64_ITEMS; k++) {
-    if (base + k < n) out[base + k] = excl;
-    excl += v[k];
-  }
-}
-__global__ void __launch_bounds__(SCAN64_B) scan64_add_kernel(uint64_t* __restrict__ out, uint32_t n, const uint64_t* __restrict__ block_offsets) {
-  uint32_t i = blockIdx.x * (SCAN64_B * SCAN64_ITEMS) + threadIdx.x;
-  uint64_t add = block_offsets[blockIdx.x];
-#pragma unroll
-  for (int k = 0; k < SCAN64_ITEMS; k++) {
-    uint32_t j = i + k * SCAN64_B;
-    if (j < n) out[j] += add;
-  }
-}
-
 // ------------------------------------------------------------------ launchers -------
 static inline uint32_t grid(uint64_t n, uint32_t b) { return (uint32_t)((n + b - 1) / b); }
-
-uint32_t scan_launches(size_t n) {
-  if (!n) return 0;
-  size_t nb = (n + 1023) / 1024;
-  return nb > 1 ? 2 + scan_launches(nb) : 1;
-}
-uint32_t exclusive_scan_u64(const uint64_t* in, uint64_t* out, uint32_t n, uint64_t* tmp, cudaStream_t st) {
-  if (!n) return 0;
-  uint32_t nb = grid(n, SCAN64_B * SCAN64_ITEMS);
-  scan64_block_kernel<<<nb, SCAN64_B, 0, st>>>(in, out, n, nb > 1 ? tmp : nullptr);
-  if (nb == 1) return 1;
-  uint32_t k = exclusive_scan_u64(tmp, tmp, nb, tmp + nb + 1, st);
-  scan64_add_kernel<<<nb, SCAN64_B, 0, st>>>(out, n, tmp);
-  return k + 2;
-}
 
 void launch_check_offsets(const uint64_t* val_off, uint32_t n, uint64_t vals_bytes, uint32_t* flag, cudaStream_t st) {
   check_offsets_kernel<<<grid(n, 256), 256, 0, st>>>(val_off, n, vals_bytes, flag);
@@ -382,9 +319,9 @@ uint32_t launch_radix_pass(const uint64_t* keys_in, const uint32_t* vals_in, uin
                            uint32_t* hist, uint32_t* hist_scan, uint32_t* scan_tmp, cudaStream_t st) {
   const uint32_t tiles = grid(n, RADIX_TILE);
   radix_tile_hist_kernel<<<tiles, RADIX_B, 0, st>>>(keys_in, n, 8 * digit, tiles, hist);
-  exclusive_scan_u32(hist, hist_scan, 256 * tiles, scan_tmp, st);
+  const uint32_t scans = exclusive_scan(hist, hist_scan, 256 * tiles, scan_tmp, st);
   radix_scatter_kernel<<<tiles, RADIX_B, 0, st>>>(keys_in, vals_in, keys_out, vals_out, n, 8 * digit, tiles, hist_scan);
-  return 2 + scan_launches(256ull * tiles);
+  return 2 + scans;
 }
 void launch_tie_flags(const uint64_t* sorted_keys, uint32_t n, uint32_t* tie, uint32_t* count, cudaStream_t st) {
   tie_flags_kernel<<<grid(n + 1, 256), 256, 0, st>>>(sorted_keys, n, tie, count);

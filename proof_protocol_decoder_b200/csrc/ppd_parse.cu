@@ -37,6 +37,7 @@
 #include "../../include/ppd_status.h"
 #include "arena.h"
 #include "ppd_kernels.h"
+#include "scan.cuh"
 
 namespace ppd {
 
@@ -393,11 +394,7 @@ __global__ void __launch_bounds__(TILE / 32) ins_scatter_kernel(const uint32_t* 
   __shared__ uint32_t wsum[TILE / 32 / 32];
   const uint32_t t = blockIdx.x, tid = threadIdx.x;
   uint32_t word = bitmap[(size_t)t * (TILE / 32) + tid];
-  uint32_t c = __popc(word), incl = c;
-  for (int off = 1; off < 32; off <<= 1) {
-    uint32_t x = __shfl_up_sync(0xffffffffu, incl, off);
-    if ((tid & 31) >= (uint32_t)off) incl += x;
-  }
+  uint32_t c = __popc(word), incl = warp_inclusive_scan(c, tid & 31);
   if ((tid & 31) == 31) wsum[tid >> 5] = incl;
   __syncthreads();
   uint32_t before = 0;
@@ -409,74 +406,6 @@ __global__ void __launch_bounds__(TILE / 32) ins_scatter_kernel(const uint32_t* 
     word &= word - 1;
     ins_pos[at++] = p0 + b;
   }
-}
-
-// ---------------------------------------------------------------------------------------------
-// multi-array exclusive scan: K arrays of n uint32 each, array k at in + k * stride
-// ---------------------------------------------------------------------------------------------
-constexpr int MS_B = 256, MS_ITEMS = 4, MS_ELEMS = MS_B * MS_ITEMS;
-
-__global__ void __launch_bounds__(MS_B) mscan_block_kernel(const uint32_t* __restrict__ in, uint32_t* __restrict__ out, uint32_t n, size_t stride,
-                                                           uint32_t* __restrict__ block_sums, size_t sums_stride) {
-  __shared__ uint32_t warp_sums[MS_B / 32];
-  const uint32_t k = blockIdx.y;
-  in += k * stride, out += k * stride;
-  uint32_t base = blockIdx.x * MS_ELEMS + threadIdx.x * MS_ITEMS;
-  uint32_t v[MS_ITEMS], sum = 0;
-#pragma unroll
-  for (int q = 0; q < MS_ITEMS; q++) {
-    v[q] = base + q < n ? in[base + q] : 0u;
-    sum += v[q];
-  }
-  uint32_t incl = sum;
-  for (int off = 1; off < 32; off <<= 1) {
-    uint32_t t = __shfl_up_sync(0xffffffffu, incl, off);
-    if ((threadIdx.x & 31) >= (uint32_t)off) incl += t;
-  }
-  if ((threadIdx.x & 31) == 31) warp_sums[threadIdx.x >> 5] = incl;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    uint32_t ws = threadIdx.x < MS_B / 32 ? warp_sums[threadIdx.x] : 0u, wi = ws;
-    for (int off = 1; off < 32; off <<= 1) {
-      uint32_t t = __shfl_up_sync(0xffffffffu, wi, off);
-      if (threadIdx.x >= (uint32_t)off) wi += t;
-    }
-    if (threadIdx.x < MS_B / 32) warp_sums[threadIdx.x] = wi - ws;
-    if (threadIdx.x == MS_B / 32 - 1 && block_sums) block_sums[k * sums_stride + blockIdx.x] = wi;
-  }
-  __syncthreads();
-  uint32_t excl = incl - sum + warp_sums[threadIdx.x >> 5];
-#pragma unroll
-  for (int q = 0; q < MS_ITEMS; q++) {
-    if (base + q < n) out[base + q] = excl;
-    excl += v[q];
-  }
-}
-__global__ void __launch_bounds__(MS_B) mscan_add_kernel(uint32_t* __restrict__ out, uint32_t n, size_t stride, const uint32_t* __restrict__ block_offsets,
-                                                         size_t sums_stride) {
-  const uint32_t k = blockIdx.y;
-  out += k * stride;
-  uint32_t add = block_offsets[k * sums_stride + blockIdx.x];
-  uint32_t i = blockIdx.x * MS_ELEMS + threadIdx.x;
-#pragma unroll
-  for (int q = 0; q < MS_ITEMS; q++) {
-    uint32_t j = i + q * MS_B;
-    if (j < n) out[j] += add;
-  }
-}
-
-// returns the number of kernels launched
-uint32_t mscan(const uint32_t* in, uint32_t* out, uint32_t n, size_t stride, uint32_t K, uint32_t* tmp, cudaStream_t st) {
-  if (!n) return 0;
-  uint32_t nb = (n + MS_ELEMS - 1) / MS_ELEMS, launches = 1;
-  size_t ss = (nb + 3) & ~(size_t)3;
-  mscan_block_kernel<<<dim3(nb, K), MS_B, 0, st>>>(in, out, n, stride, nb > 1 ? tmp : nullptr, ss);
-  if (nb > 1) {
-    launches += mscan(tmp, tmp, nb, ss, K, tmp + K * ss, st);
-    mscan_add_kernel<<<dim3(nb, K), MS_B, 0, st>>>(out, n, stride, tmp, ss);
-    launches++;
-  }
-  return launches;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -972,15 +901,6 @@ inline uint32_t cdiv(uint64_t a, uint32_t b) { return (uint32_t)((a + b - 1) / b
 // ---------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------
-size_t parse_scan_tmp_words(size_t n, uint32_t K) {
-  size_t total = 0;
-  while (n > 1) {
-    n = (n + MS_ELEMS - 1) / MS_ELEMS;
-    total += K * ((n + 3) & ~(size_t)3);
-  }
-  return total + 16;
-}
-
 uint32_t launch_parse_bounds(const ParseBounds& B, cudaStream_t st) {
   const uint32_t group_bytes = B.group_tiles * TILE;
   static const bool once = cudaFuncSetAttribute(tile_exit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TE_SMEM_BYTES) == cudaSuccess;
@@ -994,7 +914,7 @@ uint32_t launch_parse_bounds(const ParseBounds& B, cudaStream_t st) {
   cudaMemsetAsync(B.bitmap, 0, (size_t)B.n_tiles * (TILE / 8), st);
   tile_mark_thin_kernel<<<cdiv(B.n_tiles, 128), 128, 0, st>>>(B.step1, B.n_tiles, B.tile_entry, B.bitmap, B.tile_count);
   cudaMemsetAsync(B.tile_count + B.n_tiles, 0, 4, st);
-  uint32_t launches = 5 + mscan(B.tile_count, B.tile_base, B.n_tiles + 1, 0, 1, B.scan_tmp, st);
+  uint32_t launches = 5 + exclusive_scan(B.tile_count, B.tile_base, B.n_tiles + 1, B.scan_tmp, st);
   cudaMemcpyAsync(B.result + PARSE_R_NINS, B.tile_base + B.n_tiles, 4, cudaMemcpyDeviceToDevice, st);
   return launches;
 }
@@ -1007,7 +927,7 @@ uint32_t launch_parse_tree(const ParseTree& T, cudaStream_t st) {
   const uint32_t n1 = T.n_ins + 1;
   ins_info_kernel<<<cdiv(n1, 256), 256, 0, st>>>(T);
   uint32_t launches = 8;  // ins_info, heights, 3 x min64, link, shape, totals
-  launches += mscan(T.delta, T.hb, n1, 0, 1, T.scan_tmp, st);
+  launches += exclusive_scan(T.delta, T.hb, n1, T.scan_tmp, st);
   heights_kernel<<<cdiv(n1, 256), 256, 0, st>>>(T);
   const uint32_t n_m1 = cdiv(n1, 64), n_m2 = cdiv(n_m1, 64), n_m3 = cdiv(n_m2, 64);
   min8_64_i16_kernel<<<cdiv(n_m1, 128), 128, 0, st>>>(T.h16, n1, T.m0, T.m1, n_m1);
@@ -1015,7 +935,7 @@ uint32_t launch_parse_tree(const ParseTree& T, cudaStream_t st) {
   min64_i16_kernel<<<cdiv(n_m3, 128), 128, 0, st>>>(T.m2, n_m2, T.m3, n_m3);
   link_kernel16<<<cdiv(T.n_ins, 256), 256, 0, st>>>(T);
   shape_kernel<<<cdiv(n1, 256), 256, 0, st>>>(T);
-  launches += mscan(T.cnt, T.scn, n1, T.cnt_stride, PARSE_N_CNT, T.scan_tmp, st);
+  launches += exclusive_scan(T.cnt, T.scn, n1, T.scan_tmp, st, PARSE_N_CNT, T.cnt_stride);
   totals_kernel<<<1, 32, 0, st>>>(T);
   return launches;
 }
