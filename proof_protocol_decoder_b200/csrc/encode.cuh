@@ -40,27 +40,32 @@ __device__ __forceinline__ uint32_t ld_bytes(const uint8_t* p, uint32_t cnt) {
   return __funnelshift_r(lo, hi, ofs * 8);
 }
 
-// n bytes from any global address.  Branch-free in the alignment (lanes of a warp read values at
-// different alignments): always the funnel-shift path, with the look-ahead load predicated on the
-// word still holding a requested byte.
-template <int B>
-__device__ __forceinline__ void emit_bytes(Stage<B>& s, const uint8_t* p, uint32_t n) {
+// n bytes that start at byte ofs (0..3) of aligned word 0 of a word source ld(i).  Branch-free in the
+// alignment (lanes of a warp read values at different alignments): always the funnel-shift path, with
+// the look-ahead load predicated on the word still holding a requested byte.
+template <int B, class Ld>
+__device__ __forceinline__ void emit_words(Stage<B>& s, const Ld& ld, uint32_t ofs, uint32_t n) {
   if (n == 0) return;
-  uintptr_t a = reinterpret_cast<uintptr_t>(p);
-  const uint32_t* q = reinterpret_cast<const uint32_t*>(a & ~(uintptr_t)3);
-  const uint32_t ofs = (uint32_t)(a & 3), sh = ofs * 8;
+  const uint32_t sh = ofs * 8;
   const uint32_t nwords = (ofs + n + 3) >> 2;  // aligned words that hold a requested byte
   const uint32_t full = n >> 2, rem = n & 3;
-  uint32_t cur = __ldg(q);
+  uint32_t cur = ld(0u);
   for (uint32_t i = 0; i < full; i++) {
-    uint32_t nxt = (i + 1 < nwords) ? __ldg(q + i + 1) : 0u;
+    uint32_t nxt = (i + 1 < nwords) ? ld(i + 1) : 0u;
     s.put_word(__funnelshift_r(cur, nxt, sh));
     cur = nxt;
   }
   if (rem) {
-    uint32_t nxt = (full + 1 < nwords) ? __ldg(q + full + 1) : 0u;
+    uint32_t nxt = (full + 1 < nwords) ? ld(full + 1) : 0u;
     s.put_partial(__funnelshift_r(cur, nxt, sh), rem);
   }
+}
+// n bytes from any global address
+template <int B>
+__device__ __forceinline__ void emit_bytes(Stage<B>& s, const uint8_t* p, uint32_t n) {
+  uintptr_t a = reinterpret_cast<uintptr_t>(p);
+  const uint32_t* q = reinterpret_cast<const uint32_t*>(a & ~(uintptr_t)3);
+  emit_words(s, [q](uint32_t i) { return __ldg(q + i); }, (uint32_t)(a & 3), n);
 }
 
 // m bytes of a packed nibble string that starts at the high (odd == 0) or the low (odd == 1)
@@ -161,13 +166,15 @@ __device__ __forceinline__ void digest_words(const uint64_t (&a)[25], uint4& x, 
 template <int B>
 __device__ __forceinline__ void inline_ref_words(Stage<B>& s, uint32_t total, uint4& x, uint4& y) {
   s.flush_partial();
-  uint32_t nw = (total + 3) >> 2;
   uint32_t h[8] = {s.template word<0>(), s.template word<1>(), s.template word<2>(), s.template word<3>(),
                    s.template word<4>(), s.template word<5>(), s.template word<6>(), s.template word<7>()};
-  uint32_t tail = total & 3;
-  uint32_t keep = tail ? (1u << (8 * tail)) - 1 : 0xffffffffu;
+  // word k keeps its first total - 4k bytes (a mask per word: a test against the last word's index lets the
+  // compiler turn the loop into a store to h[nw - 1], which puts h in local memory)
 #pragma unroll
-  for (int k = 0; k < 8; k++) h[k] = (uint32_t)k < nw ? ((uint32_t)k == nw - 1 ? h[k] & keep : h[k]) : 0u;
+  for (int k = 0; k < 8; k++) {
+    const int rem = (int)total - 4 * k;
+    h[k] &= rem >= 4 ? 0xffffffffu : rem > 0 ? (1u << (8 * rem)) - 1 : 0u;
+  }
   x = make_uint4(h[0], h[1], h[2], h[3]);
   y = make_uint4(h[4], h[5], h[6], h[7]);
 }

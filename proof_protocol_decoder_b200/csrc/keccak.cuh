@@ -270,6 +270,46 @@ struct Stage {
   }
 };
 
+// ---------------------------------------------------------------------------------------------
+// Gather slot: source bytes of a thread's NEXT unit, copied from global memory by cp.async while
+// the permutation of the current block runs, so that the fill after it reads shared memory instead
+// of waiting on L2.  CHUNKS 16-byte chunks per thread, chunk-interleaved (chunk c of thread t at
+// slot[c * BLOCK + t]): 16-byte accesses of a warp are conflict-free, and cp.async needs 16
+// contiguous bytes.  Every thread reads only its own chunks, so no barrier is involved:
+// cp.async.wait_group 0 makes the copies visible to the thread that issued them.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ void cp_async16(uint32_t saddr, const void* gsrc) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
+__device__ __forceinline__ uint32_t lds32_at(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ uint4 lds128(uint32_t addr) {
+  uint4 v;
+  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
+  asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+
+template <int BLOCK, int CHUNKS>
+struct Gather {
+  static constexpr uint32_t STRIDE = 16u * BLOCK;  // bytes between consecutive chunks of one thread
+  static constexpr uint32_t BYTES = 16u * CHUNKS * BLOCK;
+  uint32_t lo;  // shared address of this thread's chunk 0
+
+  __device__ __forceinline__ void init(const void* base) { lo = (uint32_t)__cvta_generic_to_shared(base) + 16u * threadIdx.x; }
+  __device__ __forceinline__ uint32_t chunk(uint32_t c) const { return lo + c * STRIDE; }
+  // 32-bit word i of the slot (word i & 3 of chunk i >> 2)
+  __device__ __forceinline__ uint32_t word(uint32_t i) const { return lds32_at(lo + (i >> 2) * STRIDE + 4u * (i & 3)); }
+  __device__ __forceinline__ void put_word(uint32_t i, uint32_t v) const { sts32(lo + (i >> 2) * STRIDE + 4u * (i & 3), v); }
+};
+
 template <int BLOCK>
 __device__ __forceinline__ void absorb_stage(uint64_t (&a)[25], const Stage<BLOCK>& s) {
 #define PPD_ABSORB(i) a[i] ^= ((uint64_t)s.template word<2 * (i) + 1>() << 32) | s.template word<2 * (i)>();

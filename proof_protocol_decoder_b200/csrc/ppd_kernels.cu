@@ -95,10 +95,28 @@ __global__ void __launch_bounds__(B) keccak256_batch_kernel(const uint8_t* __res
 //   BRANCH        0: list header   1..: three children each with the empty slots before them (the last
 //                 unit also carries the trailing empty slots and the empty value)
 //   ROOT          0: the child's raw RLP (only when it is shorter than 32 bytes) or 0x80
+//
+// Gathers: a LEAF's value units and a BRANCH's child units go through the thread's gather slot.  Before
+// the permutation of a block, the thread starts cp.async copies of the unit the next fill begins with
+// (a leaf's next <= 128 value bytes, a branch's next three child refs), so the loads overlap the
+// permutation instead of following it.  A unit the fill needs beyond that one is gathered and waited
+// for on the spot.  A branch's child ids sit in the slot from the prologue on (chunks 6-9), so a unit
+// needs no reload of child_pool.  The other kinds put all their units into the first block.
+static constexpr int GATHER_CHUNKS = 10;  // branch: 3 refs (chunks 0-5) + 16 child ids (6-9); leaf: <= 144 bytes (0-8)
+static constexpr uint32_t GATHER_IDS = 6;
+
+template <int B>
+using HashGather = Gather<B, GATHER_CHUNKS>;
+template <int B>
+constexpr uint32_t hash_smem_bytes() {
+  return 4u * PPD_STAGE_WORDS * B + HashGather<B>::BYTES;
+}
+
+extern __shared__ uint4 hash_smem[];  // the block's stages, then its gather slots
 
 template <int B>
 __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uint32_t* __restrict__ order, uint32_t begin, uint32_t end) {
-  __shared__ uint32_t smem[PPD_STAGE_WORDS * B];
+  uint32_t* smem = reinterpret_cast<uint32_t*>(hash_smem);
   const uint32_t slot = begin + blockIdx.x * B + threadIdx.x;
   uint32_t hashed = 0, perms = 0, enc_bytes = 0;
   bool busy = false, force_hash = false;
@@ -109,6 +127,9 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
   uint32_t payload = 0, nunit = 0, total = 0, unit = 0;
   // LEAF: vlen, vhdr   LEAF_ACCOUNT: vlen, nn | nb << 8 | apayload << 16   BRANCH: slots left, walk state
   uint32_t v0 = 0, v1 = 0;
+  uint32_t gathered = 0;  // the unit whose source bytes are in the gather slot (0: none)
+  HashGather<B> G;
+  G.init(smem + PPD_STAGE_WORDS * B);
 #define KIND (rec.x & 0xff)
 #define NIB_START ((rec.x >> 8) & 0xff)
 #define NIB_LEN ((rec.x >> 16) & 0xff)
@@ -161,6 +182,8 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
           payload += cl == 32 ? 33u : cl;
           hashed_kids |= (cl == 32 ? 1u : 0u) << j;
         }
+#pragma unroll
+        for (int q = 0; q < 4; q++) sts128(G.chunk(GATHER_IDS + q), make_uint4(cid[4 * q], cid[4 * q + 1], cid[4 * q + 2], cid[4 * q + 3]));
         v0 = mask;               // slots still to emit
         v1 = hashed_kids << 16;  // | compact index of the next child << 8 | next slot
         nunit = 1 + (k + 2) / 3;
@@ -189,6 +212,25 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
   }
   const bool inline_ref = !force_hash && total < 32;
 
+  // starts the copies of unit u >= 1 of a LEAF or a BRANCH into the gather slot (v0, v1: the walk state before u)
+  auto gather = [&](uint32_t u) {
+    if (KIND == NK_LEAF) {
+      const uint32_t off = (u - 1) << 7;
+      const uintptr_t p = reinterpret_cast<uintptr_t>(A.val_pool + rec.z + off);
+      const uint8_t* q = reinterpret_cast<const uint8_t*>(p & ~(uintptr_t)15);  // (16-byte granules that hold a value byte)
+      const uint32_t n_chunks = ((uint32_t)(p & 15) + min(128u, v0 - off) + 15) >> 4;
+      for (uint32_t c = 0; c < n_chunks; c++) cp_async16(G.chunk(c), q + 16 * c);
+    } else {
+      const uint32_t j0 = (v1 >> 8) & 0xff, n_kids = min(3u, (uint32_t)__popc(v0));
+      for (uint32_t t = 0; t < n_kids; t++) {
+        const uint8_t* r = ref_ptr(A, G.word(4 * GATHER_IDS + j0 + t));
+        cp_async16(G.chunk(2 * t), r);
+        cp_async16(G.chunk(2 * t + 1), r + 16);
+      }
+    }
+    cp_async_commit();
+  };
+
   Stage<B> s;
   s.init(smem);
   uint64_t a[25];
@@ -200,6 +242,11 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
     if (busy) {
       // ---- fill: append whole units until a rate block is complete ----
       while (s.bytes() < 136 && unit < nunit) {
+        if (unit > 0 && (KIND == NK_LEAF || KIND == NK_BRANCH) && gathered != unit) {
+          gather(unit);
+          cp_async_wait_all();
+        }
+        gathered = 0;
         switch (KIND) {
           case NK_LEAF:
             if (unit == 0) {
@@ -207,8 +254,10 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
               emit_hex_prefix_str(s, A.key_pool + rec.y, NIB_START, NIB_LEN, 1);
               if (v1) emit_len_prefix(s, v0, 0x80, 0xb7);
             } else {
-              uint32_t off = (unit - 1) << 7;
-              emit_bytes(s, A.val_pool + rec.z + off, min(128u, v0 - off));
+              const uint32_t off = (unit - 1) << 7;
+              const uint32_t in_chunk = (uint32_t)(reinterpret_cast<uintptr_t>(A.val_pool + rec.z + off) & 15);
+              const uint32_t w0 = in_chunk >> 2;
+              emit_words(s, [&](uint32_t i) { return G.word(w0 + i); }, in_chunk & 3, min(128u, v0 - off));
             }
             break;
           case NK_LEAF_ACCOUNT: {
@@ -238,29 +287,16 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
             } else {
               // three children per unit, walked in compact order so that the lanes of a warp emit
               // their j-th child together whatever slots the children sit in
-              const uint32_t* ch = A.child_pool + rec.y;
               uint32_t j0 = (v1 >> 8) & 0xff, next_slot = v1 & 0xff;
-              uint32_t nib[3], cid[3];
-              uint4 x[3], y[3];
 #pragma unroll
               for (int t = 0; t < 3; t++) {
-                nib[t] = v0 ? (uint32_t)__ffs(v0) - 1 : 16u;
+                const uint32_t nib = v0 ? (uint32_t)__ffs(v0) - 1 : 16u;
                 v0 &= v0 - 1;
-                cid[t] = nib[t] < 16 ? __ldg(ch + j0 + t) : 0u;
-              }
-#pragma unroll
-              for (int t = 0; t < 3; t++) {  // the refs: independent loads, issued together
-                if (nib[t] < 16) {
-                  const uint4* q = reinterpret_cast<const uint4*>(ref_ptr(A, cid[t]));
-                  x[t] = __ldcg(q), y[t] = __ldcg(q + 1);
-                }
-              }
-#pragma unroll
-              for (int t = 0; t < 3; t++) {
-                if (nib[t] < 16) {
-                  emit_empty_run(s, nib[t] - next_slot);
-                  emit_ref(s, x[t], y[t], ((v1 >> (16 + j0 + t)) & 1) ? 32u : ref_len_of(A, cid[t]));
-                  next_slot = nib[t] + 1;
+                if (nib < 16) {
+                  emit_empty_run(s, nib - next_slot);
+                  const uint32_t len = ((v1 >> (16 + j0 + t)) & 1) ? 32u : ref_len_of(A, G.word(4 * GATHER_IDS + j0 + t));
+                  emit_ref(s, lds128(G.chunk(2 * t)), lds128(G.chunk(2 * t + 1)), len);
+                  next_slot = nib + 1;
                 }
               }
               if (v0 == 0) emit_empty_run(s, 17 - next_slot);  // trailing empty slots and the empty value
@@ -289,10 +325,16 @@ __global__ void __launch_bounds__(B, 4) hash_level_kernel(ArenaView A, const uin
         if (last) s.pad();
         absorb_stage<B>(a, s);
         permute = true;
+        // the next fill starts with unit `unit`: its loads run under the permutation
+        if (!last && unit < nunit && (KIND == NK_LEAF || KIND == NK_BRANCH)) {
+          gather(unit);
+          gathered = unit;
+        }
       }
     }
     if (!__any_sync(FULL, permute)) break;
     keccak_f1600(a);  // the single permutation site: the whole warp, converged
+    cp_async_wait_all();
     if (permute) {
       perms++;
       if (last) {
@@ -470,10 +512,22 @@ void launch_order_branches(const uint8_t* depth, const uint32_t* nchild_minus_1,
   counting_sort<BranchKey>(depth, nchild_minus_1, nb, BRANCH_BINS, keys, bins, order, st, 0, nullptr);
 }
 
+// Stage and gather slots exceed the 48 KB of static shared memory: the kernel takes them as dynamic shared memory,
+// with the carveout at its maximum so that four 128-thread CTAs (4 x (54 + 1) KB of the SM's 228 KB) share an SM.
+static bool hash_level_ready() {
+  static const bool once = [] {
+    bool ok = cudaFuncSetAttribute(hash_level_kernel<KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hash_smem_bytes<KB>()) == cudaSuccess;
+    ok &= cudaFuncSetAttribute(hash_level_kernel<KB>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared) == cudaSuccess;
+    return ok;
+  }();
+  return once;
+}
+
 void launch_hash_level(const ArenaView& A, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st) {
   if (end <= begin) return;
+  hash_level_ready();
   uint32_t n = end - begin;
-  hash_level_kernel<KB><<<(n + KB - 1) / KB, KB, 0, st>>>(A, order, begin, end);
+  hash_level_kernel<KB><<<(n + KB - 1) / KB, KB, hash_smem_bytes<KB>(), st>>>(A, order, begin, end);
 }
 
 }  // namespace ppd
