@@ -160,6 +160,35 @@ int ppd_trie_root_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys, uint32_t key_l
 int ppd_trie_root_leaves(ppd_ctx* ctx, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off,
                          const uint8_t* vals, size_t n, uint8_t root_out[32]);
 
+/* create_trie_subset (decoding.rs:551-602, eth_trie_utils trie_subsets.rs) of the trie over the leaves, for the m query
+ * keys: the minimal sub-trie that holds the path to every query key, each node off those paths replaced by HASH(its
+ * hash), or kept whole when it encodes to fewer than 32 bytes.  The form a pre-image takes (the Direct state trie of a
+ * DirectPreImage, every trie of a GenerationInputs), cut on the GPU from the trie the root entries build.
+ * The trie and the leaves follow the matching root entry exactly (insertion order, the last value wins,
+ * PPD_LEAVES_HASH_KEYS, the same argument checks; the sorted entry returns PPD_ERR_UNSORTED_KEYS unless the keys are
+ * strictly ascending).  Queries: m keys of key_len bytes, keccak256-hashed first under PPD_LEAVES_HASH_KEYS like the
+ * leaf keys, otherwise 32 bytes; any order, repeats allowed.  A key absent from the trie keeps the path down to where it
+ * leaves the trie (a branch with an empty slot, an extension whose nibbles differ, a leaf with another suffix): the
+ * proof of its absence.  m = 0 gives the untouched root, HASH(root) (the root of a trie of 32-byte keys always
+ * encodes to 32 bytes or more).  m >= 2^31 - 2 returns PPD_ERR_BAD_ARGUMENT.
+ * *out: one Trie in the pre-order Node form of ppd_flat.h (no header), leaves holding the value bytes as given; the
+ * empty trie gives a single PPD_NODE_EMPTY.  Release with ppd_free.  root_out: the root of the whole trie, which is also
+ * the hash of the subset.  The subset is marked, sized and written on the GPU (csrc/ppd_subset.cu) over the builder's
+ * arrays within the same call; ppd_last_stats counts its kernels in gpu_ms and kernel_launches, its copies in d2h_bytes.
+ * DEVICE pointers (keys, offsets, values and queries), complete when the call is made. */
+int ppd_trie_subset_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off,
+                               const uint8_t* d_vals, size_t n, size_t vals_bytes, const uint8_t* d_queries, size_t m,
+                               uint8_t** out, size_t* out_len, uint8_t root_out[32]);
+/* The same from host buffers. */
+int ppd_trie_subset_leaves(ppd_ctx* ctx, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off,
+                           const uint8_t* vals, size_t n, const uint8_t* queries, size_t m,
+                           uint8_t** out, size_t* out_len, uint8_t root_out[32]);
+/* The same over leaves sorted by 32-byte key (ppd_trie_root_sorted_leaves_dev: no sort), with 32-byte queries.  DEVICE
+ * pointers. */
+int ppd_trie_subset_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals,
+                                      size_t n, size_t vals_bytes, const uint8_t* d_queries32, size_t m,
+                                      uint8_t** out, size_t* out_len, uint8_t root_out[32]);
+
 /* One huge trie over several streams or GPUs (SURVEY.md 8e (3)): the leaves are split by their first `base_depth`
  * nibbles; each part is hashed like a whole trie, except that its nodes sit `base_depth` nibbles below the root
  * (ref_out = the hash of the part's top node, the 32 bytes the node above embeds).  Every key of the part must share

@@ -234,6 +234,7 @@ struct ppd_ctx {
   ppd::DevBuf d_msg, d_msg_off, d_digest;
   ppd::DevBuf d_build[13];
   ppd::DevBuf d_leaves[24];  // sort / de-duplication / gather of ppd_trie_root_leaves[_dev]
+  ppd::DevBuf d_subset[9];   // create_trie_subset of ppd_trie_subset_[sorted_]leaves[_dev] (ppd_subset.cu)
 };
 
 namespace ppd {

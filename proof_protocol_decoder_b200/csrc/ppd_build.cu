@@ -245,7 +245,8 @@ __global__ void __launch_bounds__(B, 4) hash_sorted_leaves_kernel(BuildView V) {
 // One level of branches (all at the same depth), each followed by its extension node if it has one.
 // Units of the branch message: 0 = list header, 1..4 = four child slots each (4 also carries the
 // empty value).  The extension message (header, hex-prefix nibbles, the branch's ref) is one unit.
-template <int B>
+// INNER: V.inner_ref is set (a compile-time switch: the root entries run the kernel without the stores)
+template <int B, bool INNER>
 __global__ void __launch_bounds__(B, 4) hash_branch_level_kernel(BuildView V, const uint32_t* __restrict__ order, uint32_t begin, uint32_t end) {
   __shared__ uint32_t smem[PPD_STAGE_WORDS * B];
   const uint32_t slot = begin + blockIdx.x * B + threadIdx.x;
@@ -353,6 +354,11 @@ __global__ void __launch_bounds__(B, 4) hash_branch_level_kernel(BuildView V, co
         }
       }
       if (msg_done) {
+        if (INNER && phase == 0) {
+          uint4* o = reinterpret_cast<uint4*>(V.inner_ref + 32ull * bi);
+          o[0] = rx, o[1] = ry;
+          V.inner_ref_len[bi] = (uint8_t)rlen;
+        }
         if (phase == 1 || ext_len == 0) {
           busy = false;
         } else {
@@ -419,7 +425,10 @@ void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st) {
 }
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st) {
   if (end <= begin) return;
-  hash_branch_level_kernel<HB><<<cdiv(end - begin, HB), HB, 0, st>>>(V, order, begin, end);
+  if (V.inner_ref)
+    hash_branch_level_kernel<HB, true><<<cdiv(end - begin, HB), HB, 0, st>>>(V, order, begin, end);
+  else
+    hash_branch_level_kernel<HB, false><<<cdiv(end - begin, HB), HB, 0, st>>>(V, order, begin, end);
 }
 
 }  // namespace ppd

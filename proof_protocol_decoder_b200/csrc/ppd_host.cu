@@ -587,6 +587,7 @@ void ppd_ctx_destroy(ppd_ctx* c) {
   for (DevBuf* b : bufs) b->release();
   for (DevBuf& b : c->d_build) b.release();
   for (DevBuf& b : c->d_leaves) b.release();
+  for (DevBuf& b : c->d_subset) b.release();
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->st) cudaStreamDestroy(c->st);
@@ -834,9 +835,105 @@ int ppd_block_decode(ppd_ctx* c, const uint8_t* flat, size_t len, uint8_t** out,
 // ---- trie root over sorted leaves: structure built and hashed on the GPU (ppd_build.cu) ----------
 namespace {
 
-void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n_, uint8_t root_out[32], int base_depth = 0) {
+// The keys a trie subset is cut for (ppd_trie_subset_*): m device keys of key_len bytes, keccak256-hashed first when
+// `hash`; the subset goes to *out / *out_len.
+struct SubsetQuery {
+  const uint8_t* d_keys;
+  uint32_t key_len;
+  bool hash;
+  size_t m;
+  uint8_t** out;
+  size_t* out_len;
+};
+enum { SB_QKEYS, SB_BITS, SB_LIST, SB_SO, SB_SMALL, SB_OUT, SB_IREF, SB_IREF_LEN, SB_QRAW };
+
+// create_trie_subset over the builder's arrays while they are resident (ppd_subset.cu).  end[]: the builder's branch bins
+// (depth 63 - g owns bins 16 g .. 16 g + 15).  Leaves the subset in d_subset[SB_OUT] and returns its size.
+size_t trie_subset_stage(ppd_ctx* c, const BuildView& V, uint32_t nb, const std::vector<uint32_t>& end, const SubsetQuery& q) {
+  cudaStream_t st = c->st;
+  const uint32_t n = V.n, m = (uint32_t)q.m;
+  DevBuf* D = c->d_subset;
+  SubsetView S;
+  S.keys = V.keys, S.val_off = V.val_off, S.vals = V.vals, S.n = n, S.nb = nb;
+  S.depth = V.depth, S.ext_start = V.ext_start, S.rep = V.rep, S.child = V.child, S.root_id = V.root_id;
+  S.ref = V.ref, S.ref_len = V.ref_len, S.inner_ref = V.inner_ref, S.inner_ref_len = V.inner_ref_len;
+  // a query touches at most one branch of each depth: depth d's bucket holds min(m, branches of depth d)
+  uint32_t slots = 0;
+  for (uint32_t d = 0; d < SUBSET_DEPTHS; d++) {
+    const uint32_t g = 63 - d, bd = end[16 * g + 15] - (g ? end[16 * g - 1] : 0);
+    S.base[d] = slots;
+    slots += std::min(m, bd);
+  }
+  S.base[SUBSET_DEPTHS] = slots;
+  const size_t bit_words = ((size_t)n + 2ull * nb + 31) / 32;
+  D[SB_BITS].reserve(4 * bit_words);
+  D[SB_LIST].reserve(4ull * slots + 64);
+  D[SB_SO].reserve(8ull * nb + 64);
+  D[SB_SMALL].reserve(512);  // [0, 64) counts, [64] flags, [66, 68) total
+  S.bits = D[SB_BITS].as<uint32_t>(), S.list = D[SB_LIST].as<uint32_t>(), S.so = D[SB_SO].as<uint64_t>();
+  uint32_t* small = D[SB_SMALL].as<uint32_t>();
+  S.count = small, S.flags = small + 64, S.total = reinterpret_cast<unsigned long long*>(small + 66);
+  CUDA_OK(cudaMemsetAsync(S.bits, 0, 4 * bit_words, st));
+  CUDA_OK(cudaMemsetAsync(small, 0, 512, st));
+  const uint8_t* q32 = q.d_keys;
+  if (q.hash && m) {
+    D[SB_QKEYS].reserve(32ull * m);
+    launch_hash_fixed_keys(q.d_keys, q.key_len, m, D[SB_QKEYS].as<uint8_t>(), st);
+    q32 = D[SB_QKEYS].as<uint8_t>();
+    c->stats.key_hashes += m, c->stats.key_permutations += m, c->stats.kernel_launches += 1;
+  }
+  launch_subset_mark(S, q32, m, st);
+  CUDA_OK(cudaGetLastError());
+  uint32_t count[SUBSET_DEPTHS];
+  CUDA_OK(cudaMemcpyAsync(count, small, sizeof count, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  uint32_t launches = m ? 3 : 2;
+  for (uint32_t d = SUBSET_DEPTHS; d-- > 0;)
+    if (count[d]) launch_subset_size(S, d, count[d], st), launches++;
+  launch_subset_root(S, nullptr, false, st);
+  CUDA_OK(cudaGetLastError());
+  uint32_t tail[4];  // flags, (unused), total
+  CUDA_OK(cudaMemcpyAsync(tail, small + 64, 16, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  if (tail[0] & SUBSET_F_DEEP) fail(PPD_ERR_CUDA, "internal error: an embedded subtree deeper than the subset's expansion stack");
+  uint64_t total;
+  memcpy(&total, tail + 2, 8);
+  D[SB_OUT].reserve(total + 64);
+  uint8_t* out = D[SB_OUT].as<uint8_t>();
+  launch_subset_root(S, out, true, st);
+  for (uint32_t d = 0; d < SUBSET_DEPTHS; d++)
+    if (count[d]) launch_subset_emit(S, d, count[d], out, st), launches++;
+  CUDA_OK(cudaGetLastError());
+  c->stats.kernel_launches += launches;
+  c->stats.d2h_bytes += sizeof count + 16;
+  return total;
+}
+
+// the subset of trie_subset_stage, copied to a buffer the caller releases with ppd_free
+void subset_to_host(ppd_ctx* c, size_t total, const SubsetQuery& q) {
+  uint8_t* pinned = total >= ((size_t)1 << 20) ? out_pool().take(total) : nullptr;
+  uint8_t* h = pinned ? pinned : (uint8_t*)malloc(total ? total : 1);
+  if (!h) fail(PPD_ERR_BAD_ARGUMENT, "out of host memory for the subset");
+  cudaError_t e = cudaMemcpyAsync(h, c->d_subset[SB_OUT].p, total, cudaMemcpyDeviceToHost, c->st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->st);
+  if (e != cudaSuccess) {
+    ppd_free(h);
+    throw Fail{PPD_ERR_CUDA, std::string("subset copy: ") + cudaGetErrorString(e)};
+  }
+  c->stats.d2h_bytes += (double)total;
+  *q.out = h, *q.out_len = total;
+}
+
+void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n_, uint8_t root_out[32], int base_depth = 0,
+                          const SubsetQuery* q = nullptr) {
   if (n_ == 0) {
     memcpy(root_out, EMPTY_TRIE_HASH, 32);  // HashedPartialTrie::default().hash(): keccak(0x80), types.rs:30-34
+    if (q) {
+      uint8_t* h = (uint8_t*)malloc(1);
+      if (!h) fail(PPD_ERR_BAD_ARGUMENT, "out of host memory for the subset");
+      h[0] = PPD_NODE_EMPTY;
+      *q->out = h, *q->out_len = 1;
+    }
     return;
   }
   if (n_ >= 0x7fffffffull) fail(PPD_ERR_BAD_ARGUMENT, "at most 2^31 - 2 leaves per call");
@@ -902,6 +999,12 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   V.ref_len = c->d_ref_len.as<uint8_t>();
   V.root_out = reinterpret_cast<uint8_t*>(small + 8);
   V.counters = reinterpret_cast<unsigned long long*>(small + 2);
+  V.inner_ref = nullptr, V.inner_ref_len = nullptr;
+  if (q) {
+    c->d_subset[SB_IREF].reserve(32ull * nb + 64);
+    c->d_subset[SB_IREF_LEN].reserve((size_t)nb + 64);
+    V.inner_ref = c->d_subset[SB_IREF].as<uint8_t>(), V.inner_ref_len = c->d_subset[SB_IREF_LEN].as<uint8_t>();
+  }
   D[B_NCHILD].reserve(4ull * nb + 64);
   uint32_t* nchild = D[B_NCHILD].as<uint32_t>();
   if (nb) CUDA_OK(cudaMemsetAsync(V.child, 0xff, 64ull * nb, st));
@@ -930,6 +1033,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
     begin = e;
   }
   CUDA_OK(cudaGetLastError());
+  const size_t subset_bytes = q ? trie_subset_stage(c, V, nb, end, *q) : 0;
   CUDA_OK(cudaEventRecord(c->ev1, st));
   uint32_t out[16];
   CUDA_OK(cudaMemcpyAsync(out, small, 64, cudaMemcpyDeviceToHost, st));
@@ -947,6 +1051,7 @@ void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_v
   c->stats.arena_nodes += (uint64_t)n + nb;
   c->stats.levels += levels;
   c->stats.d2h_bytes += 64 + 4096 + 8;
+  if (q) subset_to_host(c, subset_bytes, *q);
 }
 
 // ---- trie root over leaves in any order (ppd_leaves.cu): sort, keep the last of each key, gather, then the builder ----
@@ -980,13 +1085,13 @@ int sort_pairs(ppd_ctx* c, uint64_t* const k[2], uint32_t* const v[2], int in, u
 }
 
 void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
-                          size_t n_, size_t vals_bytes, uint8_t root_out[32]) {
+                          size_t n_, size_t vals_bytes, uint8_t root_out[32], const SubsetQuery* q = nullptr) {
   if (flags & ~PPD_LEAVES_HASH_KEYS) fail(PPD_ERR_BAD_ARGUMENT, "unknown flag bits");
   const bool hash = flags & PPD_LEAVES_HASH_KEYS;
   if (hash ? (key_len < 1 || key_len > 135) : key_len != 32)
     fail(PPD_ERR_BAD_ARGUMENT, hash ? "hashed keys are 1 to 135 bytes long" : "keys are 32 bytes long unless PPD_LEAVES_HASH_KEYS is set");
   if (n_ == 0) {
-    memcpy(root_out, EMPTY_TRIE_HASH, 32);
+    trie_root_sorted_dev(c, nullptr, nullptr, nullptr, 0, root_out, 0, q);
     return;
   }
   if (n_ >= 0x7fffffffull) fail(PPD_ERR_BAD_ARGUMENT, "at most 2^31 - 2 leaves per call");
@@ -1094,7 +1199,7 @@ void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, u
   CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
   c->stats.gpu_ms += ms;  // the builder adds its own part
   try {
-    trie_root_sorted_dev(c, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(), D[B_OVALS].as<uint8_t>(), kept, root_out);
+    trie_root_sorted_dev(c, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(), D[B_OVALS].as<uint8_t>(), kept, root_out, 0, q);
   } catch (const Fail& f) {
     if (f.code != PPD_ERR_UNSORTED_KEYS) throw;
     fail(PPD_ERR_CUDA, "internal error: the sorted, de-duplicated leaves are not strictly ascending (a bug of the leaf sort, or device "
@@ -1204,6 +1309,73 @@ int ppd_trie_root_leaves(ppd_ctx* c, const uint8_t* keys, uint32_t key_len, uint
     } else {
       trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out);  // the empty trie, or the argument error
     }
+  });
+}
+
+}  // extern "C"
+
+// ---- create_trie_subset of the trie over leaves (ppd_subset.cu): the root entries above, then the subset stage ----
+namespace {
+
+SubsetQuery subset_query(const uint8_t* d_queries, uint32_t key_len, uint32_t flags, size_t m, uint8_t** out, size_t* out_len) {
+  if (!out || !out_len) fail(PPD_ERR_BAD_ARGUMENT, "out and out_len are required");
+  *out = nullptr, *out_len = 0;
+  if (m >= 0x7ffffffeull) fail(PPD_ERR_BAD_ARGUMENT, "fewer than 2^31 - 2 query keys per call");
+  if (m && !d_queries) fail(PPD_ERR_BAD_ARGUMENT, "no query keys");
+  return SubsetQuery{d_queries, key_len, (flags & PPD_LEAVES_HASH_KEYS) != 0, m, out, out_len};
+}
+
+}  // namespace
+
+extern "C" {
+
+int ppd_trie_subset_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
+                               size_t n, size_t vals_bytes, const uint8_t* d_queries, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
+  return guarded(c, [&] {
+    stats_reset(c);
+    const SubsetQuery q = subset_query(d_queries, key_len, flags, m, out, out_len);
+    trie_root_leaves_dev(c, d_keys, key_len, flags, d_val_off, d_vals, n, vals_bytes, root_out, &q);
+  });
+}
+
+int ppd_trie_subset_leaves(ppd_ctx* c, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off, const uint8_t* vals, size_t n,
+                           const uint8_t* queries, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
+  return guarded(c, [&] {
+    stats_reset(c);
+    SubsetQuery q = subset_query(queries, key_len, flags, m, out, out_len);
+    if (key_len < 1 || key_len > 135) {  // the device path rejects it
+      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out, &q);
+      return;
+    }
+    if (m) {
+      c->d_subset[SB_QRAW].reserve((size_t)key_len * m);
+      CUDA_OK(cudaMemcpyAsync(c->d_subset[SB_QRAW].p, queries, (size_t)key_len * m, cudaMemcpyHostToDevice, c->st));
+      c->stats.h2d_bytes += (double)((size_t)key_len * m);
+      q.d_keys = c->d_subset[SB_QRAW].as<uint8_t>();
+    }
+    if (n && n < 0x7fffffffull) {
+      const size_t vb = val_off[n];
+      c->d_keys.reserve((size_t)key_len * n);
+      c->d_msg_off.reserve(8 * (n + 1));
+      c->d_vals.reserve(vb + 64);
+      CUDA_OK(cudaMemcpyAsync(c->d_keys.p, keys, (size_t)key_len * n, cudaMemcpyHostToDevice, c->st));
+      CUDA_OK(cudaMemcpyAsync(c->d_msg_off.p, val_off, 8 * (n + 1), cudaMemcpyHostToDevice, c->st));
+      CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
+      c->stats.h2d_bytes += (double)((size_t)key_len * n + 8 * (n + 1) + vb);
+      trie_root_leaves_dev(c, c->d_keys.as<uint8_t>(), key_len, flags, c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, vb, root_out, &q);
+    } else {
+      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out, &q);  // the empty trie, or the argument error
+    }
+  });
+}
+
+int ppd_trie_subset_sorted_leaves_dev(ppd_ctx* c, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n, size_t vals_bytes,
+                                      const uint8_t* d_queries32, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
+  (void)vals_bytes;
+  return guarded(c, [&] {
+    stats_reset(c);
+    const SubsetQuery q = subset_query(d_queries32, 32, 0, m, out, out_len);
+    trie_root_sorted_dev(c, d_keys32, d_val_off, d_vals, n, root_out, 0, &q);
   });
 }
 

@@ -78,6 +78,10 @@ struct BuildView {
   uint8_t* ref_len;          // [N + B]
   uint8_t* root_out;         // [32]
   unsigned long long* counters;
+  // optional (nullptr: not written): the ref of branch b itself, without the extension above it.  ref[N + b] is the
+  // ref of the extension when b has one; a trie subset that leaves the trie inside that extension embeds the branch.
+  uint8_t* inner_ref;        // [B][32]
+  uint8_t* inner_ref_len;    // [B]
 };
 
 void launch_lcp(const uint8_t* keys, uint32_t n, int8_t* L, uint32_t* flags, cudaStream_t st, int base_depth = 0);
@@ -88,6 +92,34 @@ void launch_branch_info(const BuildView& V, cudaStream_t st);
 void launch_child_count(const uint32_t* leader, const uint32_t* bidx, uint32_t n, uint32_t* nchild, cudaStream_t st);
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st);
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st);
+
+// ---- ppd_subset.cu: create_trie_subset over the builder's structure (ppd_trie_subset_[sorted_]leaves[_dev]) ----
+static const uint32_t SUBSET_DEPTHS = 64;  // branch depths 0 .. 63
+struct SubsetView {
+  // the builder's arrays (BuildView), read only
+  const uint8_t* keys;
+  const uint64_t* val_off;
+  const uint8_t* vals;
+  uint32_t n, nb;
+  const uint8_t *depth, *ext_start;
+  const uint32_t *rep, *child, *root_id;
+  const uint8_t *ref, *ref_len, *inner_ref, *inner_ref_len;
+  // the subset's own
+  uint32_t* bits;          // [N + 2B bits]: node id touched (leaves, branches), then N + B + b: the extension above branch b touched
+  uint32_t* list;          // touched branches, bucketed by depth: depth d owns list[base[d] .. base[d + 1])
+  uint32_t* count;         // [SUBSET_DEPTHS] touched branches of each depth
+  uint32_t base[SUBSET_DEPTHS + 1];
+  uint64_t* so;            // [B] of a touched branch: its size in the output, until its parent replaces it by its offset
+  unsigned long long* total;  // bytes of the whole subset
+  uint32_t* flags;         // SUBSET_F_*
+};
+enum : uint32_t { SUBSET_F_DEEP = 1 };  // an inline subtree deeper than the expansion stack (impossible for 32-byte refs)
+void launch_subset_mark(const SubsetView& S, const uint8_t* queries32, uint32_t m, cudaStream_t st);
+// one launch per depth: sizes deepest first (S.so = sizes), the root's offset and the total, then offsets and bytes root down
+// (count: S.count[d] as read back)
+void launch_subset_size(const SubsetView& S, uint32_t d, uint32_t count, cudaStream_t st);
+void launch_subset_root(const SubsetView& S, uint8_t* out, bool emit, cudaStream_t st);
+void launch_subset_emit(const SubsetView& S, uint32_t d, uint32_t count, uint8_t* out, cudaStream_t st);
 
 // ---- ppd_leaves.cu: leaves in any order -> the strictly ascending, de-duplicated leaves of the builder ----
 void launch_check_offsets(const uint64_t* val_off, uint32_t n, uint64_t vals_bytes, uint32_t* flag, cudaStream_t st);

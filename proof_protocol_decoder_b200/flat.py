@@ -177,6 +177,15 @@ def _node(r):
     raise ValueError("bad node kind %d" % k)
 
 
+def parse_trie(b: bytes):
+    """One Trie in the pre-order Node form (a DirectPreImage's state trie, what ppd_trie_subset_* return) -> node tuple
+    (see encode_node)"""
+    r = _R(b)
+    t = _node(r)
+    assert r.p == len(b), "trailing bytes after the Trie"
+    return t
+
+
 def parse_ir_dump(b: bytes):
     """-> list of dicts mirroring plonky2_evm GenerationInputs (decoding.rs:131-145)."""
     r = _R(b)

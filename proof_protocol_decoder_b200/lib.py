@@ -120,6 +120,9 @@ EXPORTS = [
     "ppd_direct_to_compact",
     "ppd_trie_root_leaves",
     "ppd_trie_root_leaves_dev",
+    "ppd_trie_subset_leaves",
+    "ppd_trie_subset_leaves_dev",
+    "ppd_trie_subset_sorted_leaves_dev",
 ]
 
 LEAVES_HASH_KEYS = 1  # PPD_LEAVES_HASH_KEYS: key i is keccak256 of the given key bytes
@@ -170,6 +173,10 @@ class PpdLibrary:
         L.ppd_direct_to_compact.argtypes = [ctypes.c_void_p, ctypes.c_size_t, u8pp, szp]
         L.ppd_trie_root_leaves.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_char_p]
         L.ppd_trie_root_leaves_dev.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_size_t, ctypes.c_char_p]
+        vp, sz = ctypes.c_void_p, ctypes.c_size_t
+        L.ppd_trie_subset_leaves.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
+        L.ppd_trie_subset_leaves_dev.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
+        L.ppd_trie_subset_sorted_leaves_dev.argtypes = [vp, vp, vp, vp, sz, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
 
     def exported(self):
         return [name for name in EXPORTS if hasattr(self.L, name)]
@@ -417,6 +424,47 @@ class Context:
             flags = LEAVES_HASH_KEYS if hash_keys else 0
         self._check(self.lib.L.ppd_trie_root_leaves_dev(self.h, d_keys_ptr, key_len, flags, d_val_off_ptr, d_vals_ptr, n, vals_bytes, out))
         return out.raw
+
+    def trie_subset_leaves(self, keys, val_off, vals, queries, hash_keys=False):
+        """create_trie_subset of the trie trie_root_leaves builds, for the query keys (uint8 [m, key_len], hashed like the
+        leaf keys under hash_keys; any order, repeats and absent keys allowed) -> (root, subset): the subset is one Trie in
+        the pre-order Node form of include/ppd_flat.h (flat.parse_trie reads it)."""
+        import numpy as np
+
+        keys = np.ascontiguousarray(keys, dtype=np.uint8)
+        val_off = np.ascontiguousarray(val_off, dtype=np.uint64)
+        vals = np.ascontiguousarray(vals, dtype=np.uint8)
+        queries = np.ascontiguousarray(queries, dtype=np.uint8)
+        if keys.ndim != 2 or keys.shape[0] != len(val_off) - 1:
+            raise ValueError("keys must be [n, key_len] with n = len(val_off) - 1")
+        if queries.ndim != 2 or (len(queries) and queries.shape[1] != keys.shape[1]):
+            raise ValueError("queries must be [m, key_len] with the keys' key_len")
+        root = ctypes.create_string_buffer(32)
+        out, n = ctypes.POINTER(ctypes.c_uint8)(), ctypes.c_size_t()
+        flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_subset_leaves(self.h, keys.ctypes.data, keys.shape[1], flags, val_off.ctypes.data, vals.ctypes.data, keys.shape[0],
+                                                      queries.ctypes.data, queries.shape[0], ctypes.byref(out), ctypes.byref(n), root))
+        return root.raw, self._take(out, n)
+
+    def trie_subset_leaves_dev(self, d_keys_ptr, key_len, d_val_off_ptr, d_vals_ptr, n, vals_bytes, d_queries_ptr, m, hash_keys=False, flags=None):
+        """trie_subset_leaves on device buffers (complete when it is called: torch.cuda.synchronize() first); the queries are
+        m rows of key_len bytes.  `flags` overrides hash_keys when given.  -> (root, subset)"""
+        root = ctypes.create_string_buffer(32)
+        out, nb = ctypes.POINTER(ctypes.c_uint8)(), ctypes.c_size_t()
+        if flags is None:
+            flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_subset_leaves_dev(self.h, d_keys_ptr, key_len, flags, d_val_off_ptr, d_vals_ptr, n, vals_bytes, d_queries_ptr, m,
+                                                          ctypes.byref(out), ctypes.byref(nb), root))
+        return root.raw, self._take(out, nb)
+
+    def trie_subset_sorted_leaves_dev(self, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, d_queries_ptr, m):
+        """trie_subset_leaves over leaves sorted by 32-byte key (device pointers, no sort) with m 32-byte queries.
+        -> (root, subset)"""
+        root = ctypes.create_string_buffer(32)
+        out, nb = ctypes.POINTER(ctypes.c_uint8)(), ctypes.c_size_t()
+        self._check(self.lib.L.ppd_trie_subset_sorted_leaves_dev(self.h, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, d_queries_ptr, m,
+                                                                 ctypes.byref(out), ctypes.byref(nb), root))
+        return root.raw, self._take(out, nb)
 
     def trie_subroot_sorted_leaves_dev(self, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, base_depth) -> bytes:
         """The ref of the sub-trie over n sorted leaves that share their first base_depth nibbles (device pointers)."""
