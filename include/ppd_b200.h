@@ -189,6 +189,46 @@ int ppd_trie_subset_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, con
                                       size_t n, size_t vals_bytes, const uint8_t* d_queries32, size_t m,
                                       uint8_t** out, size_t* out_len, uint8_t root_out[32]);
 
+/* A trie kept resident in HBM: built once from leaves, then cut into subsets and updated in place, each update
+ * re-hashing only the nodes on the paths of the keys it writes or deletes (csrc/gpu_trie.cu, csrc/ppd_update.cu).
+ * A handle fixes its key_len and PPD_LEAVES_HASH_KEYS when it is created; queries and update keys take the same length
+ * and are hashed the same way (the sorted create: 32-byte keys, no hashing).  A handle belongs to its context, which
+ * stays not thread-safe; other calls on the context (one-shot entries, block decodes, other handles) may come between
+ * handle calls and do not disturb it.  ppd_ctx_destroy releases every handle still alive.  A call that returns an
+ * error leaves the handle's leaves, root and subsets as they were (an out-of-memory PPD_ERR_CUDA included).  A NULL
+ * handle, or one passed with another context than the one that created it, is PPD_ERR_BAD_ARGUMENT. */
+typedef struct ppd_trie ppd_trie;
+/* Build and keep: the trie, contract and argument checks of the matching root entry (the any-order leaf entries, or
+ * the sorted device entry); root_out as they give it.  *out: the new handle.  Inputs are only borrowed for the call:
+ * the sorted create copies vals_bytes bytes of values, so it also returns PPD_ERR_BAD_ARGUMENT when val_off decreases
+ * or val_off[n] exceeds vals_bytes.  Device keys, queries and values may sit at any alignment. */
+int ppd_trie_create_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off,
+                               const uint8_t* d_vals, size_t n, size_t vals_bytes, ppd_trie** out, uint8_t root_out[32]);
+int ppd_trie_create_leaves(ppd_ctx* ctx, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off,
+                           const uint8_t* vals, size_t n, ppd_trie** out, uint8_t root_out[32]);
+int ppd_trie_create_sorted_leaves_dev(ppd_ctx* ctx, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals,
+                                      size_t n, size_t vals_bytes, ppd_trie** out, uint8_t root_out[32]);
+/* The current leaf count and root, from the host (no device work). */
+int ppd_trie_info(const ppd_trie* t, size_t* n_leaves, uint8_t root_out[32]);
+/* create_trie_subset of the current trie for m query keys; the output as the subset leaf entries give it.  Nothing is
+ * rebuilt.  DEVICE queries, or host queries. */
+int ppd_trie_subset_dev(ppd_ctx* ctx, ppd_trie* t, const uint8_t* d_queries, size_t m, uint8_t** out, size_t* out_len);
+int ppd_trie_subset(ppd_ctx* ctx, ppd_trie* t, const uint8_t* queries, size_t m, uint8_t** out, size_t* out_len);
+/* Applies k updates in input order: update i writes (key_i, vals[val_off[i] .. val_off[i + 1])), or deletes key_i when
+ * del is non-NULL and del[i] != 0 (a delete ignores its value range).  The result is that of eth_trie_utils `insert` /
+ * `delete` applied in this order: the last update of a key wins, deleting an absent key changes nothing, deleting every
+ * key gives EMPTY_TRIE_HASH.  k = 0 changes nothing and hashes nothing.  Arguments are checked as the leaf entries check
+ * them (val_off on the device, k >= 2^31 - 2 rejected), and an update that would leave 2^31 - 2 or more leaves is
+ * PPD_ERR_BAD_ARGUMENT.  root_out: the new root.  ppd_last_stats: gpu_ms covers the whole call, nodes_hashed counts the
+ * nodes the update re-hashed.  DEVICE pointers (keys, del, val_off, vals; vals_bytes = readable bytes of d_vals), or
+ * host buffers. */
+int ppd_trie_update_dev(ppd_ctx* ctx, ppd_trie* t, const uint8_t* d_keys, const uint8_t* d_del, const uint64_t* d_val_off,
+                        const uint8_t* d_vals, size_t k, size_t vals_bytes, uint8_t root_out[32]);
+int ppd_trie_update(ppd_ctx* ctx, ppd_trie* t, const uint8_t* keys, const uint8_t* del, const uint64_t* val_off,
+                    const uint8_t* vals, size_t k, uint8_t root_out[32]);
+/* Releases the handle and its device memory (NULL: no-op). */
+void ppd_trie_destroy(ppd_trie* t);
+
 /* One huge trie over several streams or GPUs (SURVEY.md 8e (3)): the leaves are split by their first `base_depth`
  * nibbles; each part is hashed like a whole trie, except that its nodes sit `base_depth` nibbles below the root
  * (ref_out = the hash of the part's top node, the 32 bytes the node above embeds).  Every key of the part must share

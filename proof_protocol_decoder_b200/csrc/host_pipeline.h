@@ -8,6 +8,8 @@
 //   gpu_pre_image.cu  witness parse + pre-image arena on the GPU (ppd_parse.cu kernels)
 //   gpu_dump.cu       IrDump serialisation on the GPU (ppd_dump.cu kernels)
 //   gpu_txn.cu        the txn loop on the GPU (ppd_txn.cu kernels)
+//   gpu_trie.cu       tries from leaves (ppd_build.cu, ppd_leaves.cu, ppd_subset.cu, ppd_update.cu kernels): the root and
+//                     subset entries and the resident trie handles
 // The host never computes a Keccak or a node encoding; there is no CPU fallback.
 #pragma once
 #include <cuda_runtime.h>
@@ -217,6 +219,22 @@ uint32_t loop_batcher_run(LoopBatcher* b, const txn::View& v, uint32_t initial_s
                           cudaEvent_t done, cudaEvent_t done_blocking);
 }  // namespace ppd
 
+namespace ppd {
+// The arrays of one trie the builder of ppd_build.cu made (BuildView): its structure, refs and branch bins.  A context
+// owns one for its one-shot root and subset entries; a trie handle owns two (the current trie, and a spare that an
+// update builds into).
+struct BuildState {
+  enum { B_L, B_M, B_LINKA, B_LINKB, B_BIDX, B_TMP, B_SMALL, B_DEPTH, B_REP, B_CHILD, B_ORDER, B_NCHILD, B_KEYS,
+         B_REF, B_REF_LEN, B_IREF, B_IREF_LEN, B_COUNT };
+  DevBuf d[B_COUNT];
+  std::vector<uint32_t> end;  // host copy of the branch bins: depth 63 - g owns bins 16 g .. 16 g + 15 (end of each)
+  uint32_t n = 0, nb = 0;     // leaves and branches of the trie last built
+  void release() {
+    for (DevBuf& b : d) b.release();
+  }
+};
+}  // namespace ppd
+
 struct ppd_ctx {
   int device = 0;
   ppd::StreamPool* pool = nullptr;      // (both null only in the host-only profiling build PPD_HOSTPROF)
@@ -232,9 +250,11 @@ struct ppd_ctx {
   // HBM buffers of the non-block entry points, grown on demand and reused across calls
   ppd::DevBuf d_keys, d_vals, d_ref, d_ref_len, d_counters;
   ppd::DevBuf d_msg, d_msg_off, d_digest;
-  ppd::DevBuf d_build[13];
-  ppd::DevBuf d_leaves[24];  // sort / de-duplication / gather of ppd_trie_root_leaves[_dev]
-  ppd::DevBuf d_subset[9];   // create_trie_subset of ppd_trie_subset_[sorted_]leaves[_dev] (ppd_subset.cu)
+  ppd::BuildState build;     // the builder's arrays of the one-shot root and subset entries
+  ppd::DevBuf d_leaves[24];  // sort / de-duplication / gather of ppd_trie_root_leaves[_dev], and an update's sort
+  ppd::DevBuf d_subset[7];   // create_trie_subset of ppd_trie_subset_* (ppd_subset.cu), and an update's marking
+  ppd::DevBuf d_merge[12];   // an update's merge and incremental hashing (ppd_update.cu)
+  std::vector<ppd_trie*> tries;  // live trie handles (gpu_trie.cu), released with the context
 };
 
 namespace ppd {
@@ -832,5 +852,26 @@ int gpu_block(ppd_ctx* c, Lane* L, Job& J, const uint8_t* flat, size_t len, uint
 bool gpu_dump_enabled();
 enum { DUMP_ON_HOST = 0, DUMP_DONE = 1 };
 int gpu_dump_block(ppd_ctx* c, Lane* L, Job& J, uint8_t** out, size_t* out_len);
+void trie_release_all(ppd_ctx* c);  // ppd_ctx_destroy: every live trie handle (gpu_trie.cu)
+
+// Runs an entry point's body: selects the context's device, and turns a Fail (or any exception) into a status code
+// and the context's error message.
+template <class F>
+int guarded(ppd_ctx* c, F f) {
+  if (!c) return PPD_ERR_BAD_ARGUMENT;
+  try {
+#ifndef PPD_HOSTPROF
+    CUDA_OK(cudaSetDevice(c->device));
+#endif
+    f();
+    return PPD_OK;
+  } catch (const Fail& e) {
+    c->err = e.msg;
+    return e.code;
+  } catch (const std::exception& e) {
+    c->err = e.what();
+    return PPD_ERR_BAD_ARGUMENT;
+  }
+}
 
 }  // namespace ppd

@@ -27,6 +27,7 @@
 #include "arena.h"
 #include "encode.cuh"
 #include "keccak.cuh"
+#include "build_leaf.cuh"
 #include "ppd_kernels.h"
 #include "pyramid.cuh"
 
@@ -149,12 +150,26 @@ __global__ void child_count_kernel(const uint32_t* __restrict__ leader, const ui
 // Both kernels loop warp-uniformly: lanes fill their stage (cheap, may diverge), then the whole warp
 // runs the single keccak_f1600 site converged; the loop ends when no lane has a block left.
 
-template <int B>
-__global__ void __launch_bounds__(B, 4) hash_sorted_leaves_kernel(BuildView V) {
+// the leaves a launch of hash_sorted_leaves_kernel hashes: all of them, or a LeafList
+__device__ __forceinline__ uint32_t leaves_of(const BuildView& V) { return V.n; }
+__device__ __forceinline__ uint32_t leaves_of(const BuildView&, LeafList l) { return l.count; }
+__device__ __forceinline__ uint32_t leaf_at(uint32_t slot) { return slot; }
+__device__ __forceinline__ uint32_t leaf_at(uint32_t slot, LeafList l) { return slot < l.count ? l.list[slot] : 0u; }
+// a leaf of the whole set is placed by the hasher; a listed leaf was placed by the update's leaf pass
+__device__ __forceinline__ void place_unlisted(const BuildView& V, uint32_t i, int dl, int dr, int dp, const uint8_t* key, bool is_root) {
+  place_leaf(V, i, dl, dr, dp, key, is_root);
+}
+__device__ __forceinline__ void place_unlisted(const BuildView&, uint32_t, int, int, int, const uint8_t*, bool, LeafList) {}
+
+// Every leaf, each placed in its parent here; or, given a LeafList (the kernel's one extra parameter), only the leaves
+// list[0 .. count), which an update's leaf pass has already placed (ppd_update.cu).  A parameter pack rather than a
+// flag, so that the root entries' instantiation keeps the single BuildView parameter.
+template <int B, class... Listed>
+__global__ void __launch_bounds__(B, 4) hash_sorted_leaves_kernel(BuildView V, Listed... listed) {
   __shared__ uint32_t smem[PPD_STAGE_WORDS * B];
-  const uint32_t i = blockIdx.x * B + threadIdx.x;
+  const uint32_t i = leaf_at(blockIdx.x * B + threadIdx.x, listed...);
   uint32_t hashed = 0, perms = 0, enc_bytes = 0;
-  bool busy = i < V.n, is_root = false;
+  bool busy = blockIdx.x * B + threadIdx.x < leaves_of(V, listed...), is_root = false;
   const uint8_t* key = nullptr;
   const uint8_t* val = nullptr;
   uint32_t nib_start = 0, nib_len = 0, vlen = 0, vhdr = 0, payload = 0, total = 0, nunit = 0, unit = 0;
@@ -164,15 +179,7 @@ __global__ void __launch_bounds__(B, 4) hash_sorted_leaves_kernel(BuildView V) {
     int dp = max(dl, dr);
     key = V.keys + 32ull * i;
     is_root = dp < V.base_depth;
-    if (is_root) {
-      *V.root_id = i;
-    } else {
-      uint32_t pl = (dl >= dr) ? i : i + 1;
-      uint32_t pb = V.bidx[V.leader[pl]];
-      uint32_t kb = __ldg(key + (dp >> 1));
-      uint32_t nib = (dp & 1) ? (kb & 15u) : (kb >> 4);
-      V.child[16ull * pb + nib] = i;
-    }
+    place_unlisted(V, i, dl, dr, dp, key, is_root, listed...);
     nib_start = (uint32_t)(dp + 1), nib_len = 64 - nib_start;
     const uint64_t vo = V.val_off[i];
     val = V.vals + vo;
@@ -422,6 +429,10 @@ void launch_child_count(const uint32_t* leader, const uint32_t* bidx, uint32_t n
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st) {
   if (!V.n) return;
   hash_sorted_leaves_kernel<HB><<<cdiv(V.n, HB), HB, 0, st>>>(V);
+}
+void launch_hash_listed_leaves(const BuildView& V, const uint32_t* list, uint32_t count, cudaStream_t st) {
+  if (!count) return;
+  hash_sorted_leaves_kernel<HB><<<cdiv(count, HB), HB, 0, st>>>(V, LeafList{list, count});
 }
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st) {
   if (end <= begin) return;

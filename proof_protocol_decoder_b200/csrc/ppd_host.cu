@@ -346,27 +346,6 @@ void fetch_pools(Lane* c, Job& J) {
 
 }  // namespace ppd
 
-namespace {
-
-template <class F>
-int guarded(ppd_ctx* c, F f) {
-  if (!c) return PPD_ERR_BAD_ARGUMENT;
-  try {
-#ifndef PPD_HOSTPROF
-    CUDA_OK(cudaSetDevice(c->device));
-#endif
-    f();
-    return PPD_OK;
-  } catch (const Fail& e) {
-    c->err = e.msg;
-    return e.code;
-  } catch (const std::exception& e) {
-    c->err = e.what();
-    return PPD_ERR_BAD_ARGUMENT;
-  }
-}
-
-}  // namespace
 
 namespace ppd {
 OutPool& out_pool() {
@@ -585,9 +564,11 @@ void ppd_ctx_destroy(ppd_ctx* c) {
   for (Lane* l : c->lanes) lane_delete(l);
   DevBuf* bufs[] = {&c->d_keys, &c->d_vals, &c->d_ref, &c->d_ref_len, &c->d_counters, &c->d_msg, &c->d_msg_off, &c->d_digest};
   for (DevBuf* b : bufs) b->release();
-  for (DevBuf& b : c->d_build) b.release();
+  trie_release_all(c);
+  c->build.release();
   for (DevBuf& b : c->d_leaves) b.release();
   for (DevBuf& b : c->d_subset) b.release();
+  for (DevBuf& b : c->d_merge) b.release();
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->st) cudaStreamDestroy(c->st);
@@ -828,555 +809,6 @@ int ppd_block_decode(ppd_ctx* c, const uint8_t* flat, size_t len, uint8_t** out,
     *out = nullptr;
   }
   return rc != PPD_OK ? rc : status;
-}
-
-}  // extern "C"
-
-// ---- trie root over sorted leaves: structure built and hashed on the GPU (ppd_build.cu) ----------
-namespace {
-
-// The keys a trie subset is cut for (ppd_trie_subset_*): m device keys of key_len bytes, keccak256-hashed first when
-// `hash`; the subset goes to *out / *out_len.
-struct SubsetQuery {
-  const uint8_t* d_keys;
-  uint32_t key_len;
-  bool hash;
-  size_t m;
-  uint8_t** out;
-  size_t* out_len;
-};
-enum { SB_QKEYS, SB_BITS, SB_LIST, SB_SO, SB_SMALL, SB_OUT, SB_IREF, SB_IREF_LEN, SB_QRAW };
-
-// create_trie_subset over the builder's arrays while they are resident (ppd_subset.cu).  end[]: the builder's branch bins
-// (depth 63 - g owns bins 16 g .. 16 g + 15).  Leaves the subset in d_subset[SB_OUT] and returns its size.
-size_t trie_subset_stage(ppd_ctx* c, const BuildView& V, uint32_t nb, const std::vector<uint32_t>& end, const SubsetQuery& q) {
-  cudaStream_t st = c->st;
-  const uint32_t n = V.n, m = (uint32_t)q.m;
-  DevBuf* D = c->d_subset;
-  SubsetView S;
-  S.keys = V.keys, S.val_off = V.val_off, S.vals = V.vals, S.n = n, S.nb = nb;
-  S.depth = V.depth, S.ext_start = V.ext_start, S.rep = V.rep, S.child = V.child, S.root_id = V.root_id;
-  S.ref = V.ref, S.ref_len = V.ref_len, S.inner_ref = V.inner_ref, S.inner_ref_len = V.inner_ref_len;
-  // a query touches at most one branch of each depth: depth d's bucket holds min(m, branches of depth d)
-  uint32_t slots = 0;
-  for (uint32_t d = 0; d < SUBSET_DEPTHS; d++) {
-    const uint32_t g = 63 - d, bd = end[16 * g + 15] - (g ? end[16 * g - 1] : 0);
-    S.base[d] = slots;
-    slots += std::min(m, bd);
-  }
-  S.base[SUBSET_DEPTHS] = slots;
-  const size_t bit_words = ((size_t)n + 2ull * nb + 31) / 32;
-  D[SB_BITS].reserve(4 * bit_words);
-  D[SB_LIST].reserve(4ull * slots + 64);
-  D[SB_SO].reserve(8ull * nb + 64);
-  D[SB_SMALL].reserve(512);  // [0, 64) counts, [64] flags, [66, 68) total
-  S.bits = D[SB_BITS].as<uint32_t>(), S.list = D[SB_LIST].as<uint32_t>(), S.so = D[SB_SO].as<uint64_t>();
-  uint32_t* small = D[SB_SMALL].as<uint32_t>();
-  S.count = small, S.flags = small + 64, S.total = reinterpret_cast<unsigned long long*>(small + 66);
-  CUDA_OK(cudaMemsetAsync(S.bits, 0, 4 * bit_words, st));
-  CUDA_OK(cudaMemsetAsync(small, 0, 512, st));
-  const uint8_t* q32 = q.d_keys;
-  if (q.hash && m) {
-    D[SB_QKEYS].reserve(32ull * m);
-    launch_hash_fixed_keys(q.d_keys, q.key_len, m, D[SB_QKEYS].as<uint8_t>(), st);
-    q32 = D[SB_QKEYS].as<uint8_t>();
-    c->stats.key_hashes += m, c->stats.key_permutations += m, c->stats.kernel_launches += 1;
-  }
-  launch_subset_mark(S, q32, m, st);
-  CUDA_OK(cudaGetLastError());
-  uint32_t count[SUBSET_DEPTHS];
-  CUDA_OK(cudaMemcpyAsync(count, small, sizeof count, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  uint32_t launches = m ? 3 : 2;
-  for (uint32_t d = SUBSET_DEPTHS; d-- > 0;)
-    if (count[d]) launch_subset_size(S, d, count[d], st), launches++;
-  launch_subset_root(S, nullptr, false, st);
-  CUDA_OK(cudaGetLastError());
-  uint32_t tail[4];  // flags, (unused), total
-  CUDA_OK(cudaMemcpyAsync(tail, small + 64, 16, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  if (tail[0] & SUBSET_F_DEEP) fail(PPD_ERR_CUDA, "internal error: an embedded subtree deeper than the subset's expansion stack");
-  uint64_t total;
-  memcpy(&total, tail + 2, 8);
-  D[SB_OUT].reserve(total + 64);
-  uint8_t* out = D[SB_OUT].as<uint8_t>();
-  launch_subset_root(S, out, true, st);
-  for (uint32_t d = 0; d < SUBSET_DEPTHS; d++)
-    if (count[d]) launch_subset_emit(S, d, count[d], out, st), launches++;
-  CUDA_OK(cudaGetLastError());
-  c->stats.kernel_launches += launches;
-  c->stats.d2h_bytes += sizeof count + 16;
-  return total;
-}
-
-// the subset of trie_subset_stage, copied to a buffer the caller releases with ppd_free
-void subset_to_host(ppd_ctx* c, size_t total, const SubsetQuery& q) {
-  uint8_t* pinned = total >= ((size_t)1 << 20) ? out_pool().take(total) : nullptr;
-  uint8_t* h = pinned ? pinned : (uint8_t*)malloc(total ? total : 1);
-  if (!h) fail(PPD_ERR_BAD_ARGUMENT, "out of host memory for the subset");
-  cudaError_t e = cudaMemcpyAsync(h, c->d_subset[SB_OUT].p, total, cudaMemcpyDeviceToHost, c->st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->st);
-  if (e != cudaSuccess) {
-    ppd_free(h);
-    throw Fail{PPD_ERR_CUDA, std::string("subset copy: ") + cudaGetErrorString(e)};
-  }
-  c->stats.d2h_bytes += (double)total;
-  *q.out = h, *q.out_len = total;
-}
-
-void trie_root_sorted_dev(ppd_ctx* c, const uint8_t* d_keys, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n_, uint8_t root_out[32], int base_depth = 0,
-                          const SubsetQuery* q = nullptr) {
-  if (n_ == 0) {
-    memcpy(root_out, EMPTY_TRIE_HASH, 32);  // HashedPartialTrie::default().hash(): keccak(0x80), types.rs:30-34
-    if (q) {
-      uint8_t* h = (uint8_t*)malloc(1);
-      if (!h) fail(PPD_ERR_BAD_ARGUMENT, "out of host memory for the subset");
-      h[0] = PPD_NODE_EMPTY;
-      *q->out = h, *q->out_len = 1;
-    }
-    return;
-  }
-  if (n_ >= 0x7fffffffull) fail(PPD_ERR_BAD_ARGUMENT, "at most 2^31 - 2 leaves per call");
-  const uint32_t n = (uint32_t)n_;
-  cudaStream_t st = c->st;
-  const uint32_t n1 = (n + 1 + 63) / 64, n2 = (n1 + 63) / 64, n3 = (n2 + 63) / 64;
-  enum { B_L, B_M, B_LINKA, B_LINKB, B_BIDX, B_TMP, B_SMALL, B_DEPTH, B_REP, B_CHILD, B_ORDER, B_NCHILD, B_KEYS };
-  DevBuf* D = c->d_build;
-  D[B_L].reserve((size_t)n + 1 + 64);
-  D[B_M].reserve((size_t)n1 + n2 + n3 + 192);
-  D[B_LINKA].reserve(4ull * (n + 1));
-  D[B_LINKB].reserve(4ull * (n + 1));
-  D[B_BIDX].reserve(4ull * (n + 1));
-  D[B_TMP].reserve(4ull * scan_tmp_words((size_t)n + 1));
-  D[B_SMALL].reserve(16384);
-  int8_t* L = D[B_L].as<int8_t>();
-  int8_t* m1 = D[B_M].as<int8_t>();
-  int8_t* m2 = m1 + ((n1 + 63) & ~63u);
-  int8_t* m3 = m2 + ((n2 + 63) & ~63u);
-  uint32_t* small = D[B_SMALL].as<uint32_t>();  // [0] error flags, [1] root id, [2..7] counters(u64 x 3), [8..15] root, [1024..2047] branch bins
-  CUDA_OK(cudaMemsetAsync(small, 0, 16384, st));
-  CUDA_OK(cudaEventRecord(c->ev0, st));
-  launch_lcp(d_keys, n, L, small + 0, st, base_depth);
-  launch_min64(L, n + 1, m1, n1, st);
-  launch_min64(m1, n1, m2, n2, st);
-  launch_min64(m2, n2, m3, n3, st);
-  uint32_t* leader = D[B_LINKA].as<uint32_t>();
-  uint32_t* flag = D[B_LINKB].as<uint32_t>();
-  launch_leaders(L, m1, m2, m3, n, leader, flag, flag, st);
-  uint32_t* bidx = D[B_BIDX].as<uint32_t>();
-  exclusive_scan(flag, bidx, n + 1, D[B_TMP].as<uint32_t>(), st);
-  CUDA_OK(cudaGetLastError());
-  uint32_t h_flags = 0, nb = 0;
-  CUDA_OK(cudaMemcpyAsync(&h_flags, small, 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaMemcpyAsync(&nb, bidx + n, 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  if (h_flags & BUILD_F_UNSORTED) fail(PPD_ERR_UNSORTED_KEYS, "keys are not strictly ascending");
-  if (h_flags & BUILD_F_PREFIX) fail(PPD_ERR_BAD_ARGUMENT, "the keys of a sub-trie do not share their first base_depth nibbles");
-  c->stats.kernel_launches += 11 + 3;
-
-  D[B_DEPTH].reserve(2ull * nb + 64);
-  D[B_REP].reserve(4ull * nb + 64);
-  D[B_CHILD].reserve(64ull * nb + 64);
-  D[B_ORDER].reserve(4ull * nb + 64);
-  c->d_ref.reserve(32ull * ((size_t)n + nb));
-  c->d_ref_len.reserve((size_t)n + nb);
-  BuildView V;
-  V.keys = d_keys;
-  V.val_off = d_val_off;
-  V.vals = d_vals;
-  V.n = n;
-  V.base_depth = base_depth;
-  V.P = Pyramid{L, m1, m2, m3};
-  V.leader = leader;
-  V.bidx = bidx;
-  V.depth = D[B_DEPTH].as<uint8_t>();
-  V.ext_start = V.depth + nb + 32;
-  V.rep = D[B_REP].as<uint32_t>();
-  V.child = D[B_CHILD].as<uint32_t>();
-  V.root_id = small + 1;
-  V.flags = small + 0;
-  V.ref =c->d_ref.as<uint8_t>();
-  V.ref_len = c->d_ref_len.as<uint8_t>();
-  V.root_out = reinterpret_cast<uint8_t*>(small + 8);
-  V.counters = reinterpret_cast<unsigned long long*>(small + 2);
-  V.inner_ref = nullptr, V.inner_ref_len = nullptr;
-  if (q) {
-    c->d_subset[SB_IREF].reserve(32ull * nb + 64);
-    c->d_subset[SB_IREF_LEN].reserve((size_t)nb + 64);
-    V.inner_ref = c->d_subset[SB_IREF].as<uint8_t>(), V.inner_ref_len = c->d_subset[SB_IREF_LEN].as<uint8_t>();
-  }
-  D[B_NCHILD].reserve(4ull * nb + 64);
-  uint32_t* nchild = D[B_NCHILD].as<uint32_t>();
-  if (nb) CUDA_OK(cudaMemsetAsync(V.child, 0xff, 64ull * nb, st));
-  if (nb) CUDA_OK(cudaMemsetAsync(nchild, 0, 4ull * nb, st));
-  launch_branch_info(V, st);
-  launch_child_count(leader, bidx, n, nchild, st);
-  // counting sort by (depth, number of children), deepest depth first: the lanes of a warp walk the same number of
-  // children and run the same number of permutations
-  D[B_KEYS].reserve(2ull * nb + 64);
-  uint32_t* order = D[B_ORDER].as<uint32_t>();
-  launch_order_branches(V.depth, nchild, nb, D[B_KEYS].as<uint16_t>(), small + 1024, order, st);
-  launch_hash_sorted_leaves(V, st);
-  c->stats.kernel_launches += 6;
-  std::vector<uint32_t> end(BRANCH_BINS);  // end of every bucket: depth 63 - g owns buckets 16 g .. 16 g + 15
-  CUDA_OK(cudaMemcpyAsync(end.data(), small + 1024, 4 * BRANCH_BINS, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  if (end[BRANCH_BINS - 1] != nb) fail(PPD_ERR_CUDA, "branch histogram does not add up");
-  uint32_t levels = 1;
-  for (uint32_t g = 0, begin = 0; g < 64; g++) {
-    const uint32_t e = end[16 * g + 15];
-    if (e > begin) {
-      launch_hash_branch_level(V, order, begin, e, st);
-      c->stats.kernel_launches++;
-      levels++;
-    }
-    begin = e;
-  }
-  CUDA_OK(cudaGetLastError());
-  const size_t subset_bytes = q ? trie_subset_stage(c, V, nb, end, *q) : 0;
-  CUDA_OK(cudaEventRecord(c->ev1, st));
-  uint32_t out[16];
-  CUDA_OK(cudaMemcpyAsync(out, small, 64, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  if (out[0] & BUILD_F_SHORT_TOP) fail(PPD_ERR_BAD_ARGUMENT, "the sub-trie's top node encodes to fewer than 32 bytes: its parent embeds it, not its hash");
-  memcpy(root_out, out + 8, 32);
-  float ms = 0;
-  CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  unsigned long long cnt[3];
-  memcpy(cnt, out + 2, 24);
-  c->stats.gpu_ms += ms;
-  c->stats.nodes_hashed += cnt[0];
-  c->stats.node_permutations += cnt[1];
-  c->stats.node_bytes += cnt[2];
-  c->stats.arena_nodes += (uint64_t)n + nb;
-  c->stats.levels += levels;
-  c->stats.d2h_bytes += 64 + 4096 + 8;
-  if (q) subset_to_host(c, subset_bytes, *q);
-}
-
-// ---- trie root over leaves in any order (ppd_leaves.cu): sort, keep the last of each key, gather, then the builder ----
-
-// byte digits of the n keys that take more than one value (bit p: digit p): the passes a sort cannot skip
-uint32_t varying_digits(ppd_ctx* c, const uint64_t* keys, uint32_t n, uint32_t* counts) {
-  CUDA_OK(cudaMemsetAsync(counts, 0, 8 * 256 * 4, c->st));
-  launch_digit_counts(keys, n, counts, c->st);
-  CUDA_OK(cudaGetLastError());
-  std::vector<uint32_t> h(8 * 256);
-  CUDA_OK(cudaMemcpyAsync(h.data(), counts, 8 * 256 * 4, cudaMemcpyDeviceToHost, c->st));
-  CUDA_OK(cudaStreamSynchronize(c->st));
-  c->stats.kernel_launches += 1;
-  c->stats.d2h_bytes += 8 * 256 * 4;
-  uint32_t mask = 0;
-  for (int p = 0; p < 8; p++)
-    if (std::find(h.begin() + 256 * p, h.begin() + 256 * (p + 1), n) == h.begin() + 256 * (p + 1)) mask |= 1u << p;
-  return mask;
-}
-
-// stable LSD radix sort of the pairs (k[in][i], v[in][i]) by key over the digits of `digits`; k[1 - in] / v[1 - in] are the
-// other halves of the ping-pong.  Returns which half holds the result.
-int sort_pairs(ppd_ctx* c, uint64_t* const k[2], uint32_t* const v[2], int in, uint32_t n, uint32_t digits, uint32_t* hist, uint32_t* tmp) {
-  for (int p = 0; p < 8; p++) {
-    if (!(digits & (1u << p))) continue;
-    c->stats.kernel_launches += launch_radix_pass(k[in], v[in], k[1 - in], v[1 - in], n, p, hist, hist + radix_hist_words(n), tmp, c->st);
-    in = 1 - in;
-  }
-  CUDA_OK(cudaGetLastError());
-  return in;
-}
-
-void trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
-                          size_t n_, size_t vals_bytes, uint8_t root_out[32], const SubsetQuery* q = nullptr) {
-  if (flags & ~PPD_LEAVES_HASH_KEYS) fail(PPD_ERR_BAD_ARGUMENT, "unknown flag bits");
-  const bool hash = flags & PPD_LEAVES_HASH_KEYS;
-  if (hash ? (key_len < 1 || key_len > 135) : key_len != 32)
-    fail(PPD_ERR_BAD_ARGUMENT, hash ? "hashed keys are 1 to 135 bytes long" : "keys are 32 bytes long unless PPD_LEAVES_HASH_KEYS is set");
-  if (n_ == 0) {
-    trie_root_sorted_dev(c, nullptr, nullptr, nullptr, 0, root_out, 0, q);
-    return;
-  }
-  if (n_ >= 0x7fffffffull) fail(PPD_ERR_BAD_ARGUMENT, "at most 2^31 - 2 leaves per call");
-  const uint32_t n = (uint32_t)n_;
-  cudaStream_t st = c->st;
-  enum { B_HKEYS, B_K0, B_K1, B_V0, B_V1, B_V2, B_TIE, B_MEMBER, B_MPOS, B_START, B_SPOS, B_CPOS, B_CIDX, B_CRUN, B_CWORD,
-         B_LEN, B_KOFF, B_HIST, B_TMP, B_TMP64, B_SMALL, B_OKEYS, B_OOFF, B_OVALS };
-  DevBuf* D = c->d_leaves;
-  const size_t hist_words = radix_hist_words(n);
-  for (int b : {B_K0, B_K1, B_CWORD}) D[b].reserve(8ull * n);
-  for (int b : {B_V0, B_V1, B_V2, B_CPOS, B_CIDX, B_CRUN}) D[b].reserve(4ull * n);
-  for (int b : {B_TIE, B_MEMBER, B_MPOS, B_START, B_SPOS}) D[b].reserve(4ull * (n + 1));
-  for (int b : {B_LEN, B_KOFF}) D[b].reserve(8ull * (n + 1));
-  D[B_HIST].reserve(4 * 2 * hist_words);
-  D[B_TMP].reserve(4 * scan_tmp_words(std::max<size_t>(hist_words, (size_t)n + 1)));
-  D[B_TMP64].reserve(8 * scan_tmp_words((size_t)n + 1));
-  D[B_SMALL].reserve(16384);
-  uint32_t* small = D[B_SMALL].as<uint32_t>();  // [0] bad offsets, [1] ties, [2] members and [3] runs (read back), [1024..3071] digit counts
-  uint32_t* hist = D[B_HIST].as<uint32_t>();
-  uint32_t* tmp = D[B_TMP].as<uint32_t>();
-  uint64_t* const K[2] = {D[B_K0].as<uint64_t>(), D[B_K1].as<uint64_t>()};
-  uint32_t* tie = D[B_TIE].as<uint32_t>();
-
-  CUDA_OK(cudaMemsetAsync(small, 0, 4096, st));
-  CUDA_OK(cudaEventRecord(c->ev0, st));
-  launch_check_offsets(d_val_off, n, vals_bytes, small + 0, st);
-  const uint8_t* keys32 = d_keys;
-  if (hash) {
-    D[B_HKEYS].reserve(32ull * n);
-    launch_hash_fixed_keys(d_keys, key_len, n, D[B_HKEYS].as<uint8_t>(), st);
-    keys32 = D[B_HKEYS].as<uint8_t>();
-    c->stats.key_hashes = n, c->stats.key_permutations = n, c->stats.kernel_launches += 1;
-  }
-  // the whole set on word 0: (word, input position) pairs
-  launch_key_word(keys32, n, 0, K[0], D[B_V0].as<uint32_t>(), st);
-  c->stats.kernel_launches += 2;
-  uint32_t digits = varying_digits(c, K[0], n, small + 1024);
-  uint32_t bad = 0;
-  CUDA_OK(cudaMemcpyAsync(&bad, small + 0, 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  if (bad) fail(PPD_ERR_BAD_ARGUMENT, "val_off decreases somewhere or val_off[n] exceeds vals_bytes");
-  uint32_t* const V01[2] = {D[B_V0].as<uint32_t>(), D[B_V1].as<uint32_t>()};
-  const int r0 = sort_pairs(c, K, V01, 0, n, digits, hist, tmp);
-  uint32_t* idx = V01[r0];  // input position of the element at each sorted position
-  launch_tie_flags(K[r0], n, tie, small + 1, st);
-  uint32_t ties = 0;
-  CUDA_OK(cudaMemcpyAsync(&ties, small + 1, 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  c->stats.kernel_launches += 1;
-  c->stats.d2h_bytes += 8;
-
-  // refine the runs that tie on the words so far by the next word; runs keep their positions, so only their members move
-  TieRuns R;
-  R.member = D[B_MEMBER].as<uint32_t>(), R.mpos = D[B_MPOS].as<uint32_t>(), R.start = D[B_START].as<uint32_t>(), R.spos = D[B_SPOS].as<uint32_t>();
-  R.cpos = D[B_CPOS].as<uint32_t>(), R.cidx = D[B_CIDX].as<uint32_t>(), R.crun = D[B_CRUN].as<uint32_t>(), R.cword = D[B_CWORD].as<uint64_t>();
-  uint32_t* const VR[2] = {V01[1 - r0], D[B_V2].as<uint32_t>()};
-  for (int w = 1; w < 4 && ties; w++) {
-    launch_tie_members(tie, n, R.member, R.start, st);
-    uint32_t scans = exclusive_scan(R.member, R.mpos, n + 1, tmp, st);
-    scans += exclusive_scan(R.start, R.spos, n + 1, tmp, st);
-    launch_tie_compact(R, keys32, idx, n, w, K[0], VR[0], st);
-    CUDA_OK(cudaMemcpyAsync(small + 2, R.mpos + n, 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_OK(cudaMemcpyAsync(small + 3, R.spos + n, 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_OK(cudaMemsetAsync(small + 1, 0, 4, st));
-    uint32_t mr[2];
-    CUDA_OK(cudaMemcpyAsync(mr, small + 2, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_OK(cudaStreamSynchronize(st));
-    const uint32_t m = mr[0], runs = mr[1];
-    c->stats.kernel_launches += 2 + scans;
-    c->stats.d2h_bytes += 8;
-    // sort A: the members by the word; sort B: stably by run (the digits a run id below `runs` can have)
-    const int ra = sort_pairs(c, K, VR, 0, m, varying_digits(c, K[0], m, small + 1024), hist, tmp);
-    launch_tie_run_key(R, VR[ra], m, K[1 - ra], VR[1 - ra], st);
-    uint32_t run_digits = 0;
-    for (int p = 0; p < 4; p++)
-      if ((uint64_t)(runs - 1) >> (8 * p)) run_digits |= 1u << p;
-    const int rb = sort_pairs(c, K, VR, 1 - ra, m, run_digits, hist, tmp);
-    launch_tie_writeback(R, VR[rb], m, idx, tie, small + 1, st);
-    CUDA_OK(cudaGetLastError());
-    CUDA_OK(cudaMemcpyAsync(&ties, small + 1, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_OK(cudaStreamSynchronize(st));
-    c->stats.kernel_launches += 2;
-    c->stats.d2h_bytes += 4;
-  }
-
-  // the last occurrence of every key, packed: sorted keys32, offsets, values
-  const uint32_t kept = n - ties;
-  uint32_t* keep = R.member;
-  uint32_t* kpos = R.mpos;
-  uint64_t* len = D[B_LEN].as<uint64_t>();
-  uint64_t* koff = D[B_KOFF].as<uint64_t>();
-  launch_keep_last(tie, idx, d_val_off, n, keep, len, st);
-  uint32_t scans = exclusive_scan(keep, kpos, n + 1, tmp, st);
-  scans += exclusive_scan(len, koff, n + 1, D[B_TMP64].as<uint64_t>(), st);
-  c->stats.kernel_launches += 2 + scans;
-  D[B_OKEYS].reserve(32ull * kept);
-  D[B_OOFF].reserve(8ull * (kept + 1));
-  D[B_OVALS].reserve(vals_bytes + 64);  // the kept values add up to at most val_off[n] - val_off[0] <= vals_bytes
-  launch_gather_leaves(keys32, idx, d_val_off, d_vals, n, keep, kpos, koff, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(),
-                       D[B_OVALS].as<uint8_t>(), st);
-  CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaEventRecord(c->ev1, st));
-  CUDA_OK(cudaEventSynchronize(c->ev1));
-  float ms = 0;
-  CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->stats.gpu_ms += ms;  // the builder adds its own part
-  try {
-    trie_root_sorted_dev(c, D[B_OKEYS].as<uint8_t>(), D[B_OOFF].as<uint64_t>(), D[B_OVALS].as<uint8_t>(), kept, root_out, 0, q);
-  } catch (const Fail& f) {
-    if (f.code != PPD_ERR_UNSORTED_KEYS) throw;
-    fail(PPD_ERR_CUDA, "internal error: the sorted, de-duplicated leaves are not strictly ascending (a bug of the leaf sort, or device "
-         "inputs that changed during the call)");
-  }
-}
-
-}  // namespace
-
-extern "C" {
-
-int ppd_trie_root_sorted_leaves_dev(ppd_ctx* c, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n,
-                                    size_t vals_bytes, uint8_t root_out[32]) {
-  (void)vals_bytes;
-  return guarded(c, [&] {
-    stats_reset(c);
-    trie_root_sorted_dev(c, d_keys32, d_val_off, d_vals, n, root_out);
-  });
-}
-
-int ppd_trie_subroot_sorted_leaves_dev(ppd_ctx* c, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n,
-                                       size_t vals_bytes, uint32_t base_depth, uint8_t ref_out[32]) {
-  (void)vals_bytes;
-  return guarded(c, [&] {
-    stats_reset(c);
-    if (base_depth >= 64 || n == 0) fail(PPD_ERR_BAD_ARGUMENT, "a sub-trie needs leaves and a base depth below 64");
-    trie_root_sorted_dev(c, d_keys32, d_val_off, d_vals, n, ref_out, (int)base_depth);
-  });
-}
-
-// The branch over up to 16 hashed children (the top of a trie whose sub-tries were hashed apart, on other streams or
-// other GPUs): a three-node arena (16 hash-pool entries, the branch, its ROOT) through the ordinary level kernel.
-int ppd_trie_root_from_children(ppd_ctx* c, const uint8_t* child_hashes16x32, uint32_t mask, uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    mask &= 0xffffu;
-    if (__builtin_popcount(mask) < 2) fail(PPD_ERR_BAD_ARGUMENT, "a branch has at least two children");
-    NodeRec nodes[2];
-    uint32_t kids[16], k = 0;
-    for (uint32_t i = 0; i < 16; i++)
-      if (mask & (1u << i)) kids[k++] = HASH_ID_BASE + i;
-    nodes[0] = NodeRec{node_w0(NK_BRANCH, 0, 0), 0, mask, 0};
-    nodes[1] = NodeRec{node_w0(NK_ROOT, 0, 0), 0, 0, 0};
-    c->d_keys.reserve(4096), c->d_vals.reserve(4096), c->d_ref.reserve(4096), c->d_ref_len.reserve(256), c->d_counters.reserve(32);
-    c->d_msg.reserve(4096);  // hash pool, nodes, children
-    uint8_t* base = c->d_msg.as<uint8_t>();
-    CUDA_OK(cudaMemcpyAsync(base, child_hashes16x32, 512, cudaMemcpyHostToDevice, c->st));
-    CUDA_OK(cudaMemcpyAsync(base + 512, nodes, sizeof nodes, cudaMemcpyHostToDevice, c->st));
-    CUDA_OK(cudaMemcpyAsync(base + 1024, kids, 4 * k, cudaMemcpyHostToDevice, c->st));
-    CUDA_OK(cudaMemsetAsync(c->d_counters.p, 0, 32, c->st));
-    ArenaView V{};
-    V.nodes = reinterpret_cast<const NodeRec*>(base + 512), V.hash_pool = base, V.child_pool = reinterpret_cast<const uint32_t*>(base + 1024);
-    V.key_pool = c->d_keys.as<uint8_t>(), V.val_pool = c->d_vals.as<uint8_t>(), V.accounts = nullptr;
-    V.ref = c->d_ref.as<uint8_t>(), V.ref_len = c->d_ref_len.as<uint8_t>(), V.counters = c->d_counters.as<unsigned long long>();
-    launch_hash_level(V, nullptr, 0, 1, c->st);
-    launch_hash_level(V, nullptr, 1, 2, c->st);
-    CUDA_OK(cudaGetLastError());
-    CUDA_OK(cudaMemcpyAsync(root_out, V.ref + 32, 32, cudaMemcpyDeviceToHost, c->st));
-    CUDA_OK(cudaStreamSynchronize(c->st));
-    c->stats.nodes_hashed = 2, c->stats.kernel_launches = 2;
-  });
-}
-
-int ppd_trie_root_sorted_leaves(ppd_ctx* c, const uint8_t* keys32, const uint64_t* val_off, const uint8_t* vals, size_t n,
-                                uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    if (!n) {
-      trie_root_sorted_dev(c, nullptr, nullptr, nullptr, 0, root_out);
-      return;
-    }
-    size_t vb = val_off[n];
-    c->d_keys.reserve(32 * n);
-    c->d_msg_off.reserve(8 * (n + 1));
-    c->d_vals.reserve(vb + 64);
-    CUDA_OK(cudaMemcpyAsync(c->d_keys.p, keys32, 32 * n, cudaMemcpyHostToDevice, c->st));
-    CUDA_OK(cudaMemcpyAsync(c->d_msg_off.p, val_off, 8 * (n + 1), cudaMemcpyHostToDevice, c->st));
-    CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
-    c->stats.h2d_bytes += (double)(32 * n + 8 * (n + 1) + vb);
-    trie_root_sorted_dev(c, c->d_keys.as<uint8_t>(), c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, root_out);
-  });
-}
-
-int ppd_trie_root_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
-                             size_t n, size_t vals_bytes, uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    trie_root_leaves_dev(c, d_keys, key_len, flags, d_val_off, d_vals, n, vals_bytes, root_out);
-  });
-}
-
-int ppd_trie_root_leaves(ppd_ctx* c, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off, const uint8_t* vals, size_t n,
-                         uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    if (n && n < 0x7fffffffull && key_len >= 1 && key_len <= 135) {
-      // upload, then the device path checks everything (the offsets included: vals_bytes is what the caller says val_off[n] is)
-      const size_t vb = val_off[n];
-      c->d_keys.reserve((size_t)key_len * n);
-      c->d_msg_off.reserve(8 * (n + 1));
-      c->d_vals.reserve(vb + 64);
-      CUDA_OK(cudaMemcpyAsync(c->d_keys.p, keys, (size_t)key_len * n, cudaMemcpyHostToDevice, c->st));
-      CUDA_OK(cudaMemcpyAsync(c->d_msg_off.p, val_off, 8 * (n + 1), cudaMemcpyHostToDevice, c->st));
-      CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
-      c->stats.h2d_bytes += (double)((size_t)key_len * n + 8 * (n + 1) + vb);
-      trie_root_leaves_dev(c, c->d_keys.as<uint8_t>(), key_len, flags, c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, vb, root_out);
-    } else {
-      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out);  // the empty trie, or the argument error
-    }
-  });
-}
-
-}  // extern "C"
-
-// ---- create_trie_subset of the trie over leaves (ppd_subset.cu): the root entries above, then the subset stage ----
-namespace {
-
-SubsetQuery subset_query(const uint8_t* d_queries, uint32_t key_len, uint32_t flags, size_t m, uint8_t** out, size_t* out_len) {
-  if (!out || !out_len) fail(PPD_ERR_BAD_ARGUMENT, "out and out_len are required");
-  *out = nullptr, *out_len = 0;
-  if (m >= 0x7ffffffeull) fail(PPD_ERR_BAD_ARGUMENT, "fewer than 2^31 - 2 query keys per call");
-  if (m && !d_queries) fail(PPD_ERR_BAD_ARGUMENT, "no query keys");
-  return SubsetQuery{d_queries, key_len, (flags & PPD_LEAVES_HASH_KEYS) != 0, m, out, out_len};
-}
-
-}  // namespace
-
-extern "C" {
-
-int ppd_trie_subset_leaves_dev(ppd_ctx* c, const uint8_t* d_keys, uint32_t key_len, uint32_t flags, const uint64_t* d_val_off, const uint8_t* d_vals,
-                               size_t n, size_t vals_bytes, const uint8_t* d_queries, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    const SubsetQuery q = subset_query(d_queries, key_len, flags, m, out, out_len);
-    trie_root_leaves_dev(c, d_keys, key_len, flags, d_val_off, d_vals, n, vals_bytes, root_out, &q);
-  });
-}
-
-int ppd_trie_subset_leaves(ppd_ctx* c, const uint8_t* keys, uint32_t key_len, uint32_t flags, const uint64_t* val_off, const uint8_t* vals, size_t n,
-                           const uint8_t* queries, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
-  return guarded(c, [&] {
-    stats_reset(c);
-    SubsetQuery q = subset_query(queries, key_len, flags, m, out, out_len);
-    if (key_len < 1 || key_len > 135) {  // the device path rejects it
-      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out, &q);
-      return;
-    }
-    if (m) {
-      c->d_subset[SB_QRAW].reserve((size_t)key_len * m);
-      CUDA_OK(cudaMemcpyAsync(c->d_subset[SB_QRAW].p, queries, (size_t)key_len * m, cudaMemcpyHostToDevice, c->st));
-      c->stats.h2d_bytes += (double)((size_t)key_len * m);
-      q.d_keys = c->d_subset[SB_QRAW].as<uint8_t>();
-    }
-    if (n && n < 0x7fffffffull) {
-      const size_t vb = val_off[n];
-      c->d_keys.reserve((size_t)key_len * n);
-      c->d_msg_off.reserve(8 * (n + 1));
-      c->d_vals.reserve(vb + 64);
-      CUDA_OK(cudaMemcpyAsync(c->d_keys.p, keys, (size_t)key_len * n, cudaMemcpyHostToDevice, c->st));
-      CUDA_OK(cudaMemcpyAsync(c->d_msg_off.p, val_off, 8 * (n + 1), cudaMemcpyHostToDevice, c->st));
-      CUDA_OK(cudaMemcpyAsync(c->d_vals.p, vals, vb, cudaMemcpyHostToDevice, c->st));
-      c->stats.h2d_bytes += (double)((size_t)key_len * n + 8 * (n + 1) + vb);
-      trie_root_leaves_dev(c, c->d_keys.as<uint8_t>(), key_len, flags, c->d_msg_off.as<uint64_t>(), c->d_vals.as<uint8_t>(), n, vb, root_out, &q);
-    } else {
-      trie_root_leaves_dev(c, nullptr, key_len, flags, nullptr, nullptr, n, 0, root_out, &q);  // the empty trie, or the argument error
-    }
-  });
-}
-
-int ppd_trie_subset_sorted_leaves_dev(ppd_ctx* c, const uint8_t* d_keys32, const uint64_t* d_val_off, const uint8_t* d_vals, size_t n, size_t vals_bytes,
-                                      const uint8_t* d_queries32, size_t m, uint8_t** out, size_t* out_len, uint8_t root_out[32]) {
-  (void)vals_bytes;
-  return guarded(c, [&] {
-    stats_reset(c);
-    const SubsetQuery q = subset_query(d_queries32, 32, 0, m, out, out_len);
-    trie_root_sorted_dev(c, d_keys32, d_val_off, d_vals, n, root_out, 0, &q);
-  });
 }
 
 }  // extern "C"

@@ -409,6 +409,14 @@ struct BranchKey {
   }
 };
 
+// after an update: the branches it hashes as BranchKey has them, then those whose refs it copied, one bucket per depth
+struct UpdateBranchKey {
+  static __device__ __forceinline__ uint32_t of(const uint8_t* __restrict__ depth, const uint32_t* __restrict__ nchild, uint32_t b) {
+    const uint32_t c = nchild[b];
+    return (c & BRANCH_CLEAN) ? BRANCH_BINS + 63u - depth[b] : (63u - depth[b]) * 16 + min(c, 15u);
+  }
+};
+
 // The items sorted are first .. first + n (n read from *n_dev - first when n_dev is given: the txn loop's node count is
 // only known on the device); keys[] and order[] are indexed from 0, order[] holds item ids.
 template <class Key, class A, class B>
@@ -510,6 +518,10 @@ void launch_order_by_level_class(const NodeRec* nodes, const uint16_t* level, ui
 void launch_order_branches(const uint8_t* depth, const uint32_t* nchild_minus_1, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
                            cudaStream_t st) {
   counting_sort<BranchKey>(depth, nchild_minus_1, nb, BRANCH_BINS, keys, bins, order, st, 0, nullptr);
+}
+void launch_order_update_branches(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
+                                  cudaStream_t st) {
+  counting_sort<UpdateBranchKey>(depth, nchild, nb, UPDATE_BRANCH_BINS, keys, bins, order, st, 0, nullptr);
 }
 
 // Stage and gather slots exceed the 48 KB of static shared memory: the kernel takes them as dynamic shared memory,

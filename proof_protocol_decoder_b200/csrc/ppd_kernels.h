@@ -31,6 +31,11 @@ void launch_order_by_level_class(const NodeRec* nodes, const uint16_t* level, ui
 static const uint32_t BRANCH_BINS = 1024;
 void launch_order_branches(const uint8_t* depth, const uint32_t* nchild_minus_1, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
                            cudaStream_t st);
+// ... after an update (ppd_update.cu): the branches to hash in the same buckets, and those whose refs were copied (nchild
+// tagged BRANCH_CLEAN) after them, in bucket BRANCH_BINS + 63 - depth; bins[UPDATE_BRANCH_BINS]
+static const uint32_t UPDATE_BRANCH_BINS = BRANCH_BINS + 64;
+void launch_order_update_branches(const uint8_t* depth, const uint32_t* nchild, uint32_t nb, uint16_t* keys, uint32_t* bins, uint32_t* order,
+                                  cudaStream_t st);
 
 // Small and medium copies done by a kernel instead of the copy engines: either side may be page-locked host memory
 // (device-accessible under unified addressing).  A copy engine serves its queue in order, so a few words a lane's host
@@ -91,7 +96,53 @@ void launch_leaders(const int8_t* L, const int8_t* m1, const int8_t* m2, const i
 void launch_branch_info(const BuildView& V, cudaStream_t st);
 void launch_child_count(const uint32_t* leader, const uint32_t* bidx, uint32_t n, uint32_t* nchild, cudaStream_t st);
 void launch_hash_sorted_leaves(const BuildView& V, cudaStream_t st);
+// the leaves list[0 .. count) only, already placed in their parents' child tables (an update's leaf pass)
+struct LeafList {
+  const uint32_t* list;
+  uint32_t count;
+};
+void launch_hash_listed_leaves(const BuildView& V, const uint32_t* list, uint32_t count, cudaStream_t st);
 void launch_hash_branch_level(const BuildView& V, const uint32_t* order, uint32_t begin, uint32_t end, cudaStream_t st);
+
+// ---- ppd_update.cu: an update of a resident trie (ppd_trie_update[_dev]) ----
+static const uint32_t MERGE_SRC_UPD = 0x80000000u;  // src[i]: the leaf is the batch's write at this sorted position
+struct MergeView {
+  // the batch, sorted: input position idx[j] of sorted position j, keep[j] = 1 at a key's last occurrence
+  const uint8_t* ukeys32;   // [k][32] in input order
+  const uint32_t *idx, *keep;
+  const uint8_t* del;       // [k] in input order, or nullptr
+  const uint64_t* uoff;     // [k + 1]
+  const uint8_t* uvals;
+  uint32_t k;
+  // the leaves before the update
+  const uint8_t* okeys;
+  const uint64_t* ooff;
+  const uint8_t* ovals;
+  uint32_t n_old;
+  // scratch: upos[k] lower bounds, written[k + 1] and its scan wpos, drop[n_old + 1] and its scan dpos, ins[n_old + 2]
+  // (writes inserted before each old leaf) and its scan ipos
+  uint32_t *upos, *written, *wpos, *drop, *dpos, *ins, *ipos;
+  // the merged leaves: src[n_new] (old position, or MERGE_SRC_UPD | sorted batch position), value lengths len[n_new + 1]
+  // and their scan noff (the new val_off), keys and values
+  uint32_t* src;
+  uint64_t *len, *noff;
+  uint8_t *nkeys, *nvals;
+  uint32_t n_new;
+};
+// the arrays of the trie before an update, read only
+struct OldTrie {
+  uint32_t n;
+  const int8_t* L;
+  const uint32_t *leader, *bidx;
+  const uint8_t *depth, *ext_start, *ref, *ref_len, *inner_ref, *inner_ref_len;
+};
+static const uint32_t BRANCH_CLEAN = 0x80000000u;  // nchild[b]: the update copied branch b's refs
+void launch_merge_locate(const MergeView& M, cudaStream_t st);  // drop, ins zeroed by the caller
+void launch_merge_place(const MergeView& M, cudaStream_t st);   // after the scans of written, drop and ins
+void launch_merge_copy(const MergeView& M, cudaStream_t st);    // after the scan of len
+void launch_update_leaves(const BuildView& V, const OldTrie& O, const uint32_t* src, uint32_t* list, uint32_t* count, cudaStream_t st);
+// bits: the marks of the batch's keys (launch_subset_mark over the new trie)
+void launch_update_branches(const BuildView& V, const OldTrie& O, const uint32_t* src, const uint32_t* bits, uint32_t* nchild, cudaStream_t st);
 
 // ---- ppd_subset.cu: create_trie_subset over the builder's structure (ppd_trie_subset_[sorted_]leaves[_dev]) ----
 static const uint32_t SUBSET_DEPTHS = 64;  // branch depths 0 .. 63

@@ -123,6 +123,15 @@ EXPORTS = [
     "ppd_trie_subset_leaves",
     "ppd_trie_subset_leaves_dev",
     "ppd_trie_subset_sorted_leaves_dev",
+    "ppd_trie_create_leaves_dev",
+    "ppd_trie_create_leaves",
+    "ppd_trie_create_sorted_leaves_dev",
+    "ppd_trie_info",
+    "ppd_trie_subset_dev",
+    "ppd_trie_subset",
+    "ppd_trie_update_dev",
+    "ppd_trie_update",
+    "ppd_trie_destroy",
 ]
 
 LEAVES_HASH_KEYS = 1  # PPD_LEAVES_HASH_KEYS: key i is keccak256 of the given key bytes
@@ -177,6 +186,17 @@ class PpdLibrary:
         L.ppd_trie_subset_leaves.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
         L.ppd_trie_subset_leaves_dev.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
         L.ppd_trie_subset_sorted_leaves_dev.argtypes = [vp, vp, vp, vp, sz, sz, vp, sz, u8pp, szp, ctypes.c_char_p]
+        tpp = ctypes.POINTER(ctypes.c_void_p)
+        L.ppd_trie_create_leaves_dev.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, sz, tpp, ctypes.c_char_p]
+        L.ppd_trie_create_leaves.argtypes = [vp, vp, ctypes.c_uint32, ctypes.c_uint32, vp, vp, sz, tpp, ctypes.c_char_p]
+        L.ppd_trie_create_sorted_leaves_dev.argtypes = [vp, vp, vp, vp, sz, sz, tpp, ctypes.c_char_p]
+        L.ppd_trie_info.argtypes = [vp, szp, ctypes.c_char_p]
+        L.ppd_trie_subset_dev.argtypes = [vp, vp, vp, sz, u8pp, szp]
+        L.ppd_trie_subset.argtypes = [vp, vp, vp, sz, u8pp, szp]
+        L.ppd_trie_update_dev.argtypes = [vp, vp, vp, vp, vp, vp, sz, sz, ctypes.c_char_p]
+        L.ppd_trie_update.argtypes = [vp, vp, vp, vp, vp, vp, sz, ctypes.c_char_p]
+        L.ppd_trie_destroy.argtypes = [vp]
+        L.ppd_trie_destroy.restype = None
 
     def exported(self):
         return [name for name in EXPORTS if hasattr(self.L, name)]
@@ -219,6 +239,71 @@ class OwnedBuffer:
             self.close()
         except Exception:
             pass
+
+
+class Trie:
+    """A ppd_trie: a trie resident in HBM, cut into subsets and updated in place (Context.trie_from_*).  It belongs to its
+    Context and is released by close(), or with the Context."""
+
+    def __init__(self, ctx, h, key_len, root):
+        self.ctx, self.h, self.key_len, self.root = ctx, h, key_len, root
+
+    @property
+    def n(self) -> int:
+        n = ctypes.c_size_t()
+        self.ctx._check(self.ctx.lib.L.ppd_trie_info(self.h, ctypes.byref(n), None))
+        return n.value
+
+    def subset(self, queries) -> bytes:
+        """create_trie_subset of the current trie for uint8 [m, key_len] query keys (as Context.trie_subset_leaves)."""
+        import numpy as np
+
+        queries = np.ascontiguousarray(queries, dtype=np.uint8)
+        if queries.ndim != 2 or (len(queries) and queries.shape[1] != self.key_len):
+            raise ValueError("queries must be [m, key_len] with the trie's key_len")
+        out, n = ctypes.POINTER(ctypes.c_uint8)(), ctypes.c_size_t()
+        self.ctx._check(self.ctx.lib.L.ppd_trie_subset(self.ctx.h, self.h, queries.ctypes.data, queries.shape[0], ctypes.byref(out), ctypes.byref(n)))
+        return self.ctx._take(out, n)
+
+    def subset_dev(self, d_queries_ptr, m) -> bytes:
+        out, n = ctypes.POINTER(ctypes.c_uint8)(), ctypes.c_size_t()
+        self.ctx._check(self.ctx.lib.L.ppd_trie_subset_dev(self.ctx.h, self.h, d_queries_ptr, m, ctypes.byref(out), ctypes.byref(n)))
+        return self.ctx._take(out, n)
+
+    def update(self, keys, val_off, vals, deletes=None) -> bytes:
+        """Applies the updates in order: row i of keys (uint8 [k, key_len]) gets vals[val_off[i]:val_off[i + 1]], or is
+        deleted where deletes[i] is true.  -> the new root."""
+        import numpy as np
+
+        keys = np.ascontiguousarray(keys, dtype=np.uint8).reshape(-1, self.key_len)
+        val_off = np.ascontiguousarray(val_off, dtype=np.uint64)
+        vals = np.ascontiguousarray(vals, dtype=np.uint8)
+        if keys.shape[0] != len(val_off) - 1:
+            raise ValueError("keys must be [k, key_len] with k = len(val_off) - 1")
+        dl = None if deletes is None else np.ascontiguousarray(deletes, dtype=np.uint8)
+        root = ctypes.create_string_buffer(32)
+        self.ctx._check(self.ctx.lib.L.ppd_trie_update(self.ctx.h, self.h, keys.ctypes.data, None if dl is None else dl.ctypes.data,
+                                                       val_off.ctypes.data, vals.ctypes.data, keys.shape[0], root))
+        self.root = root.raw
+        return self.root
+
+    def update_dev(self, d_keys_ptr, d_del_ptr, d_val_off_ptr, d_vals_ptr, k, vals_bytes) -> bytes:
+        """update on device buffers (d_del_ptr may be None)."""
+        root = ctypes.create_string_buffer(32)
+        self.ctx._check(self.ctx.lib.L.ppd_trie_update_dev(self.ctx.h, self.h, d_keys_ptr, d_del_ptr, d_val_off_ptr, d_vals_ptr, k, vals_bytes, root))
+        self.root = root.raw
+        return self.root
+
+    def close(self):
+        if self.h and self.ctx.h:
+            self.ctx.lib.L.ppd_trie_destroy(self.h)
+        self.h = ctypes.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
 
 
 class Context:
@@ -465,6 +550,36 @@ class Context:
         self._check(self.lib.L.ppd_trie_subset_sorted_leaves_dev(self.h, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, d_queries_ptr, m,
                                                                  ctypes.byref(out), ctypes.byref(nb), root))
         return root.raw, self._take(out, nb)
+
+    def trie_from_leaves(self, keys, val_off, vals, hash_keys=False) -> "Trie":
+        """A Trie handle over the leaves trie_root_leaves takes (host buffers): built once, kept in HBM."""
+        import numpy as np
+
+        keys = np.ascontiguousarray(keys, dtype=np.uint8)
+        val_off = np.ascontiguousarray(val_off, dtype=np.uint64)
+        vals = np.ascontiguousarray(vals, dtype=np.uint8)
+        if keys.ndim != 2 or keys.shape[0] != len(val_off) - 1:
+            raise ValueError("keys must be [n, key_len] with n = len(val_off) - 1")
+        h, root = ctypes.c_void_p(), ctypes.create_string_buffer(32)
+        flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_create_leaves(self.h, keys.ctypes.data, keys.shape[1], flags, val_off.ctypes.data, vals.ctypes.data,
+                                                      keys.shape[0], ctypes.byref(h), root))
+        return Trie(self, h, keys.shape[1], root.raw)
+
+    def trie_from_leaves_dev(self, d_keys_ptr, key_len, d_val_off_ptr, d_vals_ptr, n, vals_bytes, hash_keys=False, flags=None) -> "Trie":
+        """trie_from_leaves on device buffers (complete when it is called; only read during the call)."""
+        h, root = ctypes.c_void_p(), ctypes.create_string_buffer(32)
+        if flags is None:
+            flags = LEAVES_HASH_KEYS if hash_keys else 0
+        self._check(self.lib.L.ppd_trie_create_leaves_dev(self.h, d_keys_ptr, key_len, flags, d_val_off_ptr, d_vals_ptr, n, vals_bytes,
+                                                          ctypes.byref(h), root))
+        return Trie(self, h, key_len, root.raw)
+
+    def trie_from_sorted_leaves_dev(self, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes) -> "Trie":
+        """A Trie handle over leaves sorted by 32-byte key (device pointers, copied into the handle)."""
+        h, root = ctypes.c_void_p(), ctypes.create_string_buffer(32)
+        self._check(self.lib.L.ppd_trie_create_sorted_leaves_dev(self.h, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, ctypes.byref(h), root))
+        return Trie(self, h, 32, root.raw)
 
     def trie_subroot_sorted_leaves_dev(self, d_keys_ptr, d_val_off_ptr, d_vals_ptr, n, vals_bytes, base_depth) -> bytes:
         """The ref of the sub-trie over n sorted leaves that share their first base_depth nibbles (device pointers)."""
